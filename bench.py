@@ -8,18 +8,23 @@ Inputs: the "dense" synthetic regime of SURVEY.md section 8(d) (2048 encoder + 2
 1009 rgb + 1009 depth + 15 cam + 15 gaze on both sides), random-init ego-b weights (396.2 M params), bf16 tensor-core
 compute with fp32 masters / residual stream.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B_per_gpu] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B_per_gpu] [--impl reference] [--dump-outputs DIR]
 
 `value` = nominal tokens/s of the whole job (global batch x 4096 / step time, the reference's own accounting,
 run_training_egom2p.py:645-647) timed on the device with inputs resident in HBM; `e2e` = the same metric through the
 public model API with pinned-host inputs copied every step and the loss read back. `--impl reference` times the CPU
 restatement of the reference path (oracle/, fp32, all host threads) on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step computed as DIR/<name>.npy (float32): for training the loss, the
+per-modality losses, the gradient norm and a fixed seeded sample of every parameter after the update; for generation the
+generated tokens. Inputs, weights and the decoder modality order are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -116,6 +121,27 @@ def step_flops(md) -> float:
         head = sum(kept[m] * D * MI[m]["vocab_size"] for m in mods)
         total += 3 * 2.0 * (enc + ctx + dec + head)
     return total
+
+
+def param_sample(model, k: int = 4096, seed: int = 0) -> dict:
+    """A fixed, seeded sample of up to k elements of every parameter, as device tensors."""
+    rng = np.random.default_rng(seed)
+    out = {}
+    for n, p in model.named_parameters():
+        flat = p.detach().reshape(-1)
+        idx = np.arange(flat.numel()) if flat.numel() <= k else np.sort(rng.choice(flat.numel(), k, replace=False))
+        out[f"param.{n}"] = flat.index_select(0, torch.from_numpy(idx).to(flat.device))
+    return out
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes every array as out_dir/<name>.npy in float32."""
+    host = {n: np.asarray(a.detach().float().cpu() if torch.is_tensor(a) else a, dtype=np.float32) for n, a in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= 64 << 20, f"--dump-outputs: {total} bytes exceed the 64 MB budget"
+    os.makedirs(out_dir, exist_ok=True)
+    for n, a in host.items():
+        np.save(os.path.join(out_dir, n + ".npy"), a)
 
 
 def md_bytes(md):
@@ -361,7 +387,11 @@ def run_generation(args):
         sampler_clk = ClockSampler(0)
         sampler_clk.start()
         l0 = _lib.launch_count()
-        ms = timed(lambda i: call(devt[args.warmup + i]), args.steps)
+        last = {}
+
+        def timed_call(i):
+            last["tokens"] = call(devt[args.warmup + i])
+        ms = timed(timed_call, args.steps)
         launches = _lib.launch_count() - l0
         clocks = sampler_clk.stop()
         ms_e2e = timed(lambda i: call(host[args.warmup + i].to(dev, non_blocking=True)).cpu(), args.steps)
@@ -417,6 +447,8 @@ def run_generation(args):
             best = max((r["clips_per_s"] for r in res if "clips_per_s" in r), default=None)
             if best:
                 line["reference_gpu_speedup"] = line["value"] / best
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tokens": last["tokens"]})
     print(json.dumps(line), flush=True)
 
 
@@ -470,7 +502,13 @@ def main():
     ap.add_argument("--no-reference-gpu", action="store_true",
                     help="skip timing the unmodified reference (baseline/_ref, eager bf16 autocast) on this GPU (N = 1 only)")
     ap.add_argument("--cpu-steps", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU paths (--impl ours)")
     args.batch_given = args.batch is not None
     if args.batch is None:
         args.batch = int(os.environ.get("EGOM2P_BENCH_BATCH", "32"))
@@ -481,7 +519,6 @@ def main():
         args.warmup = max(args.warmup, 1) if args.workload == "depth2rgb" else max(args.warmup, 3)
         return run_generation(args)
     if args.impl == "reference":
-        args.steps = min(args.steps, 2)
         args.warmup = min(args.warmup, 1)
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -534,12 +571,12 @@ def main():
         loss, mod_loss = net(md, N_ENC, N_DEC, loss_type="mod")
         loss.backward()
         if args.optimizer == "fused":
-            opt.clip_grad_norm_(1.0)
+            grad_norm = opt.clip_grad_norm_(1.0)
         else:
-            torch.nn.utils.clip_grad_norm_(params, 1.0)
+            grad_norm = torch.nn.utils.clip_grad_norm_(params, 1.0)
         opt.step()
         opt.zero_grad(set_to_none=True)
-        return loss
+        return loss, mod_loss, grad_norm
 
     def sync():
         if world > 1:
@@ -569,21 +606,30 @@ def main():
             model.zero_grad(set_to_none=True)
 
     # ---- warm-up, then device-resident timing
+    random.seed(0)   # the decoder modality order, so that every run computes the same steps
     for i in range(args.warmup):
         step(dev_batches[i])
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
     l0 = _lib.launch_count()
-    ms = timed(lambda i: step(dev_batches[args.warmup + i]), args.steps)
+    last = {}
+
+    def timed_step(i):
+        last["out"] = step(dev_batches[args.warmup + i])
+    ms = timed(timed_step, args.steps)
     launches = _lib.launch_count() - l0
     clocks = sampler.stop() if sampler else None
+    outputs = None
+    if args.dump_outputs and rank == 0:   # before the steps below move the weights on
+        loss, mod_loss, grad_norm = last["out"]
+        outputs = {"loss": loss, "grad_norm": grad_norm, **{f"mod_loss.{m}": v for m, v in mod_loss.items()},
+                   **param_sample(model)}
 
     # ---- end-to-end through the public API: pinned host inputs copied every step, loss read back every step
     def e2e_step(i):
         md = {m: {k: v.to(dev, non_blocking=True) for k, v in d.items()} for m, d in host_batches[args.warmup + i].items()}
-        loss = step(md)
-        return loss.item()
+        return step(md)[0].item()
     e2e_step(0)
     ms_e2e = timed(e2e_step, args.steps)
     last_loss = e2e_step(0)
@@ -714,6 +760,8 @@ def main():
                     line["reference_gpu_speedup"] = value / best
             else:
                 line["reference_gpu"] = {"unavailable": "baseline/_ref/egom2p missing (tools/install_reference.py)"}
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
