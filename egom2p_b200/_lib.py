@@ -38,9 +38,13 @@ SIGNATURES = {
     "egom2p_embed_gather_bwd": [C.POINTER(EmbedDesc), vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp, vp],
     "egom2p_layernorm_fwd": [vp, vp, i64, i32, f32, vp, vp, vp, vp, vp],
     "egom2p_layernorm_bwd": [vp, vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp, vp],
+    "egom2p_layernorm_bias_fwd": [vp, vp, vp, i64, i32, f32, vp, vp, vp, vp, vp],
+    "egom2p_layernorm_bias_bwd": [vp, vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp],
     "egom2p_gemm_bf16": [vp, vp, i32, i32, i32, i64, i64, i32, i32, vp, vp, i64, vp, vp, i64, vp],
     "egom2p_gemm_swiglu_fwd": [vp, vp, i32, i32, i32, i64, i64, vp, i64, vp, i64, vp],
     "egom2p_gemm_swiglu_bwd": [vp, vp, vp, i32, i32, i32, i64, i64, i64, vp, i64, vp],
+    "egom2p_gemm_gelu_fwd": [vp, vp, vp, i32, i32, i32, i64, i64, vp, i64, vp, i64, vp],
+    "egom2p_gemm_gelu_bwd": [vp, vp, vp, i32, i32, i32, i64, i64, i64, vp, i64, vp],
     "egom2p_ce_partials": [vp, vp, vp, i32, i32, i32, i64, i64, vp, vp, vp, vp],
     "egom2p_ce_finalize": [vp, vp, vp, i32, i32, vp, vp, vp],
     "egom2p_ce_dlogits": [vp, vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, vp, i64, vp],
@@ -60,6 +64,7 @@ SIGNATURES = {
     "egom2p_sample_rows": [vp, i64, i32, i32, f32, f32, i32, vp, vp, vp, vp, vp],
     "egom2p_cfg_combine_bf16": [vp, vp, i64, f32, vp, vp],
     "egom2p_colsum_f32": [vp, i64, i32, vp, vp],
+    "egom2p_colsum_bf16": [vp, i64, i32, i64, vp, vp],
     "egom2p_gather_rows_bf16": [vp, vp, i64, i32, vp, vp],
     "egom2p_scatter_rows_f32": [vp, vp, i64, i32, vp, vp],
 }

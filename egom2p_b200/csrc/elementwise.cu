@@ -241,6 +241,42 @@ __global__ void __launch_bounds__(kEwThreads) colsum_kernel(const float* __restr
   }
 }
 
+// out[c] += sum_r x[r, c] for a bf16 (R, cols) matrix of row pitch ld: the bias gradients of the GELU / bias family (R up to
+// 65 536 rows per call). A CTA owns 256 columns (8 per lane, one 16-byte load) and a slab of rows; its 8 warps stride the
+// slab and meet in shared memory, so each column takes one atomic per slab. The slab height is chosen on the host so that
+// the grid fills the machine about four times over: ~70 atomics per column at 65 536 rows.
+__global__ void __launch_bounds__(kEwThreads) colsum_bf16_kernel(const uint16_t* __restrict__ x, int64_t rows, int cols, int64_t ld,
+                                                                 int64_t rows_per_cta, float* __restrict__ out) {
+  __shared__ float part[kEwThreads / 32][256];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int c0 = blockIdx.x * 256 + lane * 8;
+  const int64_t r0 = (int64_t)blockIdx.y * rows_per_cta, r1 = min(r0 + rows_per_cta, rows);
+  float s[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  if (c0 < cols) {
+#pragma unroll 4
+    for (int64_t r = r0 + warp; r < r1; r += kEwThreads / 32) {
+      const uint4 v = __ldg(reinterpret_cast<const uint4*>(x + r * ld + c0));
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int t = 0; t < 4; ++t) {
+        const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[t]));
+        s[2 * t] += f.x;
+        s[2 * t + 1] += f.y;
+      }
+    }
+  }
+#pragma unroll
+  for (int t = 0; t < 8; ++t) part[warp][lane * 8 + t] = s[t];
+  __syncthreads();
+  const int c = blockIdx.x * 256 + threadIdx.x;
+  if (threadIdx.x < 256 && c < cols) {
+    float t = 0.f;
+#pragma unroll
+    for (int w = 0; w < kEwThreads / 32; ++w) t += part[w][threadIdx.x];
+    atomicAdd(out + c, t);
+  }
+}
+
 // Row gather / scatter-add used to (un)compact the rows of one modality for its vocabulary head.
 __global__ void __launch_bounds__(kEwThreads) gather_rows_bf16_kernel(const uint16_t* __restrict__ src, const int64_t* __restrict__ idx,
                                                                       int64_t n, int cols8, uint16_t* __restrict__ dst) {
@@ -268,6 +304,21 @@ extern "C" int egom2p_colsum_f32(const float* x, int64_t rows, int32_t cols, flo
   EGO_REQUIRE(x && out && rows > 0 && cols > 0, "colsum_f32: bad argument");
   colsum_kernel<<<(unsigned)((rows + 63) / 64), kEwThreads, 0, (cudaStream_t)stream>>>(x, rows, cols, out);
   return check_launch("colsum_f32");
+}
+extern "C" int egom2p_colsum_bf16(const uint16_t* x, int64_t rows, int32_t cols, int64_t ld, float* out, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(x && out && rows > 0 && cols > 0 && cols % 8 == 0 && ld % 8 == 0 && ((uintptr_t)x & 15) == 0,
+              "colsum_bf16: bad argument (cols, ld multiples of 8, 16-byte aligned rows)");
+  const unsigned col_blocks = (unsigned)((cols + 255) / 256);
+  const int64_t want = 4 * (int64_t)device_sm_count();                     // CTAs for the whole grid
+  int64_t slabs = (want + col_blocks - 1) / col_blocks;
+  const int64_t min_rows = 64;                                             // keep every warp busy for a few rows
+  if (slabs > (rows + min_rows - 1) / min_rows) slabs = (rows + min_rows - 1) / min_rows;
+  if (slabs < 1) slabs = 1;
+  const int64_t rows_per_cta = (rows + slabs - 1) / slabs;
+  slabs = (rows + rows_per_cta - 1) / rows_per_cta;
+  colsum_bf16_kernel<<<dim3(col_blocks, (unsigned)slabs), kEwThreads, 0, (cudaStream_t)stream>>>(x, rows, cols, ld, rows_per_cta, out);
+  return check_launch("colsum_bf16");
 }
 extern "C" int egom2p_gather_rows_bf16(const uint16_t* src, const int64_t* idx, int64_t n, int32_t cols, uint16_t* dst, void* stream) {
   using namespace egom2p;

@@ -22,7 +22,10 @@ constexpr int BK = 64;
 constexpr int kEpiWarps = 8;
 constexpr int kGemmThreads = 64 + 32 * kEpiWarps;
 
-enum { EPI_STORE = 0, EPI_CE_PARTIAL = 1, EPI_CE_DLOGITS = 2, EPI_SWIGLU_FWD = 3, EPI_SWIGLU_BWD = 4 };
+// EPI_STORE_BIAS_BF16: EPI_STORE with bf16 output and a bias -- its own instantiation, so that the bias code does not cost
+// the plain stores registers.
+enum { EPI_STORE = 0, EPI_CE_PARTIAL = 1, EPI_CE_DLOGITS = 2, EPI_SWIGLU_FWD = 3, EPI_SWIGLU_BWD = 4, EPI_GELU_FWD = 5,
+       EPI_GELU_BWD = 6, EPI_STORE_BIAS_BF16 = 7 };
 
 struct GemmParams {
   int M, N, K;
@@ -36,7 +39,8 @@ struct GemmParams {
   const int64_t* target;
   const float* lse;
   const float* gscale;
-  // SwiGLU epilogues: ab = [a | b] interleaved in groups of 32 columns (bf16), row pitch ld_ab
+  // SwiGLU epilogues: ab = [a | b] interleaved in groups of 32 columns (bf16), row pitch ld_ab.
+  // GELU backward: ab = the saved pre-activation u (bf16), row pitch ld_ab; GELU forward: ld_ab = row pitch of GELU(u).
   const uint16_t* ab;
   int64_t ld_ab;
   int v0;
@@ -68,6 +72,13 @@ __device__ __forceinline__ float sigmoid_fast(float x) {
   float t;
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * x));
   return fmaf(0.5f, t, 0.5f);
+}
+// GELU of nn.GELU() (exact erf form) and its derivative Phi(u) + u * phi(u). erff is within 2 ulp of erf in fp32 and __expf
+// within 2 ulp + 2^-21 relative for |arg| <= 32 (|u| <= 8): both errors are below 2^-18 relative to the results, far below
+// the 2^-9 relative rounding of the bf16 values they are stored as.
+__device__ __forceinline__ float gelu_erf(float u) { return 0.5f * u * (1.f + erff(u * 0.70710678118654752f)); }
+__device__ __forceinline__ float gelu_erf_grad(float u) {
+  return 0.5f * (1.f + erff(u * 0.70710678118654752f)) + u * 0.39894228040143268f * __expf(-0.5f * u * u);
 }
 __device__ __forceinline__ uint32_t box_off(int row, int chunk) {  // 16-byte chunk inside a [32][128 B] SW128 box
   return (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
@@ -417,7 +428,122 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             tma_store_commit();
           }
         }
-      } else if (EPI == EPI_CE_DLOGITS || p.out_bf16) {
+      } else if constexpr (EPI == EPI_GELU_FWD) {
+        // ---- fc1 GEMM: u = acc + b1 and GELU(u), 64 columns (one 128-byte box row) per step. The u box (bf16, saved for
+        // backward) and the GELU(u) box (bf16, the operand of the fc2 GEMM) leave through the warp's staging box in turn.
+        auto store_box = [&](const uint32_t (&a)[32], const uint32_t (&b)[32], const CUtensorMap* map, int cbase) {
+          tma_store_wait_read();
+          __syncwarp();
+#pragma unroll
+          for (int j = 0; j < 4; ++j) {
+            *reinterpret_cast<uint4*>(box + box_off(lane, j)) =
+                make_uint4(pack_bf16(__uint_as_float(a[8 * j + 0]), __uint_as_float(a[8 * j + 1])),
+                           pack_bf16(__uint_as_float(a[8 * j + 2]), __uint_as_float(a[8 * j + 3])),
+                           pack_bf16(__uint_as_float(a[8 * j + 4]), __uint_as_float(a[8 * j + 5])),
+                           pack_bf16(__uint_as_float(a[8 * j + 6]), __uint_as_float(a[8 * j + 7])));
+            *reinterpret_cast<uint4*>(box + box_off(lane, j + 4)) =
+                make_uint4(pack_bf16(__uint_as_float(b[8 * j + 0]), __uint_as_float(b[8 * j + 1])),
+                           pack_bf16(__uint_as_float(b[8 * j + 2]), __uint_as_float(b[8 * j + 3])),
+                           pack_bf16(__uint_as_float(b[8 * j + 4]), __uint_as_float(b[8 * j + 5])),
+                           pack_bf16(__uint_as_float(b[8 * j + 6]), __uint_as_float(b[8 * j + 7])));
+          }
+          fence_async_smem();
+          __syncwarp();
+          if (lane == 0) {
+            if (row0 < p.M && cbase < p.N) tma_store_2d(map, box, cbase, row0);
+            tma_store_commit();
+          }
+        };
+#pragma unroll 1
+        for (int c = 0; c < kHalfCols / 64; ++c) {
+          uint32_t v0[32], v1[32];
+          tmem_ld32(t_addr + c * 64, v0);
+          tmem_ld32(t_addr + c * 64 + 32, v1);
+          tmem_ld_wait();
+          const int cbase = n0 + c * 64;
+          if (p.bias) {   // N % 64 == 0: the 64 columns are all inside or all outside
+            if (cbase < p.N) {
+#pragma unroll
+              for (int j = 0; j < 8; ++j) {
+                const float4 ba = __ldg(reinterpret_cast<const float4*>(p.bias + cbase) + j);
+                const float4 bb = __ldg(reinterpret_cast<const float4*>(p.bias + cbase + 32) + j);
+                v0[4 * j + 0] = __float_as_uint(__uint_as_float(v0[4 * j + 0]) + ba.x);
+                v0[4 * j + 1] = __float_as_uint(__uint_as_float(v0[4 * j + 1]) + ba.y);
+                v0[4 * j + 2] = __float_as_uint(__uint_as_float(v0[4 * j + 2]) + ba.z);
+                v0[4 * j + 3] = __float_as_uint(__uint_as_float(v0[4 * j + 3]) + ba.w);
+                v1[4 * j + 0] = __float_as_uint(__uint_as_float(v1[4 * j + 0]) + bb.x);
+                v1[4 * j + 1] = __float_as_uint(__uint_as_float(v1[4 * j + 1]) + bb.y);
+                v1[4 * j + 2] = __float_as_uint(__uint_as_float(v1[4 * j + 2]) + bb.z);
+                v1[4 * j + 3] = __float_as_uint(__uint_as_float(v1[4 * j + 3]) + bb.w);
+              }
+            }
+          }
+          store_box(v0, v1, &tmCb, cbase);   // u
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            v0[j] = __float_as_uint(gelu_erf(__uint_as_float(v0[j])));
+            v1[j] = __float_as_uint(gelu_erf(__uint_as_float(v1[j])));
+          }
+          store_box(v0, v1, &tmCf, cbase);   // aux map = GELU(u) (rows, N) bf16
+        }
+      } else if constexpr (EPI == EPI_GELU_BWD) {
+        // ---- fc2 dgrad: acc = dh, 64 columns per step; with the saved pre-activation u of the same columns emit
+        // du = dh * GELU'(u) (bf16). u is fetched coalesced (8 lanes per 128-byte row, 4 rows per instruction) and
+        // transposed through the warp's staging box, as in the SwiGLU backward; its loads are in flight while the
+        // accumulator is read. (A one-step-ahead prefetch, as there, spills at the 168-register cap.)
+        constexpr int kSteps = kHalfCols / 64;
+        uint4 ubuf[8];
+        auto fetch = [&](int c, uint4 (&dst)[8]) {
+          const int cbase = n0 + c * 64;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const int r = row0 + 4 * i + (lane >> 3);
+            dst[i] = (r < p.M && cbase < p.N)
+                         ? __ldg(reinterpret_cast<const uint4*>(p.ab + (int64_t)r * p.ld_ab + cbase) + (lane & 7))
+                         : make_uint4(0u, 0u, 0u, 0u);
+          }
+        };
+#pragma unroll 1
+        for (int c = 0; c < kSteps; ++c) {
+          uint32_t v[32];
+          fetch(c, ubuf);
+          tmem_ld32(t_addr + c * 64, v);
+          const int cbase = n0 + c * 64;
+          uint4 ur[8];
+          tma_store_wait_read();   // the previous store out of this warp's box has been read
+          __syncwarp();
+#pragma unroll
+          for (int i = 0; i < 8; ++i) *reinterpret_cast<uint4*>(box + box_off(4 * i + (lane >> 3), lane & 7)) = ubuf[i];
+          __syncwarp();
+#pragma unroll
+          for (int j = 0; j < 8; ++j) ur[j] = *reinterpret_cast<const uint4*>(box + box_off(lane, j));  // this lane's row
+          __syncwarp();            // every lane holds its row before the box is reused for the output
+          // the 64 accumulator columns are read in two halves of 32: one half in registers at a time (no spills)
+#pragma unroll
+          for (int hh = 0; hh < 2; ++hh) {
+            if (hh) tmem_ld32(t_addr + c * 64 + 32, v);
+            tmem_ld_wait();
+#pragma unroll
+            for (int j = 4 * hh; j < 4 * hh + 4; ++j) {
+              const uint32_t uw[4] = {ur[j].x, ur[j].y, ur[j].z, ur[j].w};
+              uint32_t o[4];
+#pragma unroll
+              for (int t = 0; t < 4; ++t) {
+                const float2 fu = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&uw[t]));
+                const int k = 8 * (j - 4 * hh) + 2 * t;
+                o[t] = pack_bf16(__uint_as_float(v[k]) * gelu_erf_grad(fu.x), __uint_as_float(v[k + 1]) * gelu_erf_grad(fu.y));
+              }
+              *reinterpret_cast<uint4*>(box + box_off(lane, j)) = make_uint4(o[0], o[1], o[2], o[3]);
+            }
+          }
+          fence_async_smem();
+          __syncwarp();
+          if (lane == 0) {   // (an empty group when the box is out of range keeps the wait_group accounting uniform)
+            if (row0 < p.M && cbase < p.N) tma_store_2d(&tmCb, box, cbase, row0);   // output map = du (rows, N) bf16
+            tma_store_commit();
+          }
+        }
+      } else if (EPI == EPI_CE_DLOGITS || EPI == EPI_STORE_BIAS_BF16 || p.out_bf16) {
         // ---- bf16 output: 64 columns (one 128-byte box row) per step
 #pragma unroll 1
         for (int c = 0; c < kHalfCols / 64; ++c) {
@@ -434,6 +560,20 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
               if (cbase + 32 + j == row_tgt) p1 -= 1.f;
               v0[j] = __float_as_uint(p0 * gs);
               v1[j] = __float_as_uint(p1 * gs);
+            }
+          }
+          if constexpr (EPI == EPI_STORE_BIAS_BF16) {   // N % 8 == 0: a float4 of the bias is either wholly inside or wholly outside
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+              const int k = (j & 7) * 4, col = cbase + (j >> 3) * 32 + k;
+              if (col < p.N) {
+                const float4 bv = __ldg(reinterpret_cast<const float4*>(p.bias + col));
+                uint32_t* v = j < 8 ? v0 : v1;
+                v[k + 0] = __float_as_uint(__uint_as_float(v[k + 0]) + bv.x);
+                v[k + 1] = __float_as_uint(__uint_as_float(v[k + 1]) + bv.y);
+                v[k + 2] = __float_as_uint(__uint_as_float(v[k + 2]) + bv.z);
+                v[k + 3] = __float_as_uint(__uint_as_float(v[k + 3]) + bv.w);
+              }
             }
           }
           uint8_t* bx = box;
@@ -557,7 +697,12 @@ static int launch_gemm(const uint16_t* A, const uint16_t* B, int64_t lda, int64_
   if (rc) return rc;
   tmCb = tmA;
   tmCf = tmA;
-  if (EPI == EPI_SWIGLU_BWD) {          // c_bf16 = dab (M, 2N)
+  if (EPI == EPI_GELU_BWD) {            // c_bf16 = du (M, N)
+    if ((rc = make_tmap_2d(&tmCb, c_bf16, 2, p.M, p.N, ldc, 32, 64))) return rc;
+  } else if (EPI == EPI_GELU_FWD) {     // c_bf16 = u (M, N); c_f32 slot carries GELU(u) (M, N) bf16 with pitch p.ld_ab
+    if ((rc = make_tmap_2d(&tmCb, c_bf16, 2, p.M, p.N, ldc, 32, 64))) return rc;
+    if ((rc = make_tmap_2d(&tmCf, c_f32, 2, p.M, p.N, p.ld_ab, 32, 64))) return rc;
+  } else if (EPI == EPI_SWIGLU_BWD) {   // c_bf16 = dab (M, 2N)
     if ((rc = make_tmap_2d(&tmCb, c_bf16, 2, p.M, 2 * (uint64_t)p.N, ldc, 32, 64))) return rc;
   } else if (EPI == EPI_SWIGLU_FWD) {   // c_bf16 = ab (M, N); c_f32 slot carries g (M, N/2) bf16 with pitch p.ld_ab
     if ((rc = make_tmap_2d(&tmCb, c_bf16, 2, p.M, p.N, ldc, 32, 64))) return rc;
@@ -618,12 +763,16 @@ static int dispatch_gemm(const uint16_t* A, const uint16_t* B, int64_t lda, int6
   // BN = 256 halves B re-reads per tile; BN = 128 gives better wave quantisation on small problems.
   const int sms = sm_count();
   const int64_t tiles256 = (int64_t)((p.M + BM - 1) / BM) * ((p.N + 255) / 256);
-  const bool use256 = (EPI != EPI_STORE) || (p.N >= 256 && (tiles256 >= 2 * sms || !c_bf16));
+  constexpr bool kStore = EPI == EPI_STORE || EPI == EPI_STORE_BIAS_BF16;
+  const bool use256 = !kStore || (p.N >= 256 && (tiles256 >= 2 * sms || !c_bf16));
 #define EGO_GEMM_CASE(BN_, AM, BMJ) return launch_gemm<BN_, AM, BMJ, EPI>(A, B, lda, ldb, c_bf16, c_f32, ldc, p, stream)
-  if constexpr (EPI == EPI_SWIGLU_BWD) {  // dg = dY W2 (B consumed MN-major)
+  if constexpr (EPI == EPI_SWIGLU_BWD || EPI == EPI_GELU_BWD) {  // dg / dh = dY W2 (B consumed MN-major)
     EGO_GEMM_CASE(256, false, true);
-  } else if constexpr (EPI != EPI_STORE) {  // CE / SwiGLU-forward epilogues: K-major x K-major
+  } else if constexpr (!kStore) {  // CE / SwiGLU- and GELU-forward epilogues: K-major x K-major
     EGO_GEMM_CASE(256, false, false);
+  } else if constexpr (EPI == EPI_STORE_BIAS_BF16) {  // biased projections (qkv, q, kv): K-major x K-major
+    if (use256) EGO_GEMM_CASE(256, false, false);
+    EGO_GEMM_CASE(128, false, false);
   } else if (use256) {
     if (!a_mn && !b_mn) EGO_GEMM_CASE(256, false, false);
     if (!a_mn && b_mn) EGO_GEMM_CASE(256, false, true);
@@ -650,6 +799,11 @@ extern "C" int egom2p_gemm_bf16(const uint16_t* A, const uint16_t* B, int32_t M,
   EGO_REQUIRE(!c_bf16 || (N % 8 == 0 && ldc % 8 == 0), "gemm_bf16: bf16 output needs N, ldc multiples of 8");
   GemmParams p{};
   p.M = M; p.N = N; p.K = K; p.bias = bias; p.addend = addend; p.ld_add = ld_add;
+  if (c_bf16 && bias) {
+    EGO_REQUIRE(!a_mn && !b_mn && !addend, "gemm_bf16: a bias with bf16 output needs K-major A and B and no addend");
+    EGO_REQUIRE(((uintptr_t)bias & 15) == 0, "gemm_bf16: bias must be 16-byte aligned");
+    return dispatch_gemm<EPI_STORE_BIAS_BF16>(A, B, lda, ldb, 0, 0, c_bf16, nullptr, ldc, p, (cudaStream_t)stream);
+  }
   return dispatch_gemm<EPI_STORE>(A, B, lda, ldb, a_mn, b_mn, c_bf16, c_f32, ldc, p, (cudaStream_t)stream);
 }
 
@@ -692,6 +846,27 @@ extern "C" int egom2p_gemm_swiglu_bwd(const uint16_t* dY, const uint16_t* W2, co
   GemmParams p{};
   p.M = M; p.N = hidden; p.K = K; p.ab = ab; p.ld_ab = ld_ab;
   return dispatch_gemm<EPI_SWIGLU_BWD>(dY, W2, ldy, ldw, 0, 1, dab, nullptr, ld_dab, p, (cudaStream_t)stream);
+}
+
+extern "C" int egom2p_gemm_gelu_fwd(const uint16_t* X, const uint16_t* W1, const float* b1, int32_t M, int32_t N, int32_t K,
+                                    int64_t ldx, int64_t ldw, uint16_t* u, int64_t ld_u, uint16_t* h, int64_t ldh, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(X && W1 && u && h && M > 0 && N > 0 && K > 0, "gemm_gelu_fwd: bad argument");
+  EGO_REQUIRE(N % 64 == 0 && ld_u % 8 == 0 && ldh % 8 == 0, "gemm_gelu_fwd: hidden must be a multiple of 64");
+  EGO_REQUIRE(!b1 || ((uintptr_t)b1 & 15) == 0, "gemm_gelu_fwd: bias must be 16-byte aligned");
+  GemmParams p{};
+  p.M = M; p.N = N; p.K = K; p.bias = b1; p.ld_ab = ldh;
+  return dispatch_gemm<EPI_GELU_FWD>(X, W1, ldx, ldw, 0, 0, u, reinterpret_cast<float*>(h), ld_u, p, (cudaStream_t)stream);
+}
+
+extern "C" int egom2p_gemm_gelu_bwd(const uint16_t* dY, const uint16_t* W2, const uint16_t* u, int32_t M, int32_t hidden, int32_t K,
+                                    int64_t ldy, int64_t ldw, int64_t ld_u, uint16_t* du, int64_t ld_du, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(dY && W2 && u && du && M > 0 && hidden > 0 && K > 0, "gemm_gelu_bwd: bad argument");
+  EGO_REQUIRE(hidden % 64 == 0 && ld_u % 8 == 0 && ld_du % 8 == 0, "gemm_gelu_bwd: hidden must be a multiple of 64");
+  GemmParams p{};
+  p.M = M; p.N = hidden; p.K = K; p.ab = u; p.ld_ab = ld_u;
+  return dispatch_gemm<EPI_GELU_BWD>(dY, W2, ldy, ldw, 0, 1, du, nullptr, ld_du, p, (cudaStream_t)stream);
 }
 
 namespace egom2p {

@@ -1,4 +1,5 @@
-// LayerNorm without bias (egom2p_utils.py:118-133), fp32 statistics. One warp per row, row held in registers,
+// LayerNorm without bias (egom2p_utils.py:118-133) and, as a compile-time variant, nn.LayerNorm with a learnable bias (the
+// GELU / bias family, egom2p_model.py:882-978); fp32 statistics. One warp per row, row held in registers,
 // 16-byte vector loads/stores. HBM-bound: fwd moves 4*D bytes in + 2*D (bf16) out per row.
 #include "common.cuh"
 
@@ -6,9 +7,9 @@ namespace egom2p {
 
 constexpr int kLnMaxVec = 16;  // float4 per lane -> dim <= 2048
 
-template <int NV>
+template <int NV, bool kBias>
 __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w,
-                                                     int64_t rows, int dim, float eps, uint16_t* __restrict__ yb,
+                                                     const float* __restrict__ bias, int64_t rows, int dim, float eps, uint16_t* __restrict__ yb,
                                                      float* __restrict__ yf, float* __restrict__ mean_out,
                                                      float* __restrict__ rstd_out) {
   const int64_t row = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
@@ -52,6 +53,10 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
       o.y = (v[j].y - mean) * rstd * g.y;
       o.z = (v[j].z - mean) * rstd * g.z;
       o.w = (v[j].w - mean) * rstd * g.w;
+      if (kBias) {
+        const float4 b = __ldg(reinterpret_cast<const float4*>(bias) + i);
+        o.x += b.x; o.y += b.y; o.z += b.z; o.w += b.w;
+      }
       if (yf) reinterpret_cast<float4*>(yf + row * dim)[i] = o;
       if (yb) {
         uint2 pk;
@@ -63,7 +68,7 @@ __global__ void __launch_bounds__(256) ln_fwd_kernel(const float* __restrict__ x
   }
 }
 
-// dx = rstd * (g - mean(g) - xhat * mean(g * xhat)), g = dy * w ; dw += sum_rows dy * xhat.
+// dx = rstd * (g - mean(g) - xhat * mean(g * xhat)), g = dy * w ; dw += sum_rows dy * xhat ; (kBias) db += sum_rows dy.
 // Each warp walks rows [row0 + warp, ...) with stride 8 inside its CTA's row chunk and keeps per-lane dw partials.
 // Only the raw x / dy registers stay live across the two warp reductions (xhat and g are recomputed), which keeps the
 // kernel at <= 80 registers -> 3 CTAs (24 warps) per SM to cover the load -> reduce -> store latency chain.
@@ -83,13 +88,14 @@ template <> struct DyVec<false> {
   __device__ __forceinline__ float4 get() const { return raw; }
 };
 
-template <bool kDyBf16, int NV>
+template <bool kDyBf16, int NV, bool kBias>
 __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__ dy_, const float* __restrict__ x,
                                                         const float* __restrict__ w, const float* __restrict__ mean,
                                                         const float* __restrict__ rstd, const float* __restrict__ dx_in,
                                                         int64_t rows, int dim, int rows_per_cta, float* __restrict__ dx_out,
-                                                        uint16_t* __restrict__ dx_bf16, float* __restrict__ dw) {
-  extern __shared__ float s_dw[];  // 4 warps x dim
+                                                        uint16_t* __restrict__ dx_bf16, float* __restrict__ dw,
+                                                        float* __restrict__ db) {
+  extern __shared__ float s_dw[];  // 4 warps x dim (kBias: then 4 warps x dim of db partials)
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int D4 = dim >> 2;
   const int64_t r0 = (int64_t)blockIdx.x * rows_per_cta;
@@ -97,6 +103,12 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
   float4 acc[NV];
 #pragma unroll
   for (int j = 0; j < NV; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  // kBias: the d_bias partials live in this warp's own shared-memory row (only its lanes touch it, each lane its own
+  // columns), not in registers -- a second register accumulator spills at dim 768 under the 128-register bound.
+  float4* s_db = reinterpret_cast<float4*>(s_dw + (4 + warp) * dim);
+  if (kBias) {
+    for (int i = lane; i < D4; i += 32) s_db[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
   const float4* wr = reinterpret_cast<const float4*>(w);
   for (int64_t row = r0 + warp; row < r1; row += 4) {
     const float mu = mean[row], rs = rstd[row];
@@ -121,6 +133,11 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
         const float4 d = dvr[j].get();
         const float hx = (xv[j].x - mu) * rs, hy = (xv[j].y - mu) * rs, hz = (xv[j].z - mu) * rs, hw = (xv[j].w - mu) * rs;
         acc[j].x += d.x * hx; acc[j].y += d.y * hy; acc[j].z += d.z * hz; acc[j].w += d.w * hw;
+        if (kBias) {
+          float4 t = s_db[i];
+          t.x += d.x; t.y += d.y; t.z += d.z; t.w += d.w;
+          s_db[i] = t;
+        }
         const float gx = d.x * wv.x, gy = d.y * wv.y, gz = d.z * wv.z, gw = d.w * wv.w;
         s1 += (gx + gy) + (gz + gw);
         s2 += (gx * hx + gy * hy) + (gz * hz + gw * hw);
@@ -155,7 +172,7 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
       }
     }
   }
-  if (!dw) return;
+  if (!kBias && !dw) return;
 #pragma unroll
   for (int j = 0; j < NV; ++j) {
     const int i = lane + j * 32;
@@ -166,49 +183,81 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
     float t = 0.f;
 #pragma unroll
     for (int wi = 0; wi < 4; ++wi) t += s_dw[wi * dim + c];
-    atomicAdd(dw + c, t);
+    if (!kBias || dw) atomicAdd(dw + c, t);
+    if (kBias) {
+      float tb = 0.f;
+#pragma unroll
+      for (int wi = 4; wi < 8; ++wi) tb += s_dw[wi * dim + c];
+      atomicAdd(db + c, tb);
+    }
   }
 }
 
 }  // namespace egom2p
 
-extern "C" int egom2p_layernorm_fwd(const float* x, const float* weight, int64_t rows, int32_t dim, float eps,
-                                    uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream) {
-  using namespace egom2p;
-  EGO_REQUIRE(x && weight && rows > 0, "layernorm_fwd: null input");
+namespace egom2p {
+template <bool kBias>
+static int layernorm_fwd(const float* x, const float* weight, const float* bias, int64_t rows, int32_t dim, float eps,
+                         uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream) {
+  EGO_REQUIRE(x && weight && rows > 0 && (!kBias || bias), "layernorm_fwd: null input");
   EGO_REQUIRE(dim % 4 == 0 && dim > 0 && dim <= kLnMaxVec * 128, "layernorm_fwd: dim %d unsupported (multiple of 4, <= %d)", dim, kLnMaxVec * 128);
   EGO_REQUIRE(y_bf16 || y_f32, "layernorm_fwd: no output");
   const int nv = (dim / 4 + 31) / 32;
-#define EGO_LN_FWD(NV) ln_fwd_kernel<NV><<<(unsigned)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(x, weight, rows, dim, eps, y_bf16, y_f32, mean, rstd)
+#define EGO_LN_FWD(NV) ln_fwd_kernel<NV, kBias><<<(unsigned)((rows + 7) / 8), 256, 0, (cudaStream_t)stream>>>(x, weight, bias, rows, dim, eps, y_bf16, y_f32, mean, rstd)
   if (nv <= 2) EGO_LN_FWD(2); else if (nv <= 3) EGO_LN_FWD(3); else if (nv <= 4) EGO_LN_FWD(4); else if (nv <= 6) EGO_LN_FWD(6);
   else if (nv <= 8) EGO_LN_FWD(8); else EGO_LN_FWD(16);
 #undef EGO_LN_FWD
   return check_launch("layernorm_fwd");
 }
 
-extern "C" int egom2p_layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
-                                    const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
-                                    float* dx_out, uint16_t* dx_bf16, float* d_weight, void* stream) {
-  using namespace egom2p;
+template <bool kBias>
+static int layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight, const float* mean,
+                         const float* rstd, const float* dx_in, int64_t rows, int32_t dim, float* dx_out, uint16_t* dx_bf16,
+                         float* d_weight, float* d_bias, void* stream) {
   EGO_REQUIRE((dy_bf16 != nullptr) != (dy_f32 != nullptr), "layernorm_bwd: exactly one of dy_bf16 / dy_f32");
-  EGO_REQUIRE(x && weight && mean && rstd && dx_out && rows > 0, "layernorm_bwd: null argument");
+  EGO_REQUIRE(x && weight && mean && rstd && dx_out && rows > 0 && (!kBias || d_bias), "layernorm_bwd: null argument");
   EGO_REQUIRE(dim % 4 == 0 && dim > 0 && dim <= kLnMaxVec * 128, "layernorm_bwd: dim %d unsupported", dim);
   const int rows_per_cta = 16;
   const unsigned grid = (unsigned)((rows + rows_per_cta - 1) / rows_per_cta);
-  const size_t smem = (size_t)4 * dim * sizeof(float);
+  const size_t smem = (size_t)(kBias ? 8 : 4) * dim * sizeof(float);
   const int nv = (dim / 4 + 31) / 32;
 #define EGO_LN_BWD(NV)                                                                                                  \
   do {                                                                                                                  \
     if (dy_bf16) {                                                                                                      \
-      if (smem > 48 * 1024) cudaFuncSetAttribute(ln_bwd_kernel<true, NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-      ln_bwd_kernel<true, NV><<<grid, 128, smem, (cudaStream_t)stream>>>(dy_bf16, x, weight, mean, rstd, dx_in, rows, dim, rows_per_cta, dx_out, dx_bf16, d_weight); \
+      if (smem > 48 * 1024) cudaFuncSetAttribute(ln_bwd_kernel<true, NV, kBias>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      ln_bwd_kernel<true, NV, kBias><<<grid, 128, smem, (cudaStream_t)stream>>>(dy_bf16, x, weight, mean, rstd, dx_in, rows, dim, rows_per_cta, dx_out, dx_bf16, d_weight, d_bias); \
     } else {                                                                                                            \
-      if (smem > 48 * 1024) cudaFuncSetAttribute(ln_bwd_kernel<false, NV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-      ln_bwd_kernel<false, NV><<<grid, 128, smem, (cudaStream_t)stream>>>(dy_f32, x, weight, mean, rstd, dx_in, rows, dim, rows_per_cta, dx_out, dx_bf16, d_weight); \
+      if (smem > 48 * 1024) cudaFuncSetAttribute(ln_bwd_kernel<false, NV, kBias>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      ln_bwd_kernel<false, NV, kBias><<<grid, 128, smem, (cudaStream_t)stream>>>(dy_f32, x, weight, mean, rstd, dx_in, rows, dim, rows_per_cta, dx_out, dx_bf16, d_weight, d_bias); \
     }                                                                                                                   \
   } while (0)
   if (nv <= 2) EGO_LN_BWD(2); else if (nv <= 3) EGO_LN_BWD(3); else if (nv <= 4) EGO_LN_BWD(4); else if (nv <= 6) EGO_LN_BWD(6);
   else if (nv <= 8) EGO_LN_BWD(8); else EGO_LN_BWD(16);
 #undef EGO_LN_BWD
   return check_launch("layernorm_bwd");
+}
+}  // namespace egom2p
+
+extern "C" int egom2p_layernorm_fwd(const float* x, const float* weight, int64_t rows, int32_t dim, float eps,
+                                    uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream) {
+  return egom2p::layernorm_fwd<false>(x, weight, nullptr, rows, dim, eps, y_bf16, y_f32, mean, rstd, stream);
+}
+
+extern "C" int egom2p_layernorm_bias_fwd(const float* x, const float* weight, const float* bias, int64_t rows, int32_t dim,
+                                         float eps, uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream) {
+  return egom2p::layernorm_fwd<true>(x, weight, bias, rows, dim, eps, y_bf16, y_f32, mean, rstd, stream);
+}
+
+extern "C" int egom2p_layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
+                                    const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
+                                    float* dx_out, uint16_t* dx_bf16, float* d_weight, void* stream) {
+  return egom2p::layernorm_bwd<false>(dy_bf16, dy_f32, x, weight, mean, rstd, dx_in, rows, dim, dx_out, dx_bf16, d_weight,
+                                      nullptr, stream);
+}
+
+extern "C" int egom2p_layernorm_bias_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
+                                         const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
+                                         float* dx_out, uint16_t* dx_bf16, float* d_weight, float* d_bias, void* stream) {
+  return egom2p::layernorm_bwd<true>(dy_bf16, dy_f32, x, weight, mean, rstd, dx_in, rows, dim, dx_out, dx_bf16, d_weight,
+                                     d_bias, stream);
 }

@@ -9,8 +9,9 @@ forward_logits / decoder_proj_context / mask_token / cat_encoder_tensors` for th
 range-masked flash attention, tcgen05 GEMMs with fused epilogues, vocabulary head fused with cross-entropy.
 Autograd nodes are per block, so DDP's bucketed all-reduce overlaps with backward exactly as for the reference.
 
-Scope: the swiglu / no-bias family (ego-b and its tiny/small/large siblings). Other registered variants of the
-reference (GELU+bias, QK-norm) are not built here and raise NotImplementedError at construction.
+Scope: the swiglu / no-bias family (ego-b and its tiny/small siblings) and the GELU / bias family (egom2p_*_gelu: biases
+on every Linear and LayerNorm, MLP fc2(GELU(fc1 x)), egom2p_model.py:882-978), both at head dim 64. Other registered
+variants of the reference (QK-norm, large / xlarge) are not built here and raise NotImplementedError at construction.
 """
 from __future__ import annotations
 
@@ -29,22 +30,33 @@ bf16, f32 = torch.bfloat16, torch.float32
 
 # =============================================================================================== parameter containers
 class LayerNorm(nn.Module):
-    """Parameter container mirroring egom2p_utils.LayerNorm (weight + zero `bias` buffer when bias=False)."""
+    """Parameter container mirroring egom2p_utils.LayerNorm (weight + zero `bias` buffer when bias=False) and, with
+    bias=True, nn.LayerNorm (weight + `bias` Parameter) of the GELU / bias family."""
 
     def __init__(self, normalized_shape: int, eps=1e-5, bias=True):
         super().__init__()
         self.eps = eps
         self.weight = nn.Parameter(torch.ones(normalized_shape))
         if bias:
-            raise NotImplementedError("egom2p_b200 builds the no-bias LayerNorm family only")
-        self.register_buffer("bias", torch.zeros(normalized_shape))
+            self.bias = nn.Parameter(torch.zeros(normalized_shape))
+        else:
+            self.register_buffer("bias", torch.zeros(normalized_shape))
         self.normalized_shape = (normalized_shape,)
 
     def forward(self, x):
         shape = x.shape
         _, y, _, _ = ops.layernorm_fwd(x.reshape(-1, shape[-1]).float().contiguous(), self.weight.detach(), self.eps,
-                                       out_bf16=False, out_f32=True, save_stats=False)
+                                       out_bf16=False, out_f32=True, save_stats=False, bias=_ln_bias(self))
         return y.reshape(shape)
+
+
+def _ln_bias(norm: nn.Module) -> Optional[torch.Tensor]:
+    """The learnable bias of a LayerNorm (detached), None for the zero buffer of the no-bias family."""
+    return norm.bias.detach() if isinstance(norm.bias, nn.Parameter) else None
+
+
+def _det(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    return None if t is None else t.detach()
 
 
 class _Linear(nn.Linear):
@@ -67,44 +79,53 @@ class GatedMlp(nn.Module):
         self.fc3 = _Linear(dim, hidden, bias=False)
 
 
+class Mlp(nn.Module):
+    """fc2(GELU(fc1 x)) with biases (egom2p_utils.py Mlp, the GELU / bias family)."""
+
+    def __init__(self, dim, hidden):
+        super().__init__()
+        self.fc1 = _Linear(dim, hidden, bias=True)
+        self.fc2 = _Linear(hidden, dim, bias=True)
+
+
 class Attention(nn.Module):
-    def __init__(self, dim, num_heads):
+    def __init__(self, dim, num_heads, bias=False):
         super().__init__()
         self.num_heads = num_heads
         self.scale = (dim // num_heads) ** -0.5
-        self.qkv = _Linear(dim, dim * 3, bias=False)
-        self.proj = _Linear(dim, dim, bias=False)
+        self.qkv = _Linear(dim, dim * 3, bias=bias)
+        self.proj = _Linear(dim, dim, bias=bias)
 
 
 class CrossAttention(nn.Module):
-    def __init__(self, dim, num_heads):
+    def __init__(self, dim, num_heads, bias=False):
         super().__init__()
         self.num_heads = num_heads
         self.scale = (dim // num_heads) ** -0.5
-        self.q = _Linear(dim, dim, bias=False)
-        self.kv = _Linear(dim, dim * 2, bias=False)
-        self.proj = _Linear(dim, dim, bias=False)
+        self.q = _Linear(dim, dim, bias=bias)
+        self.kv = _Linear(dim, dim * 2, bias=bias)
+        self.proj = _Linear(dim, dim, bias=bias)
 
 
 class Block(nn.Module):
-    def __init__(self, dim, num_heads, mlp_ratio, norm_layer):
+    def __init__(self, dim, num_heads, mlp_ratio, norm_layer, gelu=False):
         super().__init__()
         self.norm1 = norm_layer(dim)
-        self.attn = Attention(dim, num_heads)
+        self.attn = Attention(dim, num_heads, bias=gelu)
         self.norm2 = norm_layer(dim)
-        self.mlp = GatedMlp(dim, int(dim * mlp_ratio))
+        self.mlp = Mlp(dim, int(dim * mlp_ratio)) if gelu else GatedMlp(dim, int(dim * mlp_ratio))
 
 
 class DecoderBlock(nn.Module):
-    def __init__(self, dim, num_heads, mlp_ratio, norm_layer):
+    def __init__(self, dim, num_heads, mlp_ratio, norm_layer, gelu=False):
         super().__init__()
         self.norm1 = norm_layer(dim)
-        self.self_attn = Attention(dim, num_heads)
-        self.cross_attn = CrossAttention(dim, num_heads)
+        self.self_attn = Attention(dim, num_heads, bias=gelu)
+        self.cross_attn = CrossAttention(dim, num_heads, bias=gelu)
         self.query_norm = norm_layer(dim)
         self.context_norm = norm_layer(dim)
         self.norm2 = norm_layer(dim)
-        self.mlp = GatedMlp(dim, int(dim * mlp_ratio))
+        self.mlp = Mlp(dim, int(dim * mlp_ratio)) if gelu else GatedMlp(dim, int(dim * mlp_ratio))
 
 
 # =============================================================================================== kernels glue
@@ -190,16 +211,19 @@ def _mlp_bwd(dx2, x1, n2w, w13, w2, saved):
     return dx1, dx1b, dn2w, dw13, dw2
 
 
-def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs=None):
+def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs=None, bias=None):
+    """bias: (norm1 bias, qkv bias, proj bias) of the GELU / bias family, fp32; None for the no-bias family."""
     D = x.shape[-1]
-    h1, _, mean1, rstd1 = ops.layernorm_fwd(x, n1w, eps)
-    qkv = ops.linear_fwd(h1, wqkv)
+    n1b, bqkv, bproj = bias if bias is not None else (None, None, None)
+    h1, _, mean1, rstd1 = ops.layernorm_fwd(x, n1w, eps, bias=n1b)
+    qkv = ops.linear_fwd(h1, wqkv, bias=bqkv)
     o, lse = ops.attn_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], B, H, L, L, meta=meta, pairs=pairs)
-    x1 = ops.linear_fwd(o, wproj, addend=x, out_dtype=f32)
+    x1 = ops.linear_fwd(o, wproj, bias=bproj, addend=x, out_dtype=f32)
     return x1, (mean1, rstd1, h1, qkv, o, lse)
 
 
-def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs=None):
+def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs=None, biased=False):
+    """Returns dx, dn1w, dwqkv, dwproj and, when biased, (dn1b, dbqkv, dbproj) (else None)."""
     mean1, rstd1, h1, qkv, o, lse = saved
     D = x.shape[-1]
     dwproj = ops.linear_wgrad(dx1b, o)
@@ -210,8 +234,88 @@ def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs=N
     dwqkv = ops.linear_wgrad(dqkv, h1)
     dh1 = ops.linear_dgrad(dqkv, wqkv)
     dn1w = _zeros(n1w.numel(), x.device)
-    dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True)
-    return _with_bf16(dx, dxb), dn1w, dwqkv, dwproj
+    extra = None
+    if biased:
+        extra = (_zeros(n1w.numel(), x.device), ops.colsum_bf16(dqkv), ops.colsum_bf16(dx1b))
+    dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True,
+                                d_bias=extra[0] if biased else None)
+    return _with_bf16(dx, dxb), dn1w, dwqkv, dwproj, extra
+
+
+def _gelu_mlp_fwd(x1, n2w, n2b, w1, b1, w2, b2, eps):
+    h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps, bias=n2b)
+    u, a = ops.gemm_gelu_fwd(h2, w1, b1)   # fc1 GEMM with + b1 and GELU in its epilogue
+    x2 = ops.linear_fwd(a, w2, bias=b2, addend=x1, out_dtype=f32)
+    return x2, (mean2, rstd2, h2, u, a)
+
+
+def _gelu_mlp_bwd(dx2, x1, n2w, w1, w2, saved):
+    """Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b, dw1, db1, dw2, db2."""
+    mean2, rstd2, h2, u, a = saved
+    dev = dx2.device
+    dx2b = _bf16_of(dx2)
+    dw2 = ops.linear_wgrad(dx2b, a)
+    db2 = ops.colsum_bf16(dx2b)
+    du = ops.gemm_gelu_bwd(dx2b, w2, u)   # fc2 dgrad with GELU'(u) in its epilogue
+    dw1 = ops.linear_wgrad(du, h2)
+    db1 = ops.colsum_bf16(du)
+    dh2 = ops.linear_dgrad(du, w1)
+    dn2w, dn2b = _zeros(n2w.numel(), dev), _zeros(n2w.numel(), dev)
+    dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True, d_bias=dn2b)
+    return dx1, dx1b, dn2w, dn2b, dw1, db1, dw2, db2
+
+
+def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias=None):
+    """y2 = y1 + cross_attn(query_norm y1, context_norm context). bias: (query_norm, context_norm, q, kv, proj biases) or None."""
+    D = y1.shape[-1]
+    qnb, cnb, bq, bkv, bxproj = bias if bias is not None else (None,) * 5
+    hq, _, meanq, rstdq = ops.layernorm_fwd(y1, qnw, g.eps, bias=qnb)
+    q = ops.linear_fwd(hq, wq, bias=bq)
+    hc, _, meanc, rstdc = ops.layernorm_fwd(context, cnw, g.eps, bias=cnb)
+    kv = ops.linear_fwd(hc, wkv, bias=bkv)
+    o2, lse2 = ops.attn_fwd(q, kv[:, :D], kv[:, D:], g.B, g.H, g.M, g.N, meta=g.m_x, pairs=g.p_x)
+    y2 = ops.linear_fwd(o2, wxproj, bias=bxproj, addend=y1, out_dtype=f32)
+    return y2, (meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2)
+
+
+def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, biased=False):
+    """Backward of _cross_fwd. Returns dy1, dy1b, dctx (None unless this block returns the summed context gradient),
+    dqnw, dcnw, dwq, dwkv, dwxproj and, when biased, (dqnb, dcnb, dbq, dbkv, dbxproj) (else None)."""
+    meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2 = saved
+    D = y1.shape[-1]
+    dev = y1.device
+    dwxproj = ops.linear_wgrad(dy2b, o2)
+    do2 = ops.linear_dgrad(dy2b, wxproj)
+    dq = torch.empty_like(q)
+    dkv = torch.empty_like(kv)
+    ops.attn_bwd(q, kv[:, :D], kv[:, D:], o2, do2, lse2, g.B, g.H, g.M, g.N, dq, dkv[:, :D], dkv[:, D:], meta=g.m_x, pairs=g.p_x)
+    dwq = ops.linear_wgrad(dq, hq)
+    dhq = ops.linear_dgrad(dq, wq)
+    dwkv = ops.linear_wgrad(dkv, hc)
+    dhc = ops.linear_dgrad(dkv, wkv)
+    dqnw, dcnw = _zeros(D, dev), _zeros(D, dev)
+    extra = None
+    if biased:
+        extra = (_zeros(D, dev), _zeros(D, dev), ops.colsum_bf16(dq), ops.colsum_bf16(dkv), ops.colsum_bf16(dy2b))
+    dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True,
+                                  d_bias=extra[0] if biased else None)
+    # All decoder blocks read the same `context`: instead of letting autograd add twelve (B*N, D) fp32 gradients pairwise,
+    # each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block that runs last
+    # returns it. Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
+    acc = g.dctx_acc
+    chained = g.ctx_users > 0 and (acc is None or (acc[0] == ctx_key and acc[1].shape == context.shape))
+    last = chained and g.ctx_users == 1
+    dctx, dctxb = ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, dx_in=acc[1] if (chained and acc is not None) else None,
+                                    d_weight=dcnw, want_bf16=last, d_bias=extra[1] if biased else None)
+    if chained:
+        g.ctx_users -= 1
+        if last:
+            g.dctx_acc = None
+            dctx = _with_bf16(dctx, dctxb)
+        else:
+            g.dctx_acc = (ctx_key, dctx)
+            dctx = None
+    return dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, extra
 
 
 class _EncoderBlockFn(torch.autograd.Function):
@@ -237,7 +341,7 @@ class _EncoderBlockFn(torch.autograd.Function):
         g = ctx.geom
         dx2 = dx2.contiguous()
         dx1, dx1b, dn2w, dw13, dw2 = _mlp_bwd(dx2, x1, n2w, w13, w2, sm)
-        dx, dn1w, dwqkv, dwproj = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc)
+        dx, dn1w, dwqkv, dwproj, _ = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc)
         F = ctx.F
         d1, d3 = _split_w13_grad(dw13, F)
         return dx, dn1w, dwqkv, dwproj, dn2w, d1, dw2[:, :F], d3, None, None
@@ -252,73 +356,104 @@ class _DecoderBlockFn(torch.autograd.Function):
         g = geom
         D = y.shape[-1]
         y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec)
-        hq, _, meanq, rstdq = ops.layernorm_fwd(y1, qnw, g.eps)
-        q = ops.linear_fwd(hq, wq)
-        hc, _, meanc, rstdc = ops.layernorm_fwd(context, cnw, g.eps)
-        kv = ops.linear_fwd(hc, wkv)
-        o2, lse2 = ops.attn_fwd(q, kv[:, :D], kv[:, D:], g.B, g.H, g.M, g.N, meta=g.m_x, pairs=g.p_x)
-        y2 = ops.linear_fwd(o2, wxproj, addend=y1, out_dtype=f32)
+        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g)
         y3, sm = _mlp_fwd(y2, n2w, w13, w2, g.eps)
         ctx.geom, ctx.wb, ctx.F = geom, wb, fc1_w.shape[0]
         ctx.op_epoch = geom.epoch_ref[0]
         ctx.ctx_key = context.data_ptr()
         g.ctx_users += 1
-        ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2,
-                              *sa, *sm)
+        ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, *sx, *sa, *sm)
         return y3
 
     @staticmethod
     def backward(ctx, dy3):
         _GRAD_GEN[0] += 1
         _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
-        (y, context, n1w, qnw, cnw, n2w, y1, y2, meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2, *rest) = ctx.saved_tensors
-        sa, sm = rest[:6], rest[6:]
+        (y, context, n1w, qnw, cnw, n2w, y1, y2, *rest) = ctx.saved_tensors
+        sx, sa, sm = rest[:10], rest[10:16], rest[16:]
         wqkv, wsproj, wq, wkv, wxproj, w13, w2 = ctx.wb
         g = ctx.geom
-        D = y.shape[-1]
-        dev = y.device
         dy3 = dy3.contiguous()
         dy2, dy2b, dn2w, dw13, dw2 = _mlp_bwd(dy3, y2, n2w, w13, w2, sm)
-        # cross attention
-        dwxproj = ops.linear_wgrad(dy2b, o2)
-        do2 = ops.linear_dgrad(dy2b, wxproj)
-        dq = torch.empty_like(q)
-        dkv = torch.empty_like(kv)
-        ops.attn_bwd(q, kv[:, :D], kv[:, D:], o2, do2, lse2, g.B, g.H, g.M, g.N, dq, dkv[:, :D], dkv[:, D:], meta=g.m_x, pairs=g.p_x)
-        dwq = ops.linear_wgrad(dq, hq)
-        dhq = ops.linear_dgrad(dq, wq)
-        dwkv = ops.linear_wgrad(dkv, hc)
-        dhc = ops.linear_dgrad(dkv, wkv)
-        dqnw, dcnw = _zeros(D, dev), _zeros(D, dev)
-        dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True)
-        # All decoder blocks read the same `context`: instead of letting autograd add twelve (B*N, D) fp32 gradients pairwise,
-        # each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block that runs last
-        # returns it. Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
-        acc = g.dctx_acc
-        chained = g.ctx_users > 0 and (acc is None or (acc[0] == ctx.ctx_key and acc[1].shape == context.shape))
-        last = chained and g.ctx_users == 1
-        dctx, dctxb = ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, dx_in=acc[1] if (chained and acc is not None) else None,
-                                        d_weight=dcnw, want_bf16=last)
-        if chained:
-            g.ctx_users -= 1
-            if last:
-                g.dctx_acc = None
-                dctx = _with_bf16(dctx, dctxb)
-            else:
-                g.dctx_acc = (ctx.ctx_key, dctx)
-                dctx = None
-        dy, dn1w, dwqkv, dwsproj = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec)
+        dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, _ = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv,
+                                                                       wxproj, sx)
+        dy, dn1w, dwqkv, dwsproj, _ = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec)
         F = ctx.F
         d1, d3 = _split_w13_grad(dw13, F)
         return (dy, dctx, dn1w, dwqkv, dwsproj, dqnw, dcnw, dwq, dwkv, dwxproj, dn2w, d1, dw2[:, :F], d3, None, None)
 
 
-class _ContextFn(torch.autograd.Function):
-    """context = decoder_proj_context(encoder_norm(x)) + encoder_emb -- egom2p_model.py:499,722."""
+class _GeluEncoderBlockFn(torch.autograd.Function):
+    """GELU / bias family: x + attn(norm1 x) then + fc2(GELU(fc1 norm2 .)), every Linear and LayerNorm with a bias."""
 
     @staticmethod
-    def forward(ctx, x, enc_emb, norm_w, proj_w, proj_b, wb, eps, epoch_ref):
-        h, _, mean, rstd = ops.layernorm_fwd(x, norm_w, eps)
+    def forward(ctx, x, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, wb, geom):
+        wqkv, wproj, w1, w2 = wb
+        g = geom
+        x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, g.B, g.N, g.H, g.m_enc, g.eps, g.p_enc, bias=(n1b, qkv_b, proj_b))
+        x2, sm = _gelu_mlp_fwd(x1, n2w, n2b, w1, fc1_b, w2, fc2_b, g.eps)
+        ctx.geom, ctx.wb = geom, wb
+        ctx.op_epoch = geom.epoch_ref[0]
+        ctx.save_for_backward(x, n1w, n2w, x1, *sa, *sm)
+        return x2
+
+    @staticmethod
+    def backward(ctx, dx2):
+        _GRAD_GEN[0] += 1
+        _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
+        x, n1w, n2w, x1, *rest = ctx.saved_tensors
+        sa, sm = rest[:6], rest[6:]
+        wqkv, wproj, w1, w2 = ctx.wb
+        g = ctx.geom
+        dx1, dx1b, dn2w, dn2b, dw1, db1, dw2, db2 = _gelu_mlp_bwd(dx2.contiguous(), x1, n2w, w1, w2, sm)
+        dx, dn1w, dwqkv, dwproj, (dn1b, dbqkv, dbproj) = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H,
+                                                                        g.m_enc, g.p_enc, biased=True)
+        return dx, dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, dn2w, dn2b, dw1, db1, dw2, db2, None, None
+
+
+class _GeluDecoderBlockFn(torch.autograd.Function):
+    """GELU / bias family: self-attn -> cross-attn(query_norm y, context_norm ctx) -> GELU MLP, all with biases."""
+
+    @staticmethod
+    def forward(ctx, y, context, n1w, n1b, qkv_w, qkv_b, sproj_w, sproj_b, qnw, qnb, cnw, cnb, q_w, q_b, kv_w, kv_b,
+                xproj_w, xproj_b, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, wb, geom):
+        wqkv, wsproj, wq, wkv, wxproj, w1, w2 = wb
+        g = geom
+        y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec, bias=(n1b, qkv_b, sproj_b))
+        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias=(qnb, cnb, q_b, kv_b, xproj_b))
+        y3, sm = _gelu_mlp_fwd(y2, n2w, n2b, w1, fc1_b, w2, fc2_b, g.eps)
+        ctx.geom, ctx.wb = geom, wb
+        ctx.op_epoch = geom.epoch_ref[0]
+        ctx.ctx_key = context.data_ptr()
+        g.ctx_users += 1
+        ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, *sx, *sa, *sm)
+        return y3
+
+    @staticmethod
+    def backward(ctx, dy3):
+        _GRAD_GEN[0] += 1
+        _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
+        (y, context, n1w, qnw, cnw, n2w, y1, y2, *rest) = ctx.saved_tensors
+        sx, sa, sm = rest[:10], rest[10:16], rest[16:]
+        wqkv, wsproj, wq, wkv, wxproj, w1, w2 = ctx.wb
+        g = ctx.geom
+        dy2, dy2b, dn2w, dn2b, dw1, db1, dw2, db2 = _gelu_mlp_bwd(dy3.contiguous(), y2, n2w, w1, w2, sm)
+        dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, (dqnb, dcnb, dbq, dbkv, dbxproj) = _cross_bwd(
+            g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, biased=True)
+        dy, dn1w, dwqkv, dwsproj, (dn1b, dbqkv, dbsproj) = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H,
+                                                                          g.m_dec, g.p_dec, biased=True)
+        return (dy, dctx, dn1w, dn1b, dwqkv, dbqkv, dwsproj, dbsproj, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj,
+                dbxproj, dn2w, dn2b, dw1, db1, dw2, db2, None, None)
+
+
+class _ContextFn(torch.autograd.Function):
+    """context = decoder_proj_context(encoder_norm(x)) + encoder_emb -- egom2p_model.py:499,722. norm_b: encoder_norm's
+    bias (GELU / bias family) or None."""
+
+    @staticmethod
+    def forward(ctx, x, enc_emb, norm_w, norm_b, proj_w, proj_b, wb, eps, epoch_ref):
+        h, _, mean, rstd = ops.layernorm_fwd(x, norm_w, eps, bias=norm_b)
+        ctx.has_nb = norm_b is not None
         context = ops.linear_fwd(h, wb, bias=proj_b, addend=enc_emb, out_dtype=f32)
         ctx.wb = wb
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
@@ -336,8 +471,9 @@ class _ContextFn(torch.autograd.Function):
         db = ops.colsum(dctx, _zeros(dctx.shape[1], dctx.device))
         dh = ops.linear_dgrad(dcb, ctx.wb)
         dnw = _zeros(norm_w.numel(), x.device)
-        dx, dxb = ops.layernorm_bwd(dh, x, norm_w, mean, rstd, d_weight=dnw, want_bf16=True)
-        return _with_bf16(dx, dxb), dctx, dnw, dw, db, None, None, None
+        dnb = _zeros(norm_w.numel(), x.device) if ctx.has_nb else None
+        dx, dxb = ops.layernorm_bwd(dh, x, norm_w, mean, rstd, d_weight=dnw, want_bf16=True, d_bias=dnb)
+        return _with_bf16(dx, dxb), dctx, dnw, dnb, dw, db, None, None, None
 
 
 class _EmbedFn(torch.autograd.Function):
@@ -390,9 +526,10 @@ class _HeadLossFn(torch.autograd.Function):
     CHUNK = 8192
 
     @staticmethod
-    def forward(ctx, y, norm_w, rows, targets, wbs, eps, epoch_ref, *head_w):
+    def forward(ctx, y, norm_w, norm_b, rows, targets, wbs, eps, epoch_ref, *head_w):
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
-        yn, _, mean, rstd = ops.layernorm_fwd(y, norm_w, eps)
+        ctx.has_nb = norm_b is not None
+        yn, _, mean, rstd = ops.layernorm_fwd(y, norm_w, eps, bias=norm_b)
         losses, lses, yms = [], [], []
         for idx, tgt, wb in zip(rows, targets, wbs):
             if idx.numel() == 0:
@@ -436,8 +573,9 @@ class _HeadLossFn(torch.autograd.Function):
             ops.scatter_rows_f32(dym, idx, dyn)
             dws.append(dw)
         dnw = _zeros(D, dev)
-        dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=True)
-        return (_with_bf16(dy, dyb), dnw, None, None, None, None, None, *dws)
+        dnb = _zeros(D, dev) if ctx.has_nb else None
+        dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=True, d_bias=dnb)
+        return (_with_bf16(dy, dyb), dnw, dnb, None, None, None, None, None, *dws)
 
 
 # =============================================================================================== the module
@@ -469,8 +607,11 @@ class EgoM2P(nn.Module):
                  use_act_checkpoint: bool = False,
                  share_modality_embeddings: bool = True):
         super().__init__()
-        if qkv_bias or proj_bias or mlp_bias or not gated_mlp or qk_norm or act_layer is not nn.SiLU:
-            raise NotImplementedError("egom2p_b200 implements the swiglu / no-bias family (egom2p_*_swiglu_nobias)")
+        swiglu = not (qkv_bias or proj_bias or mlp_bias) and gated_mlp and act_layer is nn.SiLU
+        gelu = qkv_bias and proj_bias and mlp_bias and not gated_mlp and act_layer is nn.GELU
+        if qk_norm or not (swiglu or gelu):
+            raise NotImplementedError("egom2p_b200 implements the swiglu / no-bias family (egom2p_*_swiglu_nobias) and the "
+                                      "GELU / bias family (egom2p_*_gelu)")
         if drop_path_rate_encoder or drop_path_rate_decoder:
             raise NotImplementedError("drop_path > 0 is not built (the reference trains ego-b with 0)")
         if num_register_tokens:
@@ -484,8 +625,11 @@ class EgoM2P(nn.Module):
         self.use_act_checkpoint = use_act_checkpoint
         self.num_register_tokens = num_register_tokens
         eps_probe = norm_layer(4)
+        if gelu and not isinstance(getattr(eps_probe, "bias", None), nn.Parameter):
+            raise NotImplementedError("the GELU / bias family is built with LayerNorms that have a learnable bias (nn.LayerNorm)")
         self.eps = float(getattr(eps_probe, "eps", 1e-6))
-        norm = partial(LayerNorm, eps=self.eps, bias=False)  # same names/buffers as the reference's LayerNorm
+        self.gelu = bool(gelu)
+        norm = partial(LayerNorm, eps=self.eps, bias=self.gelu)  # same names/buffers as the reference's LayerNorm
 
         self.encoder_modalities = set(encoder_embeddings.keys())
         for emb in encoder_embeddings.values():
@@ -504,10 +648,10 @@ class EgoM2P(nn.Module):
         if share_modality_embeddings:
             self.share_modality_embeddings()
 
-        self.encoder = nn.ModuleList([Block(dim, num_heads, mlp_ratio, norm) for _ in range(encoder_depth)])
+        self.encoder = nn.ModuleList([Block(dim, num_heads, mlp_ratio, norm, self.gelu) for _ in range(encoder_depth)])
         self.encoder_norm = norm(dim)
         self.decoder_proj_context = _Linear(dim, dim)
-        self.decoder = nn.ModuleList([DecoderBlock(dim, num_heads, mlp_ratio, norm) for _ in range(decoder_depth)])
+        self.decoder = nn.ModuleList([DecoderBlock(dim, num_heads, mlp_ratio, norm, self.gelu) for _ in range(decoder_depth)])
         self.decoder_norm = norm(dim)
         self.mask_token = nn.Parameter(torch.zeros(1, 1, dim))
         nn.init.normal_(self.mask_token, std=self.init_std)
@@ -629,15 +773,57 @@ class EgoM2P(nn.Module):
 
     def _enc_weights(self, i: int):
         b = self.encoder[i]
+        if self.gelu:
+            return (self._bf16(("e", i, "qkv"), b.attn.qkv.weight), self._bf16(("e", i, "proj"), b.attn.proj.weight),
+                    self._bf16(("e", i, "w1"), b.mlp.fc1.weight), self._bf16(("e", i, "w2"), b.mlp.fc2.weight, pad32=True))
         return (self._bf16(("e", i, "qkv"), b.attn.qkv.weight), self._bf16(("e", i, "proj"), b.attn.proj.weight),
                 self._bf16(("e", i, "w13"), b.mlp.fc1.weight, b.mlp.fc3.weight), self._bf16(("e", i, "w2"), b.mlp.fc2.weight, pad32=True))
 
     def _dec_weights(self, i: int):
         b = self.decoder[i]
+        if self.gelu:
+            return (self._bf16(("d", i, "qkv"), b.self_attn.qkv.weight), self._bf16(("d", i, "sproj"), b.self_attn.proj.weight),
+                    self._bf16(("d", i, "q"), b.cross_attn.q.weight), self._bf16(("d", i, "kv"), b.cross_attn.kv.weight),
+                    self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight),
+                    self._bf16(("d", i, "w1"), b.mlp.fc1.weight), self._bf16(("d", i, "w2"), b.mlp.fc2.weight, pad32=True))
         return (self._bf16(("d", i, "qkv"), b.self_attn.qkv.weight), self._bf16(("d", i, "sproj"), b.self_attn.proj.weight),
                 self._bf16(("d", i, "q"), b.cross_attn.q.weight), self._bf16(("d", i, "kv"), b.cross_attn.kv.weight),
                 self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight),
                 self._bf16(("d", i, "w13"), b.mlp.fc1.weight, b.mlp.fc3.weight), self._bf16(("d", i, "w2"), b.mlp.fc2.weight, pad32=True))
+
+    # ------------------------------------------------------------------ block application (training and inference)
+    def _enc_block(self, i, blk, h, g):
+        if self.gelu:
+            a, m = blk.attn, blk.mlp
+            return _GeluEncoderBlockFn.apply(h, blk.norm1.weight, blk.norm1.bias, a.qkv.weight, a.qkv.bias, a.proj.weight, a.proj.bias,
+                                             blk.norm2.weight, blk.norm2.bias, m.fc1.weight, m.fc1.bias, m.fc2.weight, m.fc2.bias,
+                                             self._enc_weights(i), g)
+        return _EncoderBlockFn.apply(h, blk.norm1.weight, blk.attn.qkv.weight, blk.attn.proj.weight, blk.norm2.weight,
+                                     blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._enc_weights(i), g)
+
+    def _dec_block(self, i, blk, h, c, g):
+        if self.gelu:
+            sa, xa, m = blk.self_attn, blk.cross_attn, blk.mlp
+            return _GeluDecoderBlockFn.apply(h, c, blk.norm1.weight, blk.norm1.bias, sa.qkv.weight, sa.qkv.bias, sa.proj.weight,
+                                             sa.proj.bias, blk.query_norm.weight, blk.query_norm.bias, blk.context_norm.weight,
+                                             blk.context_norm.bias, xa.q.weight, xa.q.bias, xa.kv.weight, xa.kv.bias, xa.proj.weight,
+                                             xa.proj.bias, blk.norm2.weight, blk.norm2.bias, m.fc1.weight, m.fc1.bias, m.fc2.weight,
+                                             m.fc2.bias, self._dec_weights(i), g)
+        return _DecoderBlockFn.apply(h, c, blk.norm1.weight, blk.self_attn.qkv.weight, blk.self_attn.proj.weight,
+                                     blk.query_norm.weight, blk.context_norm.weight, blk.cross_attn.q.weight,
+                                     blk.cross_attn.kv.weight, blk.cross_attn.proj.weight, blk.norm2.weight,
+                                     blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._dec_weights(i), g)
+
+    def _attn_bias(self, attn: nn.Module, norm: nn.Module):
+        """(norm bias, qkv bias, proj bias) of a self-attention sub-block (detached) for _self_attn_fwd, None for swiglu."""
+        return (_ln_bias(norm), _det(attn.qkv.bias), _det(attn.proj.bias)) if self.gelu else None
+
+    def _mlp_infer(self, blk, x, wm, w2, eps):
+        """MLP sub-block without autograd (generation / sampler paths). wm: the fc1 | fc3 (swiglu) or fc1 (GELU) operand."""
+        if self.gelu:
+            return _gelu_mlp_fwd(x, blk.norm2.weight.detach(), _ln_bias(blk.norm2), wm, _det(blk.mlp.fc1.bias), w2,
+                                 _det(blk.mlp.fc2.bias), eps)[0]
+        return _mlp_fwd(x, blk.norm2.weight.detach(), wm, w2, eps)[0]
 
     # ------------------------------------------------------------------ sampler-facing pieces (reference :251-283,483-551)
     def cat_encoder_tensors(self, mod_dict):
@@ -685,8 +871,7 @@ class EgoM2P(nn.Module):
         g.build_meta(x.device)
         h = x.reshape(B * N, D).float().contiguous()
         for i, blk in enumerate(self.encoder):
-            h = _EncoderBlockFn.apply(h, blk.norm1.weight, blk.attn.qkv.weight, blk.attn.proj.weight, blk.norm2.weight,
-                                      blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._enc_weights(i), g)
+            h = self._enc_block(i, blk, h, g)
         return self.encoder_norm(h).reshape(B, N, D)
 
     def forward_decoder(self, y, context, encoder_mask, decoder_attention_mask):
@@ -700,24 +885,22 @@ class EgoM2P(nn.Module):
         c = context.reshape(B * N, D).float().contiguous() if N > 0 else torch.zeros(0, D, dtype=f32, device=y.device)
         if N == 0:
             # Unconditional branch of guided ROAR decoding (generate.py:793-802): no context token at all. Softmax over
-            # zero keys times an empty V is exactly 0 and the cross-attention projection has no bias, so every block
-            # reduces to self-attention + MLP (SURVEY.md A5). Inference only.
+            # zero keys times an empty V is exactly 0, so every block reduces to self-attention + MLP (SURVEY.md A5) plus,
+            # in the GELU / bias family, the cross-attention projection of that zero output: its bias. Inference only.
             if torch.is_grad_enabled() and (y.requires_grad or any(p.requires_grad for p in self.decoder.parameters())):
                 raise NotImplementedError("decoder with an empty context is an inference-only path (wrap it in torch.no_grad())")
+            zero = torch.zeros(B * M, D, dtype=bf16, device=y.device) if self.gelu else None
             for i, blk in enumerate(self.decoder):
-                wqkv, wsproj, _, _, _, w13, w2 = self._dec_weights(i)
-                h, _ = _self_attn_fwd(h, blk.norm1.weight, wqkv, wsproj, B, M, g.H, g.m_dec, g.eps)
-                h, _ = _mlp_fwd(h, blk.norm2.weight, w13, w2, g.eps)
+                wqkv, wsproj, _, _, wxproj, w13, w2 = self._dec_weights(i)
+                h, _ = _self_attn_fwd(h, blk.norm1.weight, wqkv, wsproj, B, M, g.H, g.m_dec, g.eps,
+                                      bias=self._attn_bias(blk.self_attn, blk.norm1))
+                if self.gelu:
+                    h = ops.linear_fwd(zero, wxproj, bias=_det(blk.cross_attn.proj.bias), addend=h, out_dtype=f32)
+                h = self._mlp_infer(blk, h, w13, w2, g.eps)
             return self.decoder_norm(h).reshape(B, M, D)
         for i, blk in enumerate(self.decoder):
             h = self._dec_block(i, blk, h, c, g)
         return self.decoder_norm(h).reshape(B, M, D)
-
-    def _dec_block(self, i, blk, h, c, g):
-        return _DecoderBlockFn.apply(h, c, blk.norm1.weight, blk.self_attn.qkv.weight, blk.self_attn.proj.weight,
-                                     blk.query_norm.weight, blk.context_norm.weight, blk.cross_attn.q.weight,
-                                     blk.cross_attn.kv.weight, blk.cross_attn.proj.weight, blk.norm2.weight,
-                                     blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._dec_weights(i), g)
 
     def forward_logits(self, y, decoder_mod_dict, decoder_mod_mask, return_all_logits: bool = False):
         out = {}
@@ -750,9 +933,11 @@ class EgoM2P(nn.Module):
         g.build_meta(dev)
         for i, blk in enumerate(self.encoder):
             wqkv, wproj, w13, w2 = self._enc_weights(i)
-            x, _ = _self_attn_fwd(x, blk.norm1.weight.detach(), wqkv, wproj, B, N, g.H, g.m_enc, g.eps)
-            x, _ = _mlp_fwd(x, blk.norm2.weight.detach(), w13, w2, g.eps)
-        h, _, _, _ = ops.layernorm_fwd(x, self.encoder_norm.weight.detach(), self.eps, save_stats=False)
+            x, _ = _self_attn_fwd(x, blk.norm1.weight.detach(), wqkv, wproj, B, N, g.H, g.m_enc, g.eps,
+                                  bias=self._attn_bias(blk.attn, blk.norm1))
+            x = self._mlp_infer(blk, x, w13, w2, g.eps)
+        h, _, _, _ = ops.layernorm_fwd(x, self.encoder_norm.weight.detach(), self.eps, save_stats=False,
+                                       bias=_ln_bias(self.encoder_norm))
         context = ops.linear_fwd(h, self._bf16("ctx", self.decoder_proj_context.weight), bias=self.decoder_proj_context.bias.detach(),
                                  addend=emb, out_dtype=f32)
         return context.reshape(B, N, D), ep.n_valid
@@ -776,16 +961,23 @@ class EgoM2P(nn.Module):
         h = y0.reshape(B * M, D).float().contiguous()
         for i, blk in enumerate(self.decoder):
             wqkv, wsproj, wq, wkv, wxproj, w13, w2 = self._dec_weights(i)
-            h, _ = _self_attn_fwd(h, blk.norm1.weight.detach(), wqkv, wsproj, B, M, g.H, g.m_dec, g.eps)
+            h, _ = _self_attn_fwd(h, blk.norm1.weight.detach(), wqkv, wsproj, B, M, g.H, g.m_dec, g.eps,
+                                  bias=self._attn_bias(blk.self_attn, blk.norm1))
+            xa = blk.cross_attn
             if N > 0:
-                hq, _, _, _ = ops.layernorm_fwd(h, blk.query_norm.weight.detach(), g.eps, save_stats=False)
-                q = ops.linear_fwd(hq, wq)
-                hc, _, _, _ = ops.layernorm_fwd(c, blk.context_norm.weight.detach(), g.eps, save_stats=False)
-                kv = ops.linear_fwd(hc, wkv)
+                hq, _, _, _ = ops.layernorm_fwd(h, blk.query_norm.weight.detach(), g.eps, save_stats=False, bias=_ln_bias(blk.query_norm))
+                q = ops.linear_fwd(hq, wq, bias=_det(xa.q.bias))
+                hc, _, _, _ = ops.layernorm_fwd(c, blk.context_norm.weight.detach(), g.eps, save_stats=False,
+                                                bias=_ln_bias(blk.context_norm))
+                kv = ops.linear_fwd(hc, wkv, bias=_det(xa.kv.bias))
                 o2, _ = ops.attn_fwd(q, kv[:, :D], kv[:, D:], B, g.H, M, N, meta=g.m_x, want_lse=False)
-                h = ops.linear_fwd(o2, wxproj, addend=h, out_dtype=f32)
-            h, _ = _mlp_fwd(h, blk.norm2.weight.detach(), w13, w2, g.eps)
-        _, yn, _, _ = ops.layernorm_fwd(h, self.decoder_norm.weight.detach(), self.eps, out_bf16=False, out_f32=True, save_stats=False)
+                h = ops.linear_fwd(o2, wxproj, bias=_det(xa.proj.bias), addend=h, out_dtype=f32)
+            elif self.gelu:   # no context anywhere: the cross-attention output is 0, its projection is the bias
+                h = ops.linear_fwd(torch.zeros(B * M, D, dtype=bf16, device=dev), wxproj, bias=_det(xa.proj.bias), addend=h,
+                                   out_dtype=f32)
+            h = self._mlp_infer(blk, h, w13, w2, g.eps)
+        _, yn, _, _ = ops.layernorm_fwd(h, self.decoder_norm.weight.detach(), self.eps, out_bf16=False, out_f32=True, save_stats=False,
+                                        bias=_ln_bias(self.decoder_norm))
         return yn
 
     def head_operand(self, mod: str) -> torch.Tensor:
@@ -927,9 +1119,9 @@ class EgoM2P(nn.Module):
 
         # ---- encoder
         for i, blk in enumerate(self.encoder):
-            x = _EncoderBlockFn.apply(x, blk.norm1.weight, blk.attn.qkv.weight, blk.attn.proj.weight, blk.norm2.weight,
-                                      blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._enc_weights(i), g)
-        context = _ContextFn.apply(x, enc_emb, self.encoder_norm.weight, self.decoder_proj_context.weight,
+            x = self._enc_block(i, blk, x, g)
+        context = _ContextFn.apply(x, enc_emb, self.encoder_norm.weight, self.encoder_norm.bias if self.gelu else None,
+                                   self.decoder_proj_context.weight,
                                    self.decoder_proj_context.bias, self._bf16("ctx", self.decoder_proj_context.weight), self.eps,
                                    self._epoch)
         # ---- decoder
@@ -955,7 +1147,8 @@ class EgoM2P(nn.Module):
             w = self.decoder_embeddings[m].to_logits.weight
             heads.append(w)
             wbs.append(self._bf16(("head", m), w))
-        per_mod = _HeadLossFn.apply(y, self.decoder_norm.weight, rows, targets, wbs, self.eps, self._epoch, *heads)
+        per_mod = _HeadLossFn.apply(y, self.decoder_norm.weight, self.decoder_norm.bias if self.gelu else None, rows, targets, wbs,
+                                    self.eps, self._epoch, *heads)
         mod_loss = {}
         for m, l in zip(dec_mods, per_mod):
             if loss_type == "weighted_mod" and rows[dec_mods.index(m)].numel():

@@ -188,7 +188,8 @@ def embed_gather_bwd(plan: Plan, dim: int, lens, vocabs, ids, pos, mod, dx0, dem
 
 
 # ----------------------------------------------------------------------------------------------- layernorm
-def layernorm_fwd(x: torch.Tensor, w: torch.Tensor, eps: float = 1e-6, out_bf16=True, out_f32=False, save_stats=True):
+def layernorm_fwd(x: torch.Tensor, w: torch.Tensor, eps: float = 1e-6, out_bf16=True, out_f32=False, save_stats=True, bias=None):
+    """bias: fp32 (D,) of a LayerNorm with a learnable bias (GELU / bias family), or None (no-bias kernel)."""
     lib = _lib.load()
     _req(x, f32, "x"); _req(w, f32, "weight")
     D = x.shape[-1]
@@ -198,11 +199,17 @@ def layernorm_fwd(x: torch.Tensor, w: torch.Tensor, eps: float = 1e-6, out_bf16=
     mean = torch.empty(rows, dtype=f32, device=x.device) if save_stats else None
     rstd = torch.empty(rows, dtype=f32, device=x.device) if save_stats else None
     with _timed("layernorm_fwd", rows * D * (4.0 + (2 if out_bf16 else 0) + (4 if out_f32 else 0)), "byte"):
-        _lib.check(lib.egom2p_layernorm_fwd(_p(x), _p(w), rows, D, eps, _p(yb), _p(yf), _p(mean), _p(rstd), _s()), "layernorm_fwd")
+        if bias is None:
+            _lib.check(lib.egom2p_layernorm_fwd(_p(x), _p(w), rows, D, eps, _p(yb), _p(yf), _p(mean), _p(rstd), _s()), "layernorm_fwd")
+        else:
+            _req(bias, f32, "bias")
+            _lib.check(lib.egom2p_layernorm_bias_fwd(_p(x), _p(w), _p(bias), rows, D, eps, _p(yb), _p(yf), _p(mean), _p(rstd), _s()),
+                       "layernorm_bias_fwd")
     return yb, yf, mean, rstd
 
 
-def layernorm_bwd(dy: torch.Tensor, x, w, mean, rstd, dx_in=None, d_weight=None, want_bf16=False):
+def layernorm_bwd(dy: torch.Tensor, x, w, mean, rstd, dx_in=None, d_weight=None, want_bf16=False, d_bias=None):
+    """d_bias: fp32 (D,) accumulator of the bias gradient (sum of dy over rows) of a LayerNorm with a bias, or None."""
     lib = _lib.load()
     D = x.shape[-1]
     rows = x.numel() // D
@@ -212,8 +219,13 @@ def layernorm_bwd(dy: torch.Tensor, x, w, mean, rstd, dx_in=None, d_weight=None,
     dyf = dy if dy.dtype == f32 else None
     nbytes = rows * D * (4.0 + dy.element_size() + 4 + (4 if dx_in is not None else 0) + (2 if want_bf16 else 0))
     with _timed("layernorm_bwd", nbytes, "byte"):
-        _lib.check(lib.egom2p_layernorm_bwd(_p(dyb), _p(dyf), _p(x), _p(w), _p(mean), _p(rstd), _p(dx_in), rows, D, _p(dx),
-                                            _p(dxb), _p(d_weight), _s()), "layernorm_bwd")
+        if d_bias is None:
+            _lib.check(lib.egom2p_layernorm_bwd(_p(dyb), _p(dyf), _p(x), _p(w), _p(mean), _p(rstd), _p(dx_in), rows, D, _p(dx),
+                                                _p(dxb), _p(d_weight), _s()), "layernorm_bwd")
+        else:
+            _req(d_bias, f32, "d_bias")
+            _lib.check(lib.egom2p_layernorm_bias_bwd(_p(dyb), _p(dyf), _p(x), _p(w), _p(mean), _p(rstd), _p(dx_in), rows, D,
+                                                     _p(dx), _p(dxb), _p(d_weight), _p(d_bias), _s()), "layernorm_bias_bwd")
     return dx, dxb
 
 
@@ -259,6 +271,33 @@ def gemm_swiglu_bwd(dy: torch.Tensor, w2: torch.Tensor, ab: torch.Tensor):
         _lib.check(lib.egom2p_gemm_swiglu_bwd(_p(dy), _p(w2), _p(ab), R, hidden, K, dy.stride(0), w2.stride(0), ab.stride(0),
                                               _p(dab), dab.stride(0), _s()), "gemm_swiglu_bwd")
     return dab
+
+
+def gemm_gelu_fwd(x: torch.Tensor, w1: torch.Tensor, b1: Optional[torch.Tensor]):
+    """u = x @ w1^T + b1 (bf16, saved for backward) and h = GELU(u) (bf16, exact erf form), activation fused into the epilogue."""
+    lib = _lib.load()
+    R, K = x.shape
+    N = w1.shape[0]
+    if b1 is not None:
+        _req(b1, f32, "b1")
+    u = torch.empty(R, N, dtype=bf16, device=x.device)
+    h = torch.empty(R, N, dtype=bf16, device=x.device)
+    with _timed("gemm", 2.0 * R * N * K, "flop"):
+        _lib.check(lib.egom2p_gemm_gelu_fwd(_p(x), _p(w1), _p(b1), R, N, K, x.stride(0), w1.stride(0), _p(u), u.stride(0), _p(h),
+                                            h.stride(0), _s()), "gemm_gelu_fwd")
+    return u, h
+
+
+def gemm_gelu_bwd(dy: torch.Tensor, w2: torch.Tensor, u: torch.Tensor):
+    """du = GELU'(u) * (dy @ w2), the derivative applied inside the fc2 dgrad epilogue; w2 is (K, hidden) bf16."""
+    lib = _lib.load()
+    R, K = dy.shape
+    hidden = w2.shape[1]
+    du = torch.empty(R, hidden, dtype=bf16, device=dy.device)
+    with _timed("gemm", 2.0 * R * hidden * K, "flop"):
+        _lib.check(lib.egom2p_gemm_gelu_bwd(_p(dy), _p(w2), _p(u), R, hidden, K, dy.stride(0), w2.stride(0), u.stride(0), _p(du),
+                                            du.stride(0), _s()), "gemm_gelu_bwd")
+    return du
 
 
 def linear_fwd(x: torch.Tensor, w: torch.Tensor, *, bias=None, addend=None, out_dtype=bf16):
@@ -445,6 +484,20 @@ def colsum(x: torch.Tensor, out: torch.Tensor):
     lib = _lib.load()
     rows, cols = x.shape
     _lib.check(lib.egom2p_colsum_f32(_p(x), rows, cols, _p(out), _s()), "colsum_f32")
+    return out
+
+
+def colsum_bf16(x: torch.Tensor, out: Optional[torch.Tensor] = None):
+    """Bias gradient out (+)= sum over rows of a bf16 (rows, cols) gradient (unit inner stride; views allowed)."""
+    lib = _lib.load()
+    _req(x, bf16, "x")
+    assert x.dim() == 2 and x.stride(1) == 1
+    rows, cols = x.shape
+    if out is None:
+        out = torch.zeros(cols, dtype=f32, device=x.device)
+    if rows:
+        with _timed("bias_grad", rows * cols * 2.0, "byte"):
+            _lib.check(lib.egom2p_colsum_bf16(_p(x), rows, cols, x.stride(0), _p(out), _s()), "colsum_bf16")
     return out
 
 

@@ -39,6 +39,26 @@ for _name, _args in {
     register_model(_fn)
 
 
+def _gelu(depth_e, depth_d, dim, heads):
+    """The GELU / bias family with the arguments the reference passes (4M's fm_*_gelu renamed fm_ -> egom2p_): biases on
+    every Linear and LayerNorm, nn.GELU MLP, everything else at the constructor defaults."""
+    def build(encoder_embeddings, decoder_embeddings, **kwargs):
+        return EgoM2P(encoder_embeddings=encoder_embeddings, decoder_embeddings=decoder_embeddings, encoder_depth=depth_e,
+                      decoder_depth=depth_d, dim=dim, num_heads=heads, mlp_ratio=4, qkv_bias=True,
+                      norm_layer=partial(nn.LayerNorm, eps=1e-6), **kwargs)
+    return build
+
+
+for _name, _args in {
+    "egom2p_tiny_6e_6d_gelu": (6, 6, 384, 6),
+    "egom2p_small_8e_8d_gelu": (8, 8, 512, 8),
+    "egom2p_base_12e_12d_gelu": (12, 12, 768, 12),
+}.items():
+    _fn = _gelu(*_args)
+    _fn.__name__ = _name
+    register_model(_fn)
+
+
 def model_entrypoint(name: str) -> Callable:
     return _ENTRYPOINTS[name]
 

@@ -99,6 +99,13 @@ int egom2p_layernorm_fwd(const float* x, const float* weight, int64_t rows, int3
 int egom2p_layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
                          const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
                          float* dx_out, uint16_t* dx_bf16, float* d_weight, void* stream);
+/* nn.LayerNorm(dim, eps) with a learnable bias (the GELU / bias family, egom2p_model.py:882-978): the forward adds bias[c]
+ * after the weight; the backward is the one above plus d_bias += sum_r dy (non-NULL), in the same pass. */
+int egom2p_layernorm_bias_fwd(const float* x, const float* weight, const float* bias, int64_t rows, int32_t dim, float eps,
+                              uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream);
+int egom2p_layernorm_bias_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
+                              const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
+                              float* dx_out, uint16_t* dx_bf16, float* d_weight, float* d_bias, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * (3b) bf16 GEMM on tcgen05/TMEM fed by TMA -- every nn.Linear on the path (egom2p_utils.py:167-169,187,203,226-228,
@@ -106,7 +113,8 @@ int egom2p_layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const flo
  *   a_mn = 0: A is (M,K) row-major (K contiguous);  a_mn = 1: A is stored (K,M) row-major (M contiguous)
  *   b_mn = 0: B is (N,K) row-major (K contiguous);  b_mn = 1: B is stored (K,N) row-major (N contiguous)
  * lda/ldb = row pitch in elements of the stored matrices. Epilogue: out = acc (+ bias[n]) (+ addend[m,n]);
- * written as bf16 (c_bf16) or fp32 (c_f32) -- exactly one; addend may alias c_f32 (accumulate). fp32 outputs with few
+ * written as bf16 (c_bf16) or fp32 (c_f32) -- exactly one; addend may alias c_f32 (accumulate). A bias with bf16 output
+ * (the biased qkv / q / kv projections) needs a_mn = b_mn = 0, no addend and a 16-byte aligned bias. fp32 outputs with few
  * tiles and long K (wgrad) are split along K and accumulated with TMA reduce-add.
  * ------------------------------------------------------------------------------------------------ */
 int egom2p_gemm_bf16(const uint16_t* A, const uint16_t* B, int32_t M, int32_t N, int32_t K, int64_t lda, int64_t ldb,
@@ -123,6 +131,15 @@ int egom2p_gemm_swiglu_fwd(const uint16_t* X, const uint16_t* W13, int32_t M, in
                            uint16_t* ab, int64_t ld_ab, uint16_t* g, int64_t ldg, void* stream);
 int egom2p_gemm_swiglu_bwd(const uint16_t* dY, const uint16_t* W2, const uint16_t* ab, int32_t M, int32_t hidden, int32_t K,
                            int64_t ldy, int64_t ldw, int64_t ld_ab, uint16_t* dab, int64_t ld_dab, void* stream);
+
+/* GELU MLP (fc2(GELU(fc1 x)) with biases, nn.GELU() exact erf form) with the activation fused into the GEMM epilogues.
+ *   fwd: u (M, N) bf16 = X W1^T + b1 (saved for backward; b1 fp32, may be NULL) and h (M, N) bf16 = GELU(u), in one pass.
+ *   bwd: dh = dY W2 (W2 stored (K, hidden), consumed MN-major) never leaves TMEM: du (M, hidden) bf16 = dh * GELU'(u).
+ * N / hidden must be multiples of 64. */
+int egom2p_gemm_gelu_fwd(const uint16_t* X, const uint16_t* W1, const float* b1, int32_t M, int32_t N, int32_t K, int64_t ldx,
+                         int64_t ldw, uint16_t* u, int64_t ld_u, uint16_t* h, int64_t ldh, void* stream);
+int egom2p_gemm_gelu_bwd(const uint16_t* dY, const uint16_t* W2, const uint16_t* u, int32_t M, int32_t hidden, int32_t K,
+                         int64_t ldy, int64_t ldw, int64_t ld_u, uint16_t* du, int64_t ld_du, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * (4) Vocabulary head fused with softmax cross-entropy (egom2p/models/decoder_embeddings.py:489-500,
@@ -216,6 +233,9 @@ int egom2p_adamw_multi(const void* items_dev, int32_t n_items, int64_t n_chunks,
                        int32_t* step_dev, const float* sumsq, float max_norm, void* stream);
 /* out[c] += sum_r x[r, c] -- bias gradient of decoder_proj_context (egom2p_model.py:157,722). */
 int egom2p_colsum_f32(const float* x, int64_t rows, int32_t cols, float* out, void* stream);
+/* out[c] += sum_r x[r, c] for a bf16 (rows, cols) matrix of row pitch ld (cols, ld multiples of 8): the bias gradients of
+ * the GELU / bias family's Linears from the bf16 output gradients, one atomic per column and row slab. */
+int egom2p_colsum_bf16(const uint16_t* x, int64_t rows, int32_t cols, int64_t ld, float* out, void* stream);
 /* dst[i, :] = src[idx[i], :] (bf16) and dst[idx[i], :] = src[i, :] (fp32): compaction of the rows of one modality for
  * its vocabulary head, replacing the boolean row-select y[decoder_mod_mask == id] (egom2p_model.py:633). */
 int egom2p_gather_rows_bf16(const uint16_t* src, const int64_t* idx, int64_t n, int32_t cols, uint16_t* dst, void* stream);
