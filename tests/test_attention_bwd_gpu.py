@@ -2,6 +2,8 @@
 import pytest
 import torch
 
+from test_kernels_gpu import attn_ranges
+
 pytestmark = pytest.mark.gpu
 
 
@@ -28,26 +30,21 @@ def _ref(q, k, v, do, lo, hi, H):
     return o.detach(), q.grad, k.grad, v.grad
 
 
+@pytest.mark.parametrize("gain", [1.0, 3.0])   # 1: |q| max|k| scale log2e ~ 15 -> bound-path softmax; 3: ~ 140 -> online-maximum path
 @pytest.mark.parametrize("B,H,Mq,Nk,mode", [(1, 1, 128, 128, "full"), (2, 3, 200, 200, "prefix"), (2, 2, 300, 517, "prefix"),
                                             (2, 2, 260, 260, "segments"), (1, 1, 20, 24, "prefix"), (1, 12, 2048, 2048, "segments"),
-                                            (2, 2, 256, 384, "prefix")])   # B > 1 with whole tiles: the TMA-store epilogue
-def test_attention_bwd(ops, B, H, Mq, Nk, mode):
+                                            (2, 2, 256, 384, "prefix"),    # B > 1 with whole tiles: the TMA-store epilogue
+                                            (2, 2, 260, 260, "causal"), (1, 3, 700, 700, "causal")])
+def test_attention_bwd(ops, B, H, Mq, Nk, mode, gain):
     gen = torch.Generator().manual_seed(Mq * 5 + Nk)
     D = H * 64
-    qkv = torch.randn(B, Mq, 3 * D, generator=gen).bfloat16()
-    kvsrc = qkv if Mq == Nk else torch.randn(B, Nk, 3 * D, generator=gen).bfloat16()
+    qkv = torch.randn(B, Mq, 3 * D, generator=gen)
+    qkv[..., :2 * D] *= gain
+    qkv = qkv.bfloat16()
+    kvsrc = qkv if Mq == Nk else torch.randn(B, Nk, 3 * D, generator=gen).mul_(torch.tensor([gain] * (2 * D) + [1.0] * D)).bfloat16()
     do = torch.randn(B, Mq, D, generator=gen).bfloat16()
     q, k, v = qkv[..., :D], kvsrc[..., D:2 * D], kvsrc[..., 2 * D:]
-    if mode == "full":
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = torch.full((B, Mq), Nk, dtype=torch.int32)
-    elif mode == "prefix":
-        n = torch.tensor([Nk - 3, 0][:B] if B > 1 else [Nk - 3], dtype=torch.int32)
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = n[:, None].expand(B, Mq).contiguous()
-    else:
-        bounds = [0, Mq // 2 - 11, Mq - 40, Mq - 25, Mq - 10]
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = torch.zeros(B, Mq, dtype=torch.int32)
-        for a, b_ in zip(bounds[:-1], bounds[1:]):
-            lo[:, a:b_] = a; hi[:, a:b_] = b_
+    lo, hi = attn_ranges(B, Mq, Nk, mode)
     o_ref, dq_ref, dk_ref, dv_ref = _ref(q, k, v, do, lo.long(), hi.long(), H)
     qd, kd = qkv.cuda().reshape(B * Mq, 3 * D), kvsrc.cuda().reshape(B * Nk, 3 * D)
     lod, hid = lo.cuda(), hi.cuda()

@@ -26,11 +26,10 @@ def _rel(a, b):
 
 
 # ------------------------------------------------------------------------------------------------ kernels
-@pytest.mark.parametrize("dim", [384, 768])
-def test_layernorm_bias_fwd_bwd(dim):
+@pytest.mark.parametrize("R,dim", [pytest.param(1000, 384, id="384"), pytest.param(1000, 768, id="768"), (34751, 768), (1, 768)])
+def test_layernorm_bias_fwd_bwd(R, dim):
     from egom2p_b200 import ops
     g = torch.Generator(device="cuda").manual_seed(0)
-    R = 1000
     x = torch.randn(R, dim, device="cuda", generator=g) * 2 + 0.5
     w = 1 + 0.1 * torch.randn(dim, device="cuda", generator=g)
     b = 0.1 * torch.randn(dim, device="cuda", generator=g)
@@ -86,7 +85,7 @@ def test_gelu_epilogues_sweep():
     assert float((du.float() - uu.grad).abs().max()) < 2e-2 * float(uu.grad.abs().max())
 
 
-@pytest.mark.parametrize("rows,cols", [(65536, 2304), (65536, 768), (333, 1536)])
+@pytest.mark.parametrize("rows,cols", [(65536, 2304), (65536, 768), (333, 1536), (34751, 2304), (1, 768)])
 def test_bias_grad_colsum(rows, cols):
     from egom2p_b200 import ops
     g = torch.Generator(device="cuda").manual_seed(3)

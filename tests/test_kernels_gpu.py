@@ -127,7 +127,7 @@ def test_embed_gather_bit_exact_and_grads(ops, golden_dir):
 
 
 # ------------------------------------------------------------------------------------------ layernorm / elementwise
-@pytest.mark.parametrize("rows,dim", [(37, 256), (1000, 768), (64, 384), (5, 48)])
+@pytest.mark.parametrize("rows,dim", [(37, 256), (1000, 768), (64, 384), (5, 48), (34751, 768), (1, 768)])
 def test_layernorm_fwd_bwd(ops, rows, dim):
     gen = torch.Generator().manual_seed(rows)
     x = torch.randn(rows, dim, generator=gen) * 2 + 0.5
@@ -266,6 +266,25 @@ def test_fused_head_cross_entropy(ops, R, V, K):
 
 
 # ------------------------------------------------------------------------------------------ attention forward
+def attn_ranges(B, Mq, Nk, mode):
+    """Key ranges [lo, hi) (B, Mq) int32 of the attention tests (shared with tests/test_attention_bwd_gpu.py)."""
+    lo = torch.zeros(B, Mq, dtype=torch.int32)
+    if mode == "full":
+        hi = torch.full((B, Mq), Nk, dtype=torch.int32)
+    elif mode == "prefix":   # encoder / cross: keys [0, n_b); one sample has an empty range -> uniform rows
+        n = torch.tensor([Nk - 3, 0][:B] if B > 1 else [Nk - 3], dtype=torch.int32)
+        hi = n[:, None].expand(B, Mq).contiguous()
+    else:                    # decoder self: contiguous modality segments + a pad tail with empty ranges
+        assert mode in ("segments", "causal")
+        bounds = [0, Mq // 2 - 11, Mq - 40, Mq - 25, Mq - 10]
+        hi = torch.zeros(B, Mq, dtype=torch.int32)
+        for a, b_ in zip(bounds[:-1], bounds[1:]):
+            lo[:, a:b_] = a
+            # causal: row i sees [segment start, i + 1) -- a different end on every row
+            hi[:, a:b_] = torch.arange(a + 1, b_ + 1, dtype=torch.int32) if mode == "causal" else b_
+    return lo, hi
+
+
 def _attn_ref(q, k, v, lo, hi, H):
     """fp64 reference with the reference's masked_fill(-finfo.max) semantics. q (B,Mq,H*64), k/v (B,Nk,H*64)."""
     B, Mq, _ = q.shape
@@ -284,7 +303,8 @@ def _attn_ref(q, k, v, lo, hi, H):
 @pytest.mark.parametrize("gain", [1.0, 3.0])   # 1: |q| max|k| scale log2e ~ 15 -> bound-path softmax; 3: ~ 140 -> online-maximum path
 @pytest.mark.parametrize("B,H,Mq,Nk,mode", [(2, 3, 200, 200, "prefix"), (1, 2, 128, 64, "full"), (2, 4, 300, 517, "prefix"),
                                             (2, 2, 260, 260, "segments"), (1, 1, 20, 24, "prefix"), (1, 12, 2048, 2048, "segments"),
-                                            (2, 2, 256, 384, "prefix")])   # B > 1 with whole tiles: the TMA-store epilogue
+                                            (2, 2, 256, 384, "prefix"),    # B > 1 with whole tiles: the TMA-store epilogue
+                                            (2, 2, 260, 260, "causal"), (1, 3, 700, 700, "causal")])
 def test_attention_fwd(ops, B, H, Mq, Nk, mode, gain):
     gen = torch.Generator().manual_seed(Mq * 7 + Nk)
     D = H * 64
@@ -293,16 +313,7 @@ def test_attention_fwd(ops, B, H, Mq, Nk, mode, gain):
     qkv = qkv.bfloat16()
     kvsrc = qkv if Mq == Nk else torch.randn(B, Nk, 3 * D, generator=gen).mul_(torch.tensor([gain] * (2 * D) + [1.0] * D)).bfloat16()
     q, k, v = qkv[..., :D], kvsrc[..., D:2 * D], kvsrc[..., 2 * D:]
-    if mode == "full":
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = torch.full((B, Mq), Nk, dtype=torch.int32)
-    elif mode == "prefix":   # encoder / cross: keys [0, n_b); one sample has an empty range -> uniform rows
-        n = torch.tensor([Nk - 3, 0][:B] if B > 1 else [Nk - 3], dtype=torch.int32)
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = n[:, None].expand(B, Mq).contiguous()
-    else:                    # decoder self: contiguous modality segments + a pad tail with empty ranges
-        bounds = [0, Mq // 2 - 11, Mq - 40, Mq - 25, Mq - 10]
-        lo = torch.zeros(B, Mq, dtype=torch.int32); hi = torch.zeros(B, Mq, dtype=torch.int32)
-        for a, b_ in zip(bounds[:-1], bounds[1:]):
-            lo[:, a:b_] = a; hi[:, a:b_] = b_
+    lo, hi = attn_ranges(B, Mq, Nk, mode)
     ref, s_ref = _attn_ref(q, k, v, lo.long(), hi.long(), H)
     qd, kd = dev(qkv).reshape(B * Mq, 3 * D), dev(kvsrc).reshape(B * Nk, 3 * D)
     o, lse = ops.attn_fwd(qd[:, :D], kd[:, D:2 * D], kd[:, 2 * D:], B, H, Mq, Nk, dev(lo), dev(hi))
