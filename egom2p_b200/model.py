@@ -46,13 +46,18 @@ class LayerNorm(nn.Module):
     def forward(self, x):
         shape = x.shape
         _, y, _, _ = ops.layernorm_fwd(x.reshape(-1, shape[-1]).float().contiguous(), self.weight.detach(), self.eps,
-                                       out_bf16=False, out_f32=True, save_stats=False, bias=_ln_bias(self))
+                                       out_bf16=False, out_f32=True, save_stats=False, bias=_det(_bias(self)))
         return y.reshape(shape)
 
 
-def _ln_bias(norm: nn.Module) -> Optional[torch.Tensor]:
-    """The learnable bias of a LayerNorm (detached), None for the zero buffer of the no-bias family."""
-    return norm.bias.detach() if isinstance(norm.bias, nn.Parameter) else None
+def _bias(m: nn.Module) -> Optional[torch.Tensor]:
+    """The learnable bias of a Linear or LayerNorm, None when it has none (the no-bias family's LayerNorms hold a zero buffer)."""
+    return m.bias if isinstance(m.bias, nn.Parameter) else None
+
+
+def _weights_and_biases(*mods: nn.Module) -> List[Optional[torch.Tensor]]:
+    """weight, bias (or None) of each module in turn: the flat parameter list the block functions take."""
+    return [t for m in mods for t in (m.weight, _bias(m))]
 
 
 def _det(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
@@ -70,13 +75,40 @@ class _Linear(nn.Linear):
         return y.reshape(*shape[:-1], -1)
 
 
+# The MLP is the only part of a block that differs between the two families. Each MLP container owns, for the shared block
+# code: params() -- its parameters, in the order the block functions take them; operands() -- their cached bf16 GEMM
+# operands; fwd() -- x1 + MLP(h2) from the normed h2, and what bwd() needs; bwd() -- dh2 and the gradients of params().
 class GatedMlp(nn.Module):
+    """fc2(SiLU(fc1 x) * fc3 x) without biases (the swiglu / no-bias family). fc1 and fc3 run as one GEMM over an operand
+    with their rows interleaved (EgoM2P._bf16), the gate in its epilogue."""
+
     def __init__(self, dim, hidden):
         super().__init__()
         hidden = int(2 * hidden / 3)
         self.fc1 = _Linear(dim, hidden, bias=False)
         self.fc2 = _Linear(hidden, dim, bias=False)
         self.fc3 = _Linear(dim, hidden, bias=False)
+
+    def params(self):
+        return self.fc1.weight, self.fc2.weight, self.fc3.weight
+
+    def operands(self, cache, key):
+        return cache((*key, "w13"), self.fc1.weight, self.fc3.weight), cache((*key, "w2"), self.fc2.weight, pad32=True)
+
+    def fwd(self, h2, x1, w, params):
+        w13, w2 = w
+        ab, g = ops.gemm_swiglu_fwd(h2, w13)   # fc1|fc3 GEMM with the SwiGLU gate in its epilogue
+        return ops.linear_fwd(g, w2, addend=x1, out_dtype=f32), (ab, g)
+
+    def bwd(self, dx2b, h2, w, saved):
+        (w13, w2), (ab, g) = w, saved
+        dw2 = ops.linear_wgrad(dx2b, g)
+        dab = ops.gemm_swiglu_bwd(dx2b, w2, ab)   # fc2 dgrad with the SwiGLU derivative in its epilogue
+        dw13 = ops.linear_wgrad(dab, h2)
+        dh2 = ops.linear_dgrad(dab, w13)
+        F = self.fc1.out_features
+        d1, d3 = _split_w13_grad(dw13, F)
+        return dh2, (d1, dw2[:, :F], d3)
 
 
 class Mlp(nn.Module):
@@ -86,6 +118,26 @@ class Mlp(nn.Module):
         super().__init__()
         self.fc1 = _Linear(dim, hidden, bias=True)
         self.fc2 = _Linear(hidden, dim, bias=True)
+
+    def params(self):
+        return self.fc1.weight, self.fc1.bias, self.fc2.weight, self.fc2.bias
+
+    def operands(self, cache, key):
+        return cache((*key, "w1"), self.fc1.weight), cache((*key, "w2"), self.fc2.weight, pad32=True)
+
+    def fwd(self, h2, x1, w, params):
+        (w1, w2), (_, b1, _, b2) = w, params
+        u, a = ops.gemm_gelu_fwd(h2, w1, b1)   # fc1 GEMM with + b1 and GELU in its epilogue
+        return ops.linear_fwd(a, w2, bias=b2, addend=x1, out_dtype=f32), (u, a)
+
+    def bwd(self, dx2b, h2, w, saved):
+        (w1, w2), (u, a) = w, saved
+        dw2 = ops.linear_wgrad(dx2b, a)
+        db2 = ops.colsum_bf16(dx2b)
+        du = ops.gemm_gelu_bwd(dx2b, w2, u)   # fc2 dgrad with GELU'(u) in its epilogue
+        dw1 = ops.linear_wgrad(du, h2)
+        db1 = ops.colsum_bf16(du)
+        return ops.linear_dgrad(du, w1), (dw1, db1, dw2, db2)
 
 
 class Attention(nn.Module):
@@ -191,30 +243,32 @@ def _bf16_of(dx):
     return ops.cast_bf16(dx)
 
 
-def _mlp_fwd(x1, n2w, w13, w2, eps):
-    h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps)
-    ab, g = ops.gemm_swiglu_fwd(h2, w13)   # fc1|fc3 GEMM with the SwiGLU gate in its epilogue
-    x2 = ops.linear_fwd(g, w2, addend=x1, out_dtype=f32)
-    return x2, (mean2, rstd2, h2, ab, g)
+def _present(*biases):
+    return tuple(b is not None for b in biases)
 
 
-def _mlp_bwd(dx2, x1, n2w, w13, w2, saved):
-    """Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dw13, dw2."""
-    mean2, rstd2, h2, ab, g = saved
-    dx2b = _bf16_of(dx2)
-    dw2 = ops.linear_wgrad(dx2b, g)
-    dab = ops.gemm_swiglu_bwd(dx2b, w2, ab)   # fc2 dgrad with the SwiGLU derivative in its epilogue
-    dw13 = ops.linear_wgrad(dab, h2)
-    dh2 = ops.linear_dgrad(dab, w13)
+def _mlp_fwd(mlp, x1, n2w, n2b, w, params, eps):
+    """x1 + mlp(norm2 x1). w: the MLP's bf16 operands (mlp.operands), params: its parameters (mlp.params)."""
+    h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps, bias=n2b)
+    x2, sm = mlp.fwd(h2, x1, w, params)
+    return x2, (mean2, rstd2, h2, *sm)
+
+
+def _mlp_bwd(mlp, dx2, x1, n2w, has_n2b, w, saved):
+    """Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b (None without a norm2 bias) and the gradients of
+    mlp.params()."""
+    mean2, rstd2, h2, *sm = saved
+    dh2, dparams = mlp.bwd(_bf16_of(dx2), h2, w, sm)
     dn2w = _zeros(n2w.numel(), dx2.device)
-    dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True)
-    return dx1, dx1b, dn2w, dw13, dw2
+    dn2b = _zeros(n2w.numel(), dx2.device) if has_n2b else None
+    dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True, d_bias=dn2b)
+    return dx1, dx1b, dn2w, dn2b, dparams
 
 
-def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs=None, bias=None):
-    """bias: (norm1 bias, qkv bias, proj bias) of the GELU / bias family, fp32; None for the no-bias family."""
+def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs, bias):
+    """bias: the (norm1, qkv, proj) biases, fp32 or None each."""
     D = x.shape[-1]
-    n1b, bqkv, bproj = bias if bias is not None else (None, None, None)
+    n1b, bqkv, bproj = bias
     h1, _, mean1, rstd1 = ops.layernorm_fwd(x, n1w, eps, bias=n1b)
     qkv = ops.linear_fwd(h1, wqkv, bias=bqkv)
     o, lse = ops.attn_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], B, H, L, L, meta=meta, pairs=pairs)
@@ -222,8 +276,9 @@ def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs=None, bias=Non
     return x1, (mean1, rstd1, h1, qkv, o, lse)
 
 
-def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs=None, biased=False):
-    """Returns dx, dn1w, dwqkv, dwproj and, when biased, (dn1b, dbqkv, dbproj) (else None)."""
+def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs, has_bias):
+    """has_bias: whether norm1, qkv and proj have a bias. Returns dx, dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, with None
+    for the gradient of an absent bias."""
     mean1, rstd1, h1, qkv, o, lse = saved
     D = x.shape[-1]
     dwproj = ops.linear_wgrad(dx1b, o)
@@ -233,42 +288,20 @@ def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs=N
                  dqkv[:, 2 * D:], meta=meta, pairs=pairs)
     dwqkv = ops.linear_wgrad(dqkv, h1)
     dh1 = ops.linear_dgrad(dqkv, wqkv)
+    has_n1b, has_bqkv, has_bproj = has_bias
     dn1w = _zeros(n1w.numel(), x.device)
-    extra = None
-    if biased:
-        extra = (_zeros(n1w.numel(), x.device), ops.colsum_bf16(dqkv), ops.colsum_bf16(dx1b))
-    dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True,
-                                d_bias=extra[0] if biased else None)
-    return _with_bf16(dx, dxb), dn1w, dwqkv, dwproj, extra
+    dn1b = _zeros(n1w.numel(), x.device) if has_n1b else None
+    dbqkv = ops.colsum_bf16(dqkv) if has_bqkv else None
+    dbproj = ops.colsum_bf16(dx1b) if has_bproj else None
+    dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True, d_bias=dn1b)
+    return _with_bf16(dx, dxb), dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj
 
 
-def _gelu_mlp_fwd(x1, n2w, n2b, w1, b1, w2, b2, eps):
-    h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps, bias=n2b)
-    u, a = ops.gemm_gelu_fwd(h2, w1, b1)   # fc1 GEMM with + b1 and GELU in its epilogue
-    x2 = ops.linear_fwd(a, w2, bias=b2, addend=x1, out_dtype=f32)
-    return x2, (mean2, rstd2, h2, u, a)
-
-
-def _gelu_mlp_bwd(dx2, x1, n2w, w1, w2, saved):
-    """Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b, dw1, db1, dw2, db2."""
-    mean2, rstd2, h2, u, a = saved
-    dev = dx2.device
-    dx2b = _bf16_of(dx2)
-    dw2 = ops.linear_wgrad(dx2b, a)
-    db2 = ops.colsum_bf16(dx2b)
-    du = ops.gemm_gelu_bwd(dx2b, w2, u)   # fc2 dgrad with GELU'(u) in its epilogue
-    dw1 = ops.linear_wgrad(du, h2)
-    db1 = ops.colsum_bf16(du)
-    dh2 = ops.linear_dgrad(du, w1)
-    dn2w, dn2b = _zeros(n2w.numel(), dev), _zeros(n2w.numel(), dev)
-    dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True, d_bias=dn2b)
-    return dx1, dx1b, dn2w, dn2b, dw1, db1, dw2, db2
-
-
-def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias=None):
-    """y2 = y1 + cross_attn(query_norm y1, context_norm context). bias: (query_norm, context_norm, q, kv, proj biases) or None."""
+def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias):
+    """y2 = y1 + cross_attn(query_norm y1, context_norm context). bias: the (query_norm, context_norm, q, kv, proj) biases,
+    fp32 or None each."""
     D = y1.shape[-1]
-    qnb, cnb, bq, bkv, bxproj = bias if bias is not None else (None,) * 5
+    qnb, cnb, bq, bkv, bxproj = bias
     hq, _, meanq, rstdq = ops.layernorm_fwd(y1, qnw, g.eps, bias=qnb)
     q = ops.linear_fwd(hq, wq, bias=bq)
     hc, _, meanc, rstdc = ops.layernorm_fwd(context, cnw, g.eps, bias=cnb)
@@ -278,9 +311,10 @@ def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias=None):
     return y2, (meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2)
 
 
-def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, biased=False):
-    """Backward of _cross_fwd. Returns dy1, dy1b, dctx (None unless this block returns the summed context gradient),
-    dqnw, dcnw, dwq, dwkv, dwxproj and, when biased, (dqnb, dcnb, dbq, dbkv, dbxproj) (else None)."""
+def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, has_bias):
+    """Backward of _cross_fwd. has_bias: whether query_norm, context_norm, q, kv and proj have a bias. Returns dy1, dy1b,
+    dctx (None unless this block returns the summed context gradient), then dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv,
+    dwxproj, dbxproj, with None for the gradient of an absent bias."""
     meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2 = saved
     D = y1.shape[-1]
     dev = y1.device
@@ -293,12 +327,14 @@ def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sa
     dhq = ops.linear_dgrad(dq, wq)
     dwkv = ops.linear_wgrad(dkv, hc)
     dhc = ops.linear_dgrad(dkv, wkv)
+    has_qnb, has_cnb, has_bq, has_bkv, has_bxproj = has_bias
     dqnw, dcnw = _zeros(D, dev), _zeros(D, dev)
-    extra = None
-    if biased:
-        extra = (_zeros(D, dev), _zeros(D, dev), ops.colsum_bf16(dq), ops.colsum_bf16(dkv), ops.colsum_bf16(dy2b))
-    dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True,
-                                  d_bias=extra[0] if biased else None)
+    dqnb = _zeros(D, dev) if has_qnb else None
+    dcnb = _zeros(D, dev) if has_cnb else None
+    dbq = ops.colsum_bf16(dq) if has_bq else None
+    dbkv = ops.colsum_bf16(dkv) if has_bkv else None
+    dbxproj = ops.colsum_bf16(dy2b) if has_bxproj else None
+    dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True, d_bias=dqnb)
     # All decoder blocks read the same `context`: instead of letting autograd add twelve (B*N, D) fp32 gradients pairwise,
     # each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block that runs last
     # returns it. Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
@@ -306,7 +342,7 @@ def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sa
     chained = g.ctx_users > 0 and (acc is None or (acc[0] == ctx_key and acc[1].shape == context.shape))
     last = chained and g.ctx_users == 1
     dctx, dctxb = ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, dx_in=acc[1] if (chained and acc is not None) else None,
-                                    d_weight=dcnw, want_bf16=last, d_bias=extra[1] if biased else None)
+                                    d_weight=dcnw, want_bf16=last, d_bias=dcnb)
     if chained:
         g.ctx_users -= 1
         if last:
@@ -315,18 +351,21 @@ def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sa
         else:
             g.dctx_acc = (ctx_key, dctx)
             dctx = None
-    return dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, extra
+    return dy1, dy1b, dctx, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj
 
 
 class _EncoderBlockFn(torch.autograd.Function):
-    """x + attn(norm1 x) then + mlp(norm2 .) -- egom2p_utils.py:356-359."""
+    """x + attn(norm1 x) then + mlp(norm2 .) -- egom2p_utils.py:356-359. Parameters: weight and bias of norm1, qkv, proj and
+    norm2, then mlp.params(); an absent bias is None and gets None as its gradient."""
 
     @staticmethod
-    def forward(ctx, x, n1w, qkv_w, proj_w, n2w, fc1_w, fc2_w, fc3_w, wb, geom):
-        wqkv, wproj, w13, w2 = wb
-        x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, geom.B, geom.N, geom.H, geom.m_enc, geom.eps, geom.p_enc)
-        x2, sm = _mlp_fwd(x1, n2w, w13, w2, geom.eps)
-        ctx.geom, ctx.wb, ctx.F = geom, wb, fc1_w.shape[0]
+    def forward(ctx, x, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, n2w, n2b, *mlp_params):
+        wqkv, wproj, *wm = wb
+        g = geom
+        x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, g.B, g.N, g.H, g.m_enc, g.eps, g.p_enc, (n1b, qkv_b, proj_b))
+        x2, sm = _mlp_fwd(mlp, x1, n2w, n2b, wm, mlp_params, g.eps)
+        ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
+        ctx.sa_bias, ctx.n2_bias = _present(n1b, qkv_b, proj_b), n2b is not None
         ctx.op_epoch = geom.epoch_ref[0]
         ctx.save_for_backward(x, n1w, n2w, x1, *sa, *sm)
         return x2
@@ -337,28 +376,29 @@ class _EncoderBlockFn(torch.autograd.Function):
         _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
         x, n1w, n2w, x1, *rest = ctx.saved_tensors
         sa, sm = rest[:6], rest[6:]
-        wqkv, wproj, w13, w2 = ctx.wb
+        wqkv, wproj, *wm = ctx.wb
         g = ctx.geom
-        dx2 = dx2.contiguous()
-        dx1, dx1b, dn2w, dw13, dw2 = _mlp_bwd(dx2, x1, n2w, w13, w2, sm)
-        dx, dn1w, dwqkv, dwproj, _ = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc)
-        F = ctx.F
-        d1, d3 = _split_w13_grad(dw13, F)
-        return dx, dn1w, dwqkv, dwproj, dn2w, d1, dw2[:, :F], d3, None, None
+        dx1, dx1b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dx2.contiguous(), x1, n2w, ctx.n2_bias, wm, sm)
+        dx, *dsa = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc, ctx.sa_bias)
+        return (dx, None, None, None, *dsa, dn2w, dn2b, *dmlp)
 
 
 class _DecoderBlockFn(torch.autograd.Function):
-    """self-attn -> cross-attn(query_norm y, context_norm ctx) -> mlp -- egom2p_utils.py:387-391."""
+    """self-attn -> cross-attn(query_norm y, context_norm ctx) -> mlp -- egom2p_utils.py:387-391. Parameters: weight and bias
+    of norm1, qkv, self-attention proj, query_norm, context_norm, q, kv, cross-attention proj and norm2, then
+    mlp.params(); an absent bias is None and gets None as its gradient."""
 
     @staticmethod
-    def forward(ctx, y, context, n1w, qkv_w, sproj_w, qnw, cnw, q_w, kv_w, xproj_w, n2w, fc1_w, fc2_w, fc3_w, wb, geom):
-        wqkv, wsproj, wq, wkv, wxproj, w13, w2 = wb
+    def forward(ctx, y, context, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, sproj_w, sproj_b, qnw, qnb, cnw, cnb, q_w, q_b, kv_w,
+                kv_b, xproj_w, xproj_b, n2w, n2b, *mlp_params):
+        wqkv, wsproj, wq, wkv, wxproj, *wm = wb
         g = geom
-        D = y.shape[-1]
-        y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec)
-        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g)
-        y3, sm = _mlp_fwd(y2, n2w, w13, w2, g.eps)
-        ctx.geom, ctx.wb, ctx.F = geom, wb, fc1_w.shape[0]
+        y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec, (n1b, qkv_b, sproj_b))
+        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, (qnb, cnb, q_b, kv_b, xproj_b))
+        y3, sm = _mlp_fwd(mlp, y2, n2w, n2b, wm, mlp_params, g.eps)
+        ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
+        ctx.sa_bias, ctx.x_bias = _present(n1b, qkv_b, sproj_b), _present(qnb, cnb, q_b, kv_b, xproj_b)
+        ctx.n2_bias = n2b is not None
         ctx.op_epoch = geom.epoch_ref[0]
         ctx.ctx_key = context.data_ptr()
         g.ctx_users += 1
@@ -371,79 +411,12 @@ class _DecoderBlockFn(torch.autograd.Function):
         _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
         (y, context, n1w, qnw, cnw, n2w, y1, y2, *rest) = ctx.saved_tensors
         sx, sa, sm = rest[:10], rest[10:16], rest[16:]
-        wqkv, wsproj, wq, wkv, wxproj, w13, w2 = ctx.wb
+        wqkv, wsproj, wq, wkv, wxproj, *wm = ctx.wb
         g = ctx.geom
-        dy3 = dy3.contiguous()
-        dy2, dy2b, dn2w, dw13, dw2 = _mlp_bwd(dy3, y2, n2w, w13, w2, sm)
-        dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, _ = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv,
-                                                                       wxproj, sx)
-        dy, dn1w, dwqkv, dwsproj, _ = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec)
-        F = ctx.F
-        d1, d3 = _split_w13_grad(dw13, F)
-        return (dy, dctx, dn1w, dwqkv, dwsproj, dqnw, dcnw, dwq, dwkv, dwxproj, dn2w, d1, dw2[:, :F], d3, None, None)
-
-
-class _GeluEncoderBlockFn(torch.autograd.Function):
-    """GELU / bias family: x + attn(norm1 x) then + fc2(GELU(fc1 norm2 .)), every Linear and LayerNorm with a bias."""
-
-    @staticmethod
-    def forward(ctx, x, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, wb, geom):
-        wqkv, wproj, w1, w2 = wb
-        g = geom
-        x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, g.B, g.N, g.H, g.m_enc, g.eps, g.p_enc, bias=(n1b, qkv_b, proj_b))
-        x2, sm = _gelu_mlp_fwd(x1, n2w, n2b, w1, fc1_b, w2, fc2_b, g.eps)
-        ctx.geom, ctx.wb = geom, wb
-        ctx.op_epoch = geom.epoch_ref[0]
-        ctx.save_for_backward(x, n1w, n2w, x1, *sa, *sm)
-        return x2
-
-    @staticmethod
-    def backward(ctx, dx2):
-        _GRAD_GEN[0] += 1
-        _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
-        x, n1w, n2w, x1, *rest = ctx.saved_tensors
-        sa, sm = rest[:6], rest[6:]
-        wqkv, wproj, w1, w2 = ctx.wb
-        g = ctx.geom
-        dx1, dx1b, dn2w, dn2b, dw1, db1, dw2, db2 = _gelu_mlp_bwd(dx2.contiguous(), x1, n2w, w1, w2, sm)
-        dx, dn1w, dwqkv, dwproj, (dn1b, dbqkv, dbproj) = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H,
-                                                                        g.m_enc, g.p_enc, biased=True)
-        return dx, dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, dn2w, dn2b, dw1, db1, dw2, db2, None, None
-
-
-class _GeluDecoderBlockFn(torch.autograd.Function):
-    """GELU / bias family: self-attn -> cross-attn(query_norm y, context_norm ctx) -> GELU MLP, all with biases."""
-
-    @staticmethod
-    def forward(ctx, y, context, n1w, n1b, qkv_w, qkv_b, sproj_w, sproj_b, qnw, qnb, cnw, cnb, q_w, q_b, kv_w, kv_b,
-                xproj_w, xproj_b, n2w, n2b, fc1_w, fc1_b, fc2_w, fc2_b, wb, geom):
-        wqkv, wsproj, wq, wkv, wxproj, w1, w2 = wb
-        g = geom
-        y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec, bias=(n1b, qkv_b, sproj_b))
-        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias=(qnb, cnb, q_b, kv_b, xproj_b))
-        y3, sm = _gelu_mlp_fwd(y2, n2w, n2b, w1, fc1_b, w2, fc2_b, g.eps)
-        ctx.geom, ctx.wb = geom, wb
-        ctx.op_epoch = geom.epoch_ref[0]
-        ctx.ctx_key = context.data_ptr()
-        g.ctx_users += 1
-        ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, *sx, *sa, *sm)
-        return y3
-
-    @staticmethod
-    def backward(ctx, dy3):
-        _GRAD_GEN[0] += 1
-        _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
-        (y, context, n1w, qnw, cnw, n2w, y1, y2, *rest) = ctx.saved_tensors
-        sx, sa, sm = rest[:10], rest[10:16], rest[16:]
-        wqkv, wsproj, wq, wkv, wxproj, w1, w2 = ctx.wb
-        g = ctx.geom
-        dy2, dy2b, dn2w, dn2b, dw1, db1, dw2, db2 = _gelu_mlp_bwd(dy3.contiguous(), y2, n2w, w1, w2, sm)
-        dy1, dy1b, dctx, dqnw, dcnw, dwq, dwkv, dwxproj, (dqnb, dcnb, dbq, dbkv, dbxproj) = _cross_bwd(
-            g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, biased=True)
-        dy, dn1w, dwqkv, dwsproj, (dn1b, dbqkv, dbsproj) = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H,
-                                                                          g.m_dec, g.p_dec, biased=True)
-        return (dy, dctx, dn1w, dn1b, dwqkv, dbqkv, dwsproj, dbsproj, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj,
-                dbxproj, dn2w, dn2b, dw1, db1, dw2, db2, None, None)
+        dy2, dy2b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dy3.contiguous(), y2, n2w, ctx.n2_bias, wm, sm)
+        dy1, dy1b, dctx, *dxa = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, ctx.x_bias)
+        dy, *dsa = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec, ctx.sa_bias)
+        return (dy, dctx, None, None, None, *dsa, *dxa, dn2w, dn2b, *dmlp)
 
 
 class _ContextFn(torch.autograd.Function):
@@ -773,57 +746,57 @@ class EgoM2P(nn.Module):
 
     def _enc_weights(self, i: int):
         b = self.encoder[i]
-        if self.gelu:
-            return (self._bf16(("e", i, "qkv"), b.attn.qkv.weight), self._bf16(("e", i, "proj"), b.attn.proj.weight),
-                    self._bf16(("e", i, "w1"), b.mlp.fc1.weight), self._bf16(("e", i, "w2"), b.mlp.fc2.weight, pad32=True))
         return (self._bf16(("e", i, "qkv"), b.attn.qkv.weight), self._bf16(("e", i, "proj"), b.attn.proj.weight),
-                self._bf16(("e", i, "w13"), b.mlp.fc1.weight, b.mlp.fc3.weight), self._bf16(("e", i, "w2"), b.mlp.fc2.weight, pad32=True))
+                *b.mlp.operands(self._bf16, ("e", i)))
 
     def _dec_weights(self, i: int):
         b = self.decoder[i]
-        if self.gelu:
-            return (self._bf16(("d", i, "qkv"), b.self_attn.qkv.weight), self._bf16(("d", i, "sproj"), b.self_attn.proj.weight),
-                    self._bf16(("d", i, "q"), b.cross_attn.q.weight), self._bf16(("d", i, "kv"), b.cross_attn.kv.weight),
-                    self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight),
-                    self._bf16(("d", i, "w1"), b.mlp.fc1.weight), self._bf16(("d", i, "w2"), b.mlp.fc2.weight, pad32=True))
         return (self._bf16(("d", i, "qkv"), b.self_attn.qkv.weight), self._bf16(("d", i, "sproj"), b.self_attn.proj.weight),
                 self._bf16(("d", i, "q"), b.cross_attn.q.weight), self._bf16(("d", i, "kv"), b.cross_attn.kv.weight),
-                self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight),
-                self._bf16(("d", i, "w13"), b.mlp.fc1.weight, b.mlp.fc3.weight), self._bf16(("d", i, "w2"), b.mlp.fc2.weight, pad32=True))
+                self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight), *b.mlp.operands(self._bf16, ("d", i)))
 
-    # ------------------------------------------------------------------ block application (training and inference)
+    # ------------------------------------------------------------------ block application (training)
     def _enc_block(self, i, blk, h, g):
-        if self.gelu:
-            a, m = blk.attn, blk.mlp
-            return _GeluEncoderBlockFn.apply(h, blk.norm1.weight, blk.norm1.bias, a.qkv.weight, a.qkv.bias, a.proj.weight, a.proj.bias,
-                                             blk.norm2.weight, blk.norm2.bias, m.fc1.weight, m.fc1.bias, m.fc2.weight, m.fc2.bias,
-                                             self._enc_weights(i), g)
-        return _EncoderBlockFn.apply(h, blk.norm1.weight, blk.attn.qkv.weight, blk.attn.proj.weight, blk.norm2.weight,
-                                     blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._enc_weights(i), g)
+        return _EncoderBlockFn.apply(h, blk.mlp, self._enc_weights(i), g,
+                                     *_weights_and_biases(blk.norm1, blk.attn.qkv, blk.attn.proj, blk.norm2), *blk.mlp.params())
 
     def _dec_block(self, i, blk, h, c, g):
-        if self.gelu:
-            sa, xa, m = blk.self_attn, blk.cross_attn, blk.mlp
-            return _GeluDecoderBlockFn.apply(h, c, blk.norm1.weight, blk.norm1.bias, sa.qkv.weight, sa.qkv.bias, sa.proj.weight,
-                                             sa.proj.bias, blk.query_norm.weight, blk.query_norm.bias, blk.context_norm.weight,
-                                             blk.context_norm.bias, xa.q.weight, xa.q.bias, xa.kv.weight, xa.kv.bias, xa.proj.weight,
-                                             xa.proj.bias, blk.norm2.weight, blk.norm2.bias, m.fc1.weight, m.fc1.bias, m.fc2.weight,
-                                             m.fc2.bias, self._dec_weights(i), g)
-        return _DecoderBlockFn.apply(h, c, blk.norm1.weight, blk.self_attn.qkv.weight, blk.self_attn.proj.weight,
-                                     blk.query_norm.weight, blk.context_norm.weight, blk.cross_attn.q.weight,
-                                     blk.cross_attn.kv.weight, blk.cross_attn.proj.weight, blk.norm2.weight,
-                                     blk.mlp.fc1.weight, blk.mlp.fc2.weight, blk.mlp.fc3.weight, self._dec_weights(i), g)
+        sa, xa = blk.self_attn, blk.cross_attn
+        return _DecoderBlockFn.apply(h, c, blk.mlp, self._dec_weights(i), g,
+                                     *_weights_and_biases(blk.norm1, sa.qkv, sa.proj, blk.query_norm, blk.context_norm, xa.q,
+                                                          xa.kv, xa.proj, blk.norm2), *blk.mlp.params())
 
-    def _attn_bias(self, attn: nn.Module, norm: nn.Module):
-        """(norm bias, qkv bias, proj bias) of a self-attention sub-block (detached) for _self_attn_fwd, None for swiglu."""
-        return (_ln_bias(norm), _det(attn.qkv.bias), _det(attn.proj.bias)) if self.gelu else None
+    # ------------------------------------------------------------------ blocks without autograd (generation / sampler paths)
+    def _self_attn_infer(self, attn, norm, h, wqkv, wproj, B, L, meta):
+        return _self_attn_fwd(h, norm.weight, wqkv, wproj, B, L, self.num_heads, meta, self.eps, None,
+                              (_bias(norm), _bias(attn.qkv), _bias(attn.proj)))[0]
 
-    def _mlp_infer(self, blk, x, wm, w2, eps):
-        """MLP sub-block without autograd (generation / sampler paths). wm: the fc1 | fc3 (swiglu) or fc1 (GELU) operand."""
-        if self.gelu:
-            return _gelu_mlp_fwd(x, blk.norm2.weight.detach(), _ln_bias(blk.norm2), wm, _det(blk.mlp.fc1.bias), w2,
-                                 _det(blk.mlp.fc2.bias), eps)[0]
-        return _mlp_fwd(x, blk.norm2.weight.detach(), wm, w2, eps)[0]
+    def _mlp_infer(self, blk, h, wm):
+        return _mlp_fwd(blk.mlp, h, blk.norm2.weight, _bias(blk.norm2), wm, blk.mlp.params(), self.eps)[0]
+
+    def _decoder_infer(self, h, c, g):
+        """The decoder blocks over h (g.B * g.M rows, fp32). c: the context rows that g.m_x ranges over, or None when no
+        sample has context: a softmax over zero keys times an empty V is exactly 0 (SURVEY.md A5), so each cross-attention
+        then adds only its projection's bias, if it has one."""
+        B, M, D = g.B, g.M, g.D
+        zero = None
+        for i, blk in enumerate(self.decoder):
+            wqkv, wsproj, wq, wkv, wxproj, *wm = self._dec_weights(i)
+            h = self._self_attn_infer(blk.self_attn, blk.norm1, h, wqkv, wsproj, B, M, g.m_dec)
+            xa = blk.cross_attn
+            if c is not None:
+                hq, _, _, _ = ops.layernorm_fwd(h, blk.query_norm.weight, g.eps, save_stats=False, bias=_bias(blk.query_norm))
+                q = ops.linear_fwd(hq, wq, bias=_bias(xa.q))
+                hc, _, _, _ = ops.layernorm_fwd(c, blk.context_norm.weight, g.eps, save_stats=False, bias=_bias(blk.context_norm))
+                kv = ops.linear_fwd(hc, wkv, bias=_bias(xa.kv))
+                o2, _ = ops.attn_fwd(q, kv[:, :D], kv[:, D:], B, g.H, M, g.N, meta=g.m_x, want_lse=False)
+                h = ops.linear_fwd(o2, wxproj, bias=_bias(xa.proj), addend=h, out_dtype=f32)
+            elif _bias(xa.proj) is not None:
+                if zero is None:
+                    zero = torch.zeros(B * M, D, dtype=bf16, device=h.device)
+                h = ops.linear_fwd(zero, wxproj, bias=_bias(xa.proj), addend=h, out_dtype=f32)
+            h = self._mlp_infer(blk, h, wm)
+        return h
 
     # ------------------------------------------------------------------ sampler-facing pieces (reference :251-283,483-551)
     def cat_encoder_tensors(self, mod_dict):
@@ -882,24 +855,15 @@ class EgoM2P(nn.Module):
         g.dec_lo, g.dec_hi = self._prefix_ranges(decoder_attention_mask, B, M, M, y.device)
         g.build_meta(y.device, encoder=False)  # no encoder self-attention on this path
         h = y.reshape(B * M, D).float().contiguous()
-        c = context.reshape(B * N, D).float().contiguous() if N > 0 else torch.zeros(0, D, dtype=f32, device=y.device)
         if N == 0:
-            # Unconditional branch of guided ROAR decoding (generate.py:793-802): no context token at all. Softmax over
-            # zero keys times an empty V is exactly 0, so every block reduces to self-attention + MLP (SURVEY.md A5) plus,
-            # in the GELU / bias family, the cross-attention projection of that zero output: its bias. Inference only.
+            # Unconditional branch of guided ROAR decoding (generate.py:793-802): no context token at all. Inference only.
             if torch.is_grad_enabled() and (y.requires_grad or any(p.requires_grad for p in self.decoder.parameters())):
                 raise NotImplementedError("decoder with an empty context is an inference-only path (wrap it in torch.no_grad())")
-            zero = torch.zeros(B * M, D, dtype=bf16, device=y.device) if self.gelu else None
+            h = self._decoder_infer(h, None, g)
+        else:
+            c = context.reshape(B * N, D).float().contiguous()
             for i, blk in enumerate(self.decoder):
-                wqkv, wsproj, _, _, wxproj, w13, w2 = self._dec_weights(i)
-                h, _ = _self_attn_fwd(h, blk.norm1.weight, wqkv, wsproj, B, M, g.H, g.m_dec, g.eps,
-                                      bias=self._attn_bias(blk.self_attn, blk.norm1))
-                if self.gelu:
-                    h = ops.linear_fwd(zero, wxproj, bias=_det(blk.cross_attn.proj.bias), addend=h, out_dtype=f32)
-                h = self._mlp_infer(blk, h, w13, w2, g.eps)
-            return self.decoder_norm(h).reshape(B, M, D)
-        for i, blk in enumerate(self.decoder):
-            h = self._dec_block(i, blk, h, c, g)
+                h = self._dec_block(i, blk, h, c, g)
         return self.decoder_norm(h).reshape(B, M, D)
 
     def forward_logits(self, y, decoder_mod_dict, decoder_mod_mask, return_all_logits: bool = False):
@@ -932,12 +896,11 @@ class EgoM2P(nn.Module):
         g.enc_hi = ep.n_valid[:, None].expand(B, N).contiguous()
         g.build_meta(dev)
         for i, blk in enumerate(self.encoder):
-            wqkv, wproj, w13, w2 = self._enc_weights(i)
-            x, _ = _self_attn_fwd(x, blk.norm1.weight.detach(), wqkv, wproj, B, N, g.H, g.m_enc, g.eps,
-                                  bias=self._attn_bias(blk.attn, blk.norm1))
-            x = self._mlp_infer(blk, x, w13, w2, g.eps)
+            wqkv, wproj, *wm = self._enc_weights(i)
+            x = self._self_attn_infer(blk.attn, blk.norm1, x, wqkv, wproj, B, N, g.m_enc)
+            x = self._mlp_infer(blk, x, wm)
         h, _, _, _ = ops.layernorm_fwd(x, self.encoder_norm.weight.detach(), self.eps, save_stats=False,
-                                       bias=_ln_bias(self.encoder_norm))
+                                       bias=_det(_bias(self.encoder_norm)))
         context = ops.linear_fwd(h, self._bf16("ctx", self.decoder_proj_context.weight), bias=self.decoder_proj_context.bias.detach(),
                                  addend=emb, out_dtype=f32)
         return context.reshape(B, N, D), ep.n_valid
@@ -952,33 +915,14 @@ class EgoM2P(nn.Module):
         dev = y0.device
         N = 0 if context is None else context.shape[1]
         g = self._geom(B, N, M)
+        c = None
         if N > 0:
             g.x_lo = torch.zeros(B, M, dtype=torch.int32, device=dev)
             g.x_hi = n_ctx.to(torch.int32)[:, None].expand(B, M).contiguous()
             g.m_x = ops.attn_ranges(B, M, N, g.x_lo, g.x_hi, device=dev, empty_zero=True)
             c = context.reshape(B * N, D)
         g.m_dec = ops.attn_ranges(B, M, M, device=dev)
-        h = y0.reshape(B * M, D).float().contiguous()
-        for i, blk in enumerate(self.decoder):
-            wqkv, wsproj, wq, wkv, wxproj, w13, w2 = self._dec_weights(i)
-            h, _ = _self_attn_fwd(h, blk.norm1.weight.detach(), wqkv, wsproj, B, M, g.H, g.m_dec, g.eps,
-                                  bias=self._attn_bias(blk.self_attn, blk.norm1))
-            xa = blk.cross_attn
-            if N > 0:
-                hq, _, _, _ = ops.layernorm_fwd(h, blk.query_norm.weight.detach(), g.eps, save_stats=False, bias=_ln_bias(blk.query_norm))
-                q = ops.linear_fwd(hq, wq, bias=_det(xa.q.bias))
-                hc, _, _, _ = ops.layernorm_fwd(c, blk.context_norm.weight.detach(), g.eps, save_stats=False,
-                                                bias=_ln_bias(blk.context_norm))
-                kv = ops.linear_fwd(hc, wkv, bias=_det(xa.kv.bias))
-                o2, _ = ops.attn_fwd(q, kv[:, :D], kv[:, D:], B, g.H, M, N, meta=g.m_x, want_lse=False)
-                h = ops.linear_fwd(o2, wxproj, bias=_det(xa.proj.bias), addend=h, out_dtype=f32)
-            elif self.gelu:   # no context anywhere: the cross-attention output is 0, its projection is the bias
-                h = ops.linear_fwd(torch.zeros(B * M, D, dtype=bf16, device=dev), wxproj, bias=_det(xa.proj.bias), addend=h,
-                                   out_dtype=f32)
-            h = self._mlp_infer(blk, h, w13, w2, g.eps)
-        _, yn, _, _ = ops.layernorm_fwd(h, self.decoder_norm.weight.detach(), self.eps, out_bf16=False, out_f32=True, save_stats=False,
-                                        bias=_ln_bias(self.decoder_norm))
-        return yn
+        return self.decoder_norm(self._decoder_infer(y0.reshape(B * M, D).float().contiguous(), c, g))
 
     def head_operand(self, mod: str) -> torch.Tensor:
         """Cached bf16 operand of a modality's vocabulary head (V, D)."""
@@ -1120,8 +1064,7 @@ class EgoM2P(nn.Module):
         # ---- encoder
         for i, blk in enumerate(self.encoder):
             x = self._enc_block(i, blk, x, g)
-        context = _ContextFn.apply(x, enc_emb, self.encoder_norm.weight, self.encoder_norm.bias if self.gelu else None,
-                                   self.decoder_proj_context.weight,
+        context = _ContextFn.apply(x, enc_emb, self.encoder_norm.weight, _bias(self.encoder_norm), self.decoder_proj_context.weight,
                                    self.decoder_proj_context.bias, self._bf16("ctx", self.decoder_proj_context.weight), self.eps,
                                    self._epoch)
         # ---- decoder
@@ -1147,7 +1090,7 @@ class EgoM2P(nn.Module):
             w = self.decoder_embeddings[m].to_logits.weight
             heads.append(w)
             wbs.append(self._bf16(("head", m), w))
-        per_mod = _HeadLossFn.apply(y, self.decoder_norm.weight, self.decoder_norm.bias if self.gelu else None, rows, targets, wbs,
+        per_mod = _HeadLossFn.apply(y, self.decoder_norm.weight, _bias(self.decoder_norm), rows, targets, wbs,
                                     self.eps, self._epoch, *heads)
         mod_loss = {}
         for m, l in zip(dec_mods, per_mod):

@@ -312,6 +312,24 @@ def test_forward_hidden_guided_step_against_oracle():
         assert diff < 2e-2, (branch, diff)
 
 
+def test_decoder_without_context_against_oracle():
+    """No context token in any sample (the sampler's call when no branch has conditioning): forward_decoder with N = 0 and
+    decode_tokens(y0, None, None). Each cross-attention then adds only its projection's bias."""
+    s, cfg, sd = _sampler()
+    B, k, D = 2, 5, cfg["dim"]
+    d = "decoder_embeddings.tok_cam."
+    pos = torch.tensor([[7, 11, 29, 5, 20], [0, 3, 4, 17, 28]])
+    y0 = sd["mask_token"] + sd[d + "pos_emb"][0, pos] + sd[d + "mod_emb"]
+    ref = go.forward_decoder(y0, torch.zeros(B, 0, D), None, None, sd, cfg["dec_depth"], cfg["heads"])
+    with torch.no_grad():
+        got = {"forward_decoder": s.model.forward_decoder(y0.cuda(), torch.zeros(B, 0, D, device="cuda"), None, None),
+               "decode_tokens": s.model.decode_tokens(y0.cuda(), None, None).reshape(B, k, D)}
+    head = sd[d + "to_logits.weight"]
+    for name, yn in got.items():
+        diff = float((F.linear(yn.cpu(), head) - F.linear(ref, head)).abs().max())
+        assert diff < 2e-2, (name, diff)
+
+
 def test_generate_rgb_to_cam_guided():
     from egom2p_b200.generate import build_chained_generation_schedules, init_empty_target_modality, init_full_input_modality
     s, cfg, _ = _sampler()
