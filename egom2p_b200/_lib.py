@@ -59,7 +59,7 @@ SIGNATURES = {
     "egom2p_cast_f32_to_bf16_multi": [vp, i32, i64, vp],
     "egom2p_add_f32": [vp, vp, i64, vp, vp, vp],
     "egom2p_sumsq_multi": [vp, i32, i64, vp, vp, vp],
-    "egom2p_adamw_multi": [vp, i32, i64, f32, f32, f32, vp, vp, f32, vp],
+    "egom2p_adamw_multi_steps": [vp, i32, i64, f32, f32, f32, vp, vp, f32, vp],
     "egom2p_image_masks": [vp, C.c_uint64, C.c_uint64, i32, i32, i32, vp, vp, vp, vp, vp, vp],
     "egom2p_sample_rows": [vp, i64, i32, i32, f32, f32, i32, vp, vp, vp, vp, vp],
     "egom2p_cfg_combine_bf16": [vp, vp, i64, f32, vp, vp],

@@ -122,7 +122,7 @@ struct OptItem {
 static_assert(sizeof(OptItem) == 56, "OptItem layout is part of the C ABI (egom2p_opt_item)");
 constexpr int kOptChunk = 8192;
 
-__device__ __forceinline__ OptItem find_item(const OptItem* __restrict__ items, int n_items, OptItem* sh) {
+__device__ __forceinline__ OptItem find_item(const OptItem* __restrict__ items, int n_items, OptItem* sh, int* sh_idx = nullptr) {
   if (threadIdx.x == 0) {
     int lo = 0, hi = n_items - 1;
     while (lo < hi) {  // last item with first_chunk <= blockIdx.x
@@ -130,6 +130,7 @@ __device__ __forceinline__ OptItem find_item(const OptItem* __restrict__ items, 
       if (items[mid].first_chunk <= (int64_t)blockIdx.x) lo = mid; else hi = mid - 1;
     }
     *sh = items[lo];
+    if (sh_idx) *sh_idx = lo;
   }
   __syncthreads();
   return *sh;
@@ -187,17 +188,23 @@ __device__ __forceinline__ void adamw_one(float& p, float g, float& m, float& v,
   p -= step_size * (m / denom);
 }
 
-// step_dev holds the number of steps taken BEFORE this one (incremented by step_inc_kernel afterwards), so that the whole
-// tail is capturable in a CUDA graph: no host-side scalar changes from step to step.
+// steps[i] holds the number of steps item i took BEFORE this one (torch.optim.AdamW counts per tensor: a tensor that sat out
+// steps with no gradient starts its bias correction where it left off). steps_inc_kernel advances the counts afterwards, in a
+// launch of its own because every chunk of an item reads its count; nothing host-side changes from step to step, so the
+// whole tail is capturable in a CUDA graph.
 __global__ void __launch_bounds__(kEwThreads) adamw_multi_kernel(const OptItem* __restrict__ items, int n_items, float b1, float b2,
-                                                                 float eps, const int32_t* __restrict__ step_dev,
+                                                                 float eps, const int32_t* __restrict__ steps,
                                                                  const float* __restrict__ sumsq, float max_norm) {
   __shared__ OptItem sh_it;
-  const OptItem it = find_item(items, n_items, &sh_it);
-  const float t = (float)(*step_dev + 1);
+  __shared__ int sh_idx;
+  const OptItem it = find_item(items, n_items, &sh_it, &sh_idx);
+  const float t = (float)(steps[sh_idx] + 1);
   const float bc1 = 1.f - powf(b1, t), inv_bc2_sqrt = rsqrtf(1.f - powf(b2, t));
   float gs = 1.f;
-  if (sumsq) gs = fminf(1.f, max_norm / (sqrtf(*sumsq) + 1e-6f));   // torch.nn.utils.clip_grad_norm_
+  if (sumsq) {   // torch.nn.utils.clip_grad_norm_: clamp(max = 1) keeps a NaN ratio NaN, so a NaN norm poisons every update
+    const float c = max_norm / (sqrtf(*sumsq) + 1e-6f);
+    gs = c > 1.f ? 1.f : c;
+  }
   const float step_size = it.lr / bc1;
   const int64_t e0 = ((int64_t)blockIdx.x - it.first_chunk) * kOptChunk;
   const int ne = (int)min((int64_t)kOptChunk, it.n - e0);
@@ -229,7 +236,10 @@ __global__ void __launch_bounds__(kEwThreads) adamw_multi_kernel(const OptItem* 
     p[i] = pi; m[i] = mi; v[i] = vi;
   }
 }
-__global__ void step_inc_kernel(int32_t* step) { *step += 1; }
+__global__ void steps_inc_kernel(int32_t* __restrict__ steps, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) steps[i] += 1;
+}
 
 // out[c] += sum_r x[r, c]; each CTA reduces a 64-row slab, threads own columns (coalesced), one atomic per column.
 __global__ void __launch_bounds__(kEwThreads) colsum_kernel(const float* __restrict__ x, int64_t rows, int cols, float* __restrict__ out) {
@@ -362,14 +372,14 @@ extern "C" int egom2p_sumsq_multi(const void* items_dev, int32_t n_items, int64_
   sumsq_finalize_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(partials, n_chunks, sumsq);
   return check_launch("sumsq_multi finalize");
 }
-extern "C" int egom2p_adamw_multi(const void* items_dev, int32_t n_items, int64_t n_chunks, float beta1, float beta2, float eps,
-                                  int32_t* step_dev, const float* sumsq, float max_norm, void* stream) {
+extern "C" int egom2p_adamw_multi_steps(const void* items_dev, int32_t n_items, int64_t n_chunks, float beta1, float beta2,
+                                        float eps, int32_t* steps, const float* sumsq, float max_norm, void* stream) {
   using namespace egom2p;
-  EGO_REQUIRE(items_dev && step_dev && n_items > 0 && n_chunks > 0 && n_chunks < (int64_t)INT32_MAX, "adamw_multi: bad argument");
+  EGO_REQUIRE(items_dev && steps && n_items > 0 && n_chunks > 0 && n_chunks < (int64_t)INT32_MAX, "adamw_multi_steps: bad argument");
   adamw_multi_kernel<<<(unsigned)n_chunks, kEwThreads, 0, (cudaStream_t)stream>>>(reinterpret_cast<const OptItem*>(items_dev), n_items,
-                                                                                 beta1, beta2, eps, step_dev, sumsq, max_norm);
-  int rc = check_launch("adamw_multi");
+                                                                                 beta1, beta2, eps, steps, sumsq, max_norm);
+  int rc = check_launch("adamw_multi_steps");
   if (rc) return rc;
-  step_inc_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(step_dev);
-  return check_launch("adamw_multi step");
+  steps_inc_kernel<<<(unsigned)((n_items + kEwThreads - 1) / kEwThreads), kEwThreads, 0, (cudaStream_t)stream>>>(steps, n_items);
+  return check_launch("adamw_multi_steps increment");
 }

@@ -3,7 +3,7 @@
 At the reference's own batch size (4 per GPU, cfgs/default/egom2p/models/main/ego-b_mod4_500b_clariden_2048_camcv_depthdenoise.yaml:9)
 one step is ~1100 kernel launches of 5-50 us each: issued one at a time from Python the step is bound by the host, not the
 GPU (round 1: 33.6 ms / step at b = 4 against ~24 ms of kernel time). `GraphedTrainStep` captures forward + backward +
-gradient-norm clip + AdamW (egom2p_b200.optim.FusedAdamW, whose step counter lives on the device) ONCE into a CUDA graph and
+gradient-norm clip + AdamW (egom2p_b200.optim.FusedAdamW, whose step counts live on the device) ONCE into a CUDA graph and
 replays it per step: inputs are copied into static buffers, the loss is read from a static tensor.
 
 What a captured step fixes (checked, not assumed):
@@ -27,7 +27,7 @@ class GraphedTrainStep:
     def __init__(self, model, optimizer: FusedAdamW, example_md: Dict[str, Dict[str, torch.Tensor]], num_encoder_tokens: int,
                  num_decoder_tokens: int, clip_grad: Optional[float] = 1.0, loss_type: str = "mod", warmup: int = 3):
         if not isinstance(optimizer, FusedAdamW):
-            raise TypeError("GraphedTrainStep needs egom2p_b200.optim.FusedAdamW (device-side step counter)")
+            raise TypeError("GraphedTrainStep needs egom2p_b200.optim.FusedAdamW (device-side step counts)")
         self.model, self.opt = model, optimizer
         self.n_enc, self.n_dec, self.clip, self.loss_type = num_encoder_tokens, num_decoder_tokens, clip_grad, loss_type
         dev = next(model.parameters()).device
@@ -47,9 +47,13 @@ class GraphedTrainStep:
         model.fixed_decoder_order = random.sample(mods, len(mods))
         model.static_target_rows = rows
 
-        # ---- warm-up on a side stream (allocator, lazy state, cudaFuncSetAttribute), then undo its effect on the weights
+        # ---- warm-up on a side stream (allocator, lazy state, cudaFuncSetAttribute), then undo its effect on the weights and on
+        # the optimizer state: moments and step counts the optimizer arrived with (e.g. after a resume) are restored, state the
+        # warm-up created is left as zero moments at step 0
         params = [p for p in model.parameters() if p.requires_grad]
         backup = [p.detach().clone() for p in params]
+        opt_backup = {p: {k: optimizer.state[p][k].detach().clone() for k in ("exp_avg", "exp_avg_sq", "step")}
+                      for p in params if "exp_avg" in optimizer.state.get(p, {})}
         s = torch.cuda.Stream(device=dev)
         s.wait_stream(torch.cuda.current_stream(dev))
         with torch.cuda.stream(s):
@@ -62,10 +66,12 @@ class GraphedTrainStep:
                 p.copy_(b)
                 st = optimizer.state.get(p)
                 if st:
-                    st["exp_avg"].zero_()
-                    st["exp_avg_sq"].zero_()
-            optimizer._step_dev.zero_()
-        del backup
+                    for k in ("exp_avg", "exp_avg_sq", "step"):
+                        if p in opt_backup:
+                            st[k].copy_(opt_backup[p][k])
+                        else:
+                            st[k].zero_()
+        del backup, opt_backup
         model.invalidate_weight_cache()
         optimizer.zero_grad(set_to_none=True)
 

@@ -216,9 +216,13 @@ int egom2p_add_f32(const float* a, const float* b, int64_t n, float* out, uint16
  * ceil(n / 8192) over the items before i, n_chunks = the total.
  *   egom2p_sumsq_multi: *sumsq = sum over all items of sum(g^2); deterministic (per-chunk partial sums in `partials`,
  *     n_chunks floats of scratch, added in a fixed order) so that data-parallel replicas compute identical clip factors.
- *   egom2p_adamw_multi: torch.optim.AdamW update of every item with its own lr / weight decay; the gradient is read as
- *     g * min(1, max_norm / (sqrt(*sumsq) + 1e-6)) when sumsq != NULL (clip folded in: gradients are not rewritten);
- *     bias corrections use *step_dev + 1, and *step_dev is incremented afterwards (CUDA-graph capturable). */
+ *   egom2p_adamw_multi_steps: torch.optim.AdamW update of every item with its own lr / weight decay; the gradient is read as
+ *     g * min(1, max_norm / (sqrt(*sumsq) + 1e-6)) when sumsq != NULL (clip folded in: gradients are not rewritten; a NaN
+ *     norm gives a NaN coefficient, as torch's clamp does). `steps` is a device array of n_items int32 step counts, one per
+ *     item: item i's bias corrections use steps[i] + 1, and steps[0 .. n_items) are incremented afterwards (CUDA-graph
+ *     capturable). It replaces egom2p_adamw_multi, which read one count shared by all items from the same argument
+ *     position: the old symbol is gone, so a caller built against it fails to resolve it instead of passing a single
+ *     counter where an array is read, and the ABI version is unchanged. */
 typedef struct {
   float* param;
   const float* grad;
@@ -229,8 +233,8 @@ typedef struct {
   float lr, weight_decay;
 } egom2p_opt_item;
 int egom2p_sumsq_multi(const void* items_dev, int32_t n_items, int64_t n_chunks, float* partials, float* sumsq, void* stream);
-int egom2p_adamw_multi(const void* items_dev, int32_t n_items, int64_t n_chunks, float beta1, float beta2, float eps,
-                       int32_t* step_dev, const float* sumsq, float max_norm, void* stream);
+int egom2p_adamw_multi_steps(const void* items_dev, int32_t n_items, int64_t n_chunks, float beta1, float beta2, float eps,
+                             int32_t* steps, const float* sumsq, float max_norm, void* stream);
 /* out[c] += sum_r x[r, c] -- bias gradient of decoder_proj_context (egom2p_model.py:157,722). */
 int egom2p_colsum_f32(const float* x, int64_t rows, int32_t cols, float* out, void* stream);
 /* out[c] += sum_r x[r, c] for a bf16 (rows, cols) matrix of row pitch ld (cols, ld multiples of 8): the bias gradients of
