@@ -310,7 +310,12 @@ __global__ void __launch_bounds__(kSmpThreads, 1) sample_rows_kernel(SampleParam
   float w4[4];
 #pragma unroll
   for (int c = 0; c < 4; ++c) w4[c] = (v0 + c < p.V && tk.keep(q[c]) && tp.keep(q[c])) ? __expf((q[c] - gmax) * invT) : 0.f;
-  if (myw > 0.f && pre <= target && target < pre + myw) {
+  // The owner of the target is the first thread, in token order, with weight whose inclusive prefix pre + myw exceeds it
+  // (searchsorted). Claiming pre <= target < pre + myw instead would leave gaps: the next thread's pre comes out of the scan
+  // along a different rounding path than pre + myw and can exceed it by an ulp. The first candidate of every warp enters
+  // a block min-reduction over token indices.
+  const unsigned cand = __ballot_sync(0xffffffffu, myw > 0.f && target < pre + myw);
+  if (cand != 0u && (t & 31) == __ffs(cand) - 1) {
     float cacc = pre;
     int pick = -1;
 #pragma unroll
@@ -323,7 +328,7 @@ __global__ void __launch_bounds__(kSmpThreads, 1) sample_rows_kernel(SampleParam
     atomicMin(&s_i, v0 + pick);
   }
   __syncthreads();
-  if (s_i == 0x7fffffff) {   // the target fell into a rounding gap between threads: last kept token of the chunk
+  if (s_i == 0x7fffffff) {   // the target lies past the chunk's last bound (chunk sums and scan round differently): its last kept token
     __syncthreads();
     if (t == 0) s_i = -1;
     __syncthreads();

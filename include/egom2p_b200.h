@@ -265,8 +265,11 @@ int egom2p_image_masks(const float* noise, uint64_t seed, uint64_t offset, int32
  * then top-p on softmax(remaining) at temperature 1 (a token is removed when the mass ranked strictly above it exceeds
  * top_p; 0 = off), then one draw from softmax(kept / temperature) -- here by inverse CDF in ascending token order with the
  * uniform u[row] in [0, 1); temperature == 0: argmax, prob 1. No sort and no second copy of the logits: threshold search by
- * nested 2048-bin mass histograms. Outputs: token (rows) int64, prob (rows) fp32 of the drawn token (may be NULL),
- * n_kept (rows) int32 size of the filtered set (may be NULL). V <= 65536. */
+ * nested 2048-bin mass histograms. The filtered set is always the n_kept largest logits, and tokens of equal logit are kept
+ * or removed together: at top-k this is the reference's rule (nothing equal to the k-th value is removed); at top-p, where
+ * the reference's stable sort keeps only the lower-index part of a tie group that straddles top_p, the whole group is kept.
+ * Outputs: token (rows) int64, prob (rows) fp32 of the drawn token (may be NULL), n_kept (rows) int32 size of the filtered
+ * set (may be NULL). V <= 65536. */
 int egom2p_sample_rows(const float* logits, int64_t ld, int32_t rows, int32_t V, float temperature, float top_p,
                        int32_t top_k, const float* u, int64_t* token, float* prob, int32_t* n_kept, void* stream);
 /* out = bf16(y_uncond + (y_cond - y_uncond) * scale): classifier-free guidance (generate.py:804) applied to the decoder
