@@ -172,7 +172,7 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
       }
     }
   }
-  if (!kBias && !dw) return;
+  if (!dw && !db) return;  // a frozen LayerNorm: no reduction (db is null in the no-bias instantiation)
 #pragma unroll
   for (int j = 0; j < NV; ++j) {
     const int i = lane + j * 32;
@@ -183,8 +183,8 @@ __global__ void __launch_bounds__(128, 4) ln_bwd_kernel(const void* __restrict__
     float t = 0.f;
 #pragma unroll
     for (int wi = 0; wi < 4; ++wi) t += s_dw[wi * dim + c];
-    if (!kBias || dw) atomicAdd(dw + c, t);
-    if (kBias) {
+    if (dw) atomicAdd(dw + c, t);
+    if (kBias && db) {
       float tb = 0.f;
 #pragma unroll
       for (int wi = 4; wi < 8; ++wi) tb += s_dw[wi * dim + c];
@@ -215,7 +215,8 @@ static int layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const flo
                          const float* rstd, const float* dx_in, int64_t rows, int32_t dim, float* dx_out, uint16_t* dx_bf16,
                          float* d_weight, float* d_bias, void* stream) {
   EGO_REQUIRE((dy_bf16 != nullptr) != (dy_f32 != nullptr), "layernorm_bwd: exactly one of dy_bf16 / dy_f32");
-  EGO_REQUIRE(x && weight && mean && rstd && dx_out && rows > 0 && (!kBias || d_bias), "layernorm_bwd: null argument");
+  // d_weight / d_bias may each be null: the gradient of a frozen LayerNorm parameter is not reduced
+  EGO_REQUIRE(x && weight && mean && rstd && dx_out && rows > 0, "layernorm_bwd: null argument");
   EGO_REQUIRE(dim % 4 == 0 && dim > 0 && dim <= kLnMaxVec * 128, "layernorm_bwd: dim %d unsupported", dim);
   const int rows_per_cta = 16;
   const unsigned grid = (unsigned)((rows + rows_per_cta - 1) / rows_per_cta);

@@ -77,7 +77,8 @@ class _Linear(nn.Linear):
 
 # The MLP is the only part of a block that differs between the two families. Each MLP container owns, for the shared block
 # code: params() -- its parameters, in the order the block functions take them; operands() -- their cached bf16 GEMM
-# operands; fwd() -- x1 + MLP(h2) from the normed h2, and what bwd() needs; bwd() -- dh2 and the gradients of params().
+# operands; fwd() -- x1 + MLP(h2) from the normed h2, and what bwd() needs; bwd() -- dh2 and the gradients of params(), None
+# for each parameter whose flag in `need` is False (a frozen parameter gets neither its wgrad GEMM nor its bias column sum).
 class GatedMlp(nn.Module):
     """fc2(SiLU(fc1 x) * fc3 x) without biases (the swiglu / no-bias family). fc1 and fc3 run as one GEMM over an operand
     with their rows interleaved (EgoM2P._bf16), the gate in its epilogue."""
@@ -100,15 +101,16 @@ class GatedMlp(nn.Module):
         ab, g = ops.gemm_swiglu_fwd(h2, w13)   # fc1|fc3 GEMM with the SwiGLU gate in its epilogue
         return ops.linear_fwd(g, w2, addend=x1, out_dtype=f32), (ab, g)
 
-    def bwd(self, dx2b, h2, w, saved):
+    def bwd(self, dx2b, h2, w, saved, need):
         (w13, w2), (ab, g) = w, saved
-        dw2 = ops.linear_wgrad(dx2b, g)
+        n1, n2, n3 = need
+        dw2 = ops.linear_wgrad(dx2b, g) if n2 else None
         dab = ops.gemm_swiglu_bwd(dx2b, w2, ab)   # fc2 dgrad with the SwiGLU derivative in its epilogue
-        dw13 = ops.linear_wgrad(dab, h2)
+        dw13 = ops.linear_wgrad(dab, h2) if (n1 or n3) else None   # one interleaved GEMM for fc1 and fc3
         dh2 = ops.linear_dgrad(dab, w13)
         F = self.fc1.out_features
-        d1, d3 = _split_w13_grad(dw13, F)
-        return dh2, (d1, dw2[:, :F], d3)
+        d1, d3 = _split_w13_grad(dw13, F) if dw13 is not None else (None, None)
+        return dh2, (d1 if n1 else None, dw2[:, :F] if n2 else None, d3 if n3 else None)
 
 
 class Mlp(nn.Module):
@@ -130,13 +132,14 @@ class Mlp(nn.Module):
         u, a = ops.gemm_gelu_fwd(h2, w1, b1)   # fc1 GEMM with + b1 and GELU in its epilogue
         return ops.linear_fwd(a, w2, bias=b2, addend=x1, out_dtype=f32), (u, a)
 
-    def bwd(self, dx2b, h2, w, saved):
+    def bwd(self, dx2b, h2, w, saved, need):
         (w1, w2), (u, a) = w, saved
-        dw2 = ops.linear_wgrad(dx2b, a)
-        db2 = ops.colsum_bf16(dx2b)
+        n1, nb1, n2, nb2 = need
+        dw2 = ops.linear_wgrad(dx2b, a) if n2 else None
+        db2 = ops.colsum_bf16(dx2b) if nb2 else None
         du = ops.gemm_gelu_bwd(dx2b, w2, u)   # fc2 dgrad with GELU'(u) in its epilogue
-        dw1 = ops.linear_wgrad(du, h2)
-        db1 = ops.colsum_bf16(du)
+        dw1 = ops.linear_wgrad(du, h2) if n1 else None
+        db1 = ops.colsum_bf16(du) if nb1 else None
         return ops.linear_dgrad(du, w1), (dw1, db1, dw2, db2)
 
 
@@ -243,10 +246,6 @@ def _bf16_of(dx):
     return ops.cast_bf16(dx)
 
 
-def _present(*biases):
-    return tuple(b is not None for b in biases)
-
-
 def _mlp_fwd(mlp, x1, n2w, n2b, w, params, eps):
     """x1 + mlp(norm2 x1). w: the MLP's bf16 operands (mlp.operands), params: its parameters (mlp.params)."""
     h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps, bias=n2b)
@@ -254,13 +253,14 @@ def _mlp_fwd(mlp, x1, n2w, n2b, w, params, eps):
     return x2, (mean2, rstd2, h2, *sm)
 
 
-def _mlp_bwd(mlp, dx2, x1, n2w, has_n2b, w, saved):
-    """Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b (None without a norm2 bias) and the gradients of
-    mlp.params()."""
+def _mlp_bwd(mlp, dx2, x1, n2w, w, saved, need):
+    """need: whether norm2's weight and bias, then each of mlp.params(), want a gradient (False for an absent bias).
+    Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b and the gradients of mlp.params(), None where not
+    wanted."""
     mean2, rstd2, h2, *sm = saved
-    dh2, dparams = mlp.bwd(_bf16_of(dx2), h2, w, sm)
-    dn2w = _zeros(n2w.numel(), dx2.device)
-    dn2b = _zeros(n2w.numel(), dx2.device) if has_n2b else None
+    dh2, dparams = mlp.bwd(_bf16_of(dx2), h2, w, sm, need[2:])
+    dn2w = _zeros(n2w.numel(), dx2.device) if need[0] else None
+    dn2b = _zeros(n2w.numel(), dx2.device) if need[1] else None
     dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True, d_bias=dn2b)
     return dx1, dx1b, dn2w, dn2b, dparams
 
@@ -276,23 +276,23 @@ def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs, bias):
     return x1, (mean1, rstd1, h1, qkv, o, lse)
 
 
-def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs, has_bias):
-    """has_bias: whether norm1, qkv and proj have a bias. Returns dx, dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, with None
-    for the gradient of an absent bias."""
+def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs, need):
+    """need: whether the weight and bias of norm1, qkv and proj want a gradient (False for an absent bias). Returns dx,
+    dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, None for each gradient not wanted."""
     mean1, rstd1, h1, qkv, o, lse = saved
     D = x.shape[-1]
-    dwproj = ops.linear_wgrad(dx1b, o)
+    need_n1w, need_n1b, need_wqkv, need_bqkv, need_wproj, need_bproj = need
+    dwproj = ops.linear_wgrad(dx1b, o) if need_wproj else None
     do = ops.linear_dgrad(dx1b, wproj)
     dqkv = torch.empty_like(qkv)
     ops.attn_bwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], o, do, lse, B, H, L, L, dqkv[:, :D], dqkv[:, D:2 * D],
                  dqkv[:, 2 * D:], meta=meta, pairs=pairs)
-    dwqkv = ops.linear_wgrad(dqkv, h1)
+    dwqkv = ops.linear_wgrad(dqkv, h1) if need_wqkv else None
     dh1 = ops.linear_dgrad(dqkv, wqkv)
-    has_n1b, has_bqkv, has_bproj = has_bias
-    dn1w = _zeros(n1w.numel(), x.device)
-    dn1b = _zeros(n1w.numel(), x.device) if has_n1b else None
-    dbqkv = ops.colsum_bf16(dqkv) if has_bqkv else None
-    dbproj = ops.colsum_bf16(dx1b) if has_bproj else None
+    dn1w = _zeros(n1w.numel(), x.device) if need_n1w else None
+    dn1b = _zeros(n1w.numel(), x.device) if need_n1b else None
+    dbqkv = ops.colsum_bf16(dqkv) if need_bqkv else None
+    dbproj = ops.colsum_bf16(dx1b) if need_bproj else None
     dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True, d_bias=dn1b)
     return _with_bf16(dx, dxb), dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj
 
@@ -311,33 +311,42 @@ def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias):
     return y2, (meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2)
 
 
-def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, has_bias):
-    """Backward of _cross_fwd. has_bias: whether query_norm, context_norm, q, kv and proj have a bias. Returns dy1, dy1b,
-    dctx (None unless this block returns the summed context gradient), then dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv,
-    dwxproj, dbxproj, with None for the gradient of an absent bias."""
+def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, need, need_ctx):
+    """Backward of _cross_fwd. need: whether the weight and bias of query_norm, context_norm, q, kv and proj want a gradient
+    (False for an absent bias); need_ctx: whether `context` does. Returns dy1, dy1b, dctx (None unless this block returns
+    the summed context gradient), then dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj, None for each
+    gradient not wanted."""
     meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2 = saved
     D = y1.shape[-1]
     dev = y1.device
-    dwxproj = ops.linear_wgrad(dy2b, o2)
+    need_qnw, need_qnb, need_cnw, need_cnb, need_wq, need_bq, need_wkv, need_bkv, need_wxproj, need_bxproj = need
+    # the context side (kv dgrad, context_norm backward) runs for the context's gradient or for context_norm's own
+    ctx_side = need_ctx or need_cnw or need_cnb
+    dwxproj = ops.linear_wgrad(dy2b, o2) if need_wxproj else None
     do2 = ops.linear_dgrad(dy2b, wxproj)
     dq = torch.empty_like(q)
     dkv = torch.empty_like(kv)
     ops.attn_bwd(q, kv[:, :D], kv[:, D:], o2, do2, lse2, g.B, g.H, g.M, g.N, dq, dkv[:, :D], dkv[:, D:], meta=g.m_x, pairs=g.p_x)
-    dwq = ops.linear_wgrad(dq, hq)
+    dwq = ops.linear_wgrad(dq, hq) if need_wq else None
     dhq = ops.linear_dgrad(dq, wq)
-    dwkv = ops.linear_wgrad(dkv, hc)
-    dhc = ops.linear_dgrad(dkv, wkv)
-    has_qnb, has_cnb, has_bq, has_bkv, has_bxproj = has_bias
-    dqnw, dcnw = _zeros(D, dev), _zeros(D, dev)
-    dqnb = _zeros(D, dev) if has_qnb else None
-    dcnb = _zeros(D, dev) if has_cnb else None
-    dbq = ops.colsum_bf16(dq) if has_bq else None
-    dbkv = ops.colsum_bf16(dkv) if has_bkv else None
-    dbxproj = ops.colsum_bf16(dy2b) if has_bxproj else None
+    dwkv = ops.linear_wgrad(dkv, hc) if need_wkv else None
+    dhc = ops.linear_dgrad(dkv, wkv) if ctx_side else None
+    dqnw = _zeros(D, dev) if need_qnw else None
+    dcnw = _zeros(D, dev) if need_cnw else None
+    dqnb = _zeros(D, dev) if need_qnb else None
+    dcnb = _zeros(D, dev) if need_cnb else None
+    dbq = ops.colsum_bf16(dq) if need_bq else None
+    dbkv = ops.colsum_bf16(dkv) if need_bkv else None
+    dbxproj = ops.colsum_bf16(dy2b) if need_bxproj else None
     dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True, d_bias=dqnb)
+    if not need_ctx:
+        if ctx_side:   # only context_norm's parameter reductions are wanted; its dx is discarded
+            ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, d_weight=dcnw, d_bias=dcnb)
+        return dy1, dy1b, None, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj
     # All decoder blocks read the same `context`: instead of letting autograd add twelve (B*N, D) fp32 gradients pairwise,
     # each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block that runs last
-    # returns it. Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
+    # returns it. g.ctx_users counts the blocks whose forward saw a context that wants a gradient (_DecoderBlockFn.forward).
+    # Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
     acc = g.dctx_acc
     chained = g.ctx_users > 0 and (acc is None or (acc[0] == ctx_key and acc[1].shape == context.shape))
     last = chained and g.ctx_users == 1
@@ -356,7 +365,8 @@ def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sa
 
 class _EncoderBlockFn(torch.autograd.Function):
     """x + attn(norm1 x) then + mlp(norm2 .) -- egom2p_utils.py:356-359. Parameters: weight and bias of norm1, qkv, proj and
-    norm2, then mlp.params(); an absent bias is None and gets None as its gradient."""
+    norm2, then mlp.params(); an absent bias is None. The backward computes the gradient of a parameter only when it
+    requires one (ctx.needs_input_grad): a frozen parameter gets None and no work is launched for it. dx is always computed."""
 
     @staticmethod
     def forward(ctx, x, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, n2w, n2b, *mlp_params):
@@ -365,7 +375,6 @@ class _EncoderBlockFn(torch.autograd.Function):
         x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, g.B, g.N, g.H, g.m_enc, g.eps, g.p_enc, (n1b, qkv_b, proj_b))
         x2, sm = _mlp_fwd(mlp, x1, n2w, n2b, wm, mlp_params, g.eps)
         ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
-        ctx.sa_bias, ctx.n2_bias = _present(n1b, qkv_b, proj_b), n2b is not None
         ctx.op_epoch = geom.epoch_ref[0]
         ctx.save_for_backward(x, n1w, n2w, x1, *sa, *sm)
         return x2
@@ -378,15 +387,17 @@ class _EncoderBlockFn(torch.autograd.Function):
         sa, sm = rest[:6], rest[6:]
         wqkv, wproj, *wm = ctx.wb
         g = ctx.geom
-        dx1, dx1b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dx2.contiguous(), x1, n2w, ctx.n2_bias, wm, sm)
-        dx, *dsa = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc, ctx.sa_bias)
+        need = ctx.needs_input_grad
+        dx1, dx1b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dx2.contiguous(), x1, n2w, wm, sm, need[10:])
+        dx, *dsa = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc, need[4:10])
         return (dx, None, None, None, *dsa, dn2w, dn2b, *dmlp)
 
 
 class _DecoderBlockFn(torch.autograd.Function):
     """self-attn -> cross-attn(query_norm y, context_norm ctx) -> mlp -- egom2p_utils.py:387-391. Parameters: weight and bias
     of norm1, qkv, self-attention proj, query_norm, context_norm, q, kv, cross-attention proj and norm2, then
-    mlp.params(); an absent bias is None and gets None as its gradient."""
+    mlp.params(); an absent bias is None. As in _EncoderBlockFn, only the parameters that require a gradient get one. dy is
+    always computed; the context's gradient (kv dgrad + context_norm backward) only when `context` requires one."""
 
     @staticmethod
     def forward(ctx, y, context, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, sproj_w, sproj_b, qnw, qnb, cnw, cnb, q_w, q_b, kv_w,
@@ -397,11 +408,10 @@ class _DecoderBlockFn(torch.autograd.Function):
         y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, (qnb, cnb, q_b, kv_b, xproj_b))
         y3, sm = _mlp_fwd(mlp, y2, n2w, n2b, wm, mlp_params, g.eps)
         ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
-        ctx.sa_bias, ctx.x_bias = _present(n1b, qkv_b, sproj_b), _present(qnb, cnb, q_b, kv_b, xproj_b)
-        ctx.n2_bias = n2b is not None
         ctx.op_epoch = geom.epoch_ref[0]
         ctx.ctx_key = context.data_ptr()
-        g.ctx_users += 1
+        if ctx.needs_input_grad[1]:   # this block's backward adds to the summed context gradient (_cross_bwd)
+            g.ctx_users += 1
         ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, *sx, *sa, *sm)
         return y3
 
@@ -413,20 +423,22 @@ class _DecoderBlockFn(torch.autograd.Function):
         sx, sa, sm = rest[:10], rest[10:16], rest[16:]
         wqkv, wsproj, wq, wkv, wxproj, *wm = ctx.wb
         g = ctx.geom
-        dy2, dy2b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dy3.contiguous(), y2, n2w, ctx.n2_bias, wm, sm)
-        dy1, dy1b, dctx, *dxa = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, ctx.x_bias)
-        dy, *dsa = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec, ctx.sa_bias)
+        need = ctx.needs_input_grad
+        dy2, dy2b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dy3.contiguous(), y2, n2w, wm, sm, need[21:])
+        dy1, dy1b, dctx, *dxa = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, need[11:21],
+                                           need[1])
+        dy, *dsa = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec, need[5:11])
         return (dy, dctx, None, None, None, *dsa, *dxa, dn2w, dn2b, *dmlp)
 
 
 class _ContextFn(torch.autograd.Function):
     """context = decoder_proj_context(encoder_norm(x)) + encoder_emb -- egom2p_model.py:499,722. norm_b: encoder_norm's
-    bias (GELU / bias family) or None."""
+    bias (GELU / bias family) or None. The backward skips the projection's dw / db when frozen, and the dgrad and
+    encoder_norm backward when neither x nor encoder_norm wants a gradient."""
 
     @staticmethod
     def forward(ctx, x, enc_emb, norm_w, norm_b, proj_w, proj_b, wb, eps, epoch_ref):
         h, _, mean, rstd = ops.layernorm_fwd(x, norm_w, eps, bias=norm_b)
-        ctx.has_nb = norm_b is not None
         context = ops.linear_fwd(h, wb, bias=proj_b, addend=enc_emb, out_dtype=f32)
         ctx.wb = wb
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
@@ -438,15 +450,20 @@ class _ContextFn(torch.autograd.Function):
         _GRAD_GEN[0] += 1
         _check_epoch(ctx.epoch_ref, ctx.op_epoch)
         x, norm_w, mean, rstd, h = ctx.saved_tensors
+        need_x, need_emb, need_nw, need_nb, need_pw, need_pb = ctx.needs_input_grad[:6]
+        upstream = need_x or need_nw or need_nb
         dctx = dctx.contiguous()
-        dcb = _bf16_of(dctx)
-        dw = ops.linear_wgrad(dcb, h)
-        db = ops.colsum(dctx, _zeros(dctx.shape[1], dctx.device))
-        dh = ops.linear_dgrad(dcb, ctx.wb)
-        dnw = _zeros(norm_w.numel(), x.device)
-        dnb = _zeros(norm_w.numel(), x.device) if ctx.has_nb else None
-        dx, dxb = ops.layernorm_bwd(dh, x, norm_w, mean, rstd, d_weight=dnw, want_bf16=True, d_bias=dnb)
-        return _with_bf16(dx, dxb), dctx, dnw, dnb, dw, db, None, None, None
+        dcb = _bf16_of(dctx) if (need_pw or upstream) else None
+        dw = ops.linear_wgrad(dcb, h) if need_pw else None
+        db = ops.colsum(dctx, _zeros(dctx.shape[1], dctx.device)) if need_pb else None
+        dx = dnw = dnb = None
+        if upstream:
+            dh = ops.linear_dgrad(dcb, ctx.wb)
+            dnw = _zeros(norm_w.numel(), x.device) if need_nw else None
+            dnb = _zeros(norm_w.numel(), x.device) if need_nb else None
+            dx, dxb = ops.layernorm_bwd(dh, x, norm_w, mean, rstd, d_weight=dnw, want_bf16=need_x, d_bias=dnb)
+            dx = _with_bf16(dx, dxb) if need_x else None
+        return dx, dctx if need_emb else None, dnw, dnb, dw, db, None, None, None
 
 
 class _EmbedFn(torch.autograd.Function):
@@ -479,29 +496,32 @@ class _EmbedFn(torch.autograd.Function):
         mods = ctx.saved_tensors
         dev = dx0.device
         dx0 = dx0.contiguous()
-        d_mods = [_zeros(dim, dev) for _ in range(n)]
+        # a frozen table, mask token or modality embedding gets no gradient buffer: the kernel skips null outputs
+        need = ctx.needs_input_grad[3:]
+        d_mods = [_zeros(dim, dev) if nd else None for nd in need[len(need) - n:]]
         if ctx.is_decoder:
-            d_tok = _zeros(dim, dev)
+            d_tok = _zeros(dim, dev) if need[0] else None
             ops.embed_gather_bwd(ctx.plan, dim, lens, vocabs, None, pos, [m.reshape(-1) for m in mods], dx0, None, None,
                                  d_mods, d_tok)
-            grads = [d_tok.reshape(ctx.shapes[0])] + [g.reshape(s) for g, s in zip(d_mods, ctx.shapes[1:])]
+            grads = [d_tok] + d_mods
         else:
-            d_tabs = [torch.zeros(s, dtype=f32, device=dev) for s in ctx.shapes[:n]]
+            d_tabs = [torch.zeros(s, dtype=f32, device=dev) if nd else None for s, nd in zip(ctx.shapes[:n], need[:n])]
             ops.embed_gather_bwd(ctx.plan, dim, lens, vocabs, ids, pos, [m.reshape(-1) for m in mods], dx0,
                                  demb.contiguous() if demb is not None else None, d_tabs, d_mods, None)
-            grads = d_tabs + [g.reshape(s) for g, s in zip(d_mods, ctx.shapes[n:])]
-        return (None, None, None, *grads)
+            grads = d_tabs + d_mods
+        return (None, None, None, *[None if g is None else g.reshape(s) for g, s in zip(grads, ctx.shapes)])
 
 
 class _HeadLossFn(torch.autograd.Function):
     """decoder_norm -> per-modality vocabulary head -> cross-entropy (egom2p_model.py:523,614-680) with the head GEMM
-    fused into the softmax statistics: logits live in TMEM only. Returns the per-modality mean CE (0 for empty)."""
+    fused into the softmax statistics: logits live in TMEM only. Returns the per-modality mean CE (0 for empty). The
+    backward skips the dW GEMM of a frozen head, and the dY GEMMs, the scatter and the decoder_norm backward when neither
+    y nor decoder_norm wants a gradient."""
     CHUNK = 8192
 
     @staticmethod
     def forward(ctx, y, norm_w, norm_b, rows, targets, wbs, eps, epoch_ref, *head_w):
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
-        ctx.has_nb = norm_b is not None
         yn, _, mean, rstd = ops.layernorm_fwd(y, norm_w, eps, bias=norm_b)
         losses, lses, yms = [], [], []
         for idx, tgt, wb in zip(rows, targets, wbs):
@@ -524,31 +544,40 @@ class _HeadLossFn(torch.autograd.Function):
         y, norm_w, mean, rstd = ctx.saved_tensors
         dev = y.device
         D = y.shape[1]
-        dyn = torch.zeros_like(y)  # rows of pads / modalities without targets get zero gradient
+        need_y, need_nw, need_nb = ctx.needs_input_grad[:3]
+        need_heads = ctx.needs_input_grad[8:]
+        want_dyn = need_y or need_nw or need_nb   # the dY GEMMs, the scatter and the decoder_norm backward
+        dyn = torch.zeros_like(y) if want_dyn else None  # rows of pads / modalities without targets get zero gradient
         dws = []
-        for idx, tgt, wb, lse, ym, dl in zip(ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms, dlosses):
+        for idx, tgt, wb, lse, ym, dl, need_w in zip(ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms, dlosses, need_heads):
             V = wb.shape[0]
-            if idx.numel() == 0 or dl is None:
-                dws.append(torch.zeros(V, D, dtype=f32, device=dev))
+            if idx.numel() == 0 or dl is None or not (need_w or want_dyn):
+                dws.append(torch.zeros(V, D, dtype=f32, device=dev) if need_w else None)
                 continue
             R = idx.numel()
             gscale = (dl.reshape(1).to(f32) / R).contiguous()
-            dw = torch.empty(V, D, dtype=f32, device=dev)
-            dym = torch.empty(R, D, dtype=f32, device=dev)
+            dw = torch.empty(V, D, dtype=f32, device=dev) if need_w else None
+            dym = torch.empty(R, D, dtype=f32, device=dev) if want_dyn else None
             chunk = min(V, _HeadLossFn.CHUNK)
             buf = torch.empty(R, chunk, dtype=bf16, device=dev)
             for v0 in range(0, V, chunk):
                 vc = min(chunk, V - v0)
                 dlog = buf[:, :vc]
                 ops.ce_dlogits(ym, wb, tgt, lse, gscale, v0, vc, dlog)
-                ops.gemm(dlog, wb[v0:v0 + vc], R, D, vc, b_mn=True, addend=dym if v0 else None, out_f32=dym)
-                ops.gemm(dlog, ym, vc, D, R, a_mn=True, b_mn=True, out_f32=dw[v0:v0 + vc])
-            ops.scatter_rows_f32(dym, idx, dyn)
+                if want_dyn:
+                    ops.gemm(dlog, wb[v0:v0 + vc], R, D, vc, b_mn=True, addend=dym if v0 else None, out_f32=dym)
+                if need_w:   # a frozen (tied) head gets no dW GEMM
+                    ops.gemm(dlog, ym, vc, D, R, a_mn=True, b_mn=True, out_f32=dw[v0:v0 + vc])
+            if want_dyn:
+                ops.scatter_rows_f32(dym, idx, dyn)
             dws.append(dw)
-        dnw = _zeros(D, dev)
-        dnb = _zeros(D, dev) if ctx.has_nb else None
-        dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=True, d_bias=dnb)
-        return (_with_bf16(dy, dyb), dnw, dnb, None, None, None, None, None, *dws)
+        dy = dnw = dnb = None
+        if want_dyn:
+            dnw = _zeros(D, dev) if need_nw else None
+            dnb = _zeros(D, dev) if need_nb else None
+            dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=need_y, d_bias=dnb)
+            dy = _with_bf16(dy, dyb) if need_y else None
+        return (dy, dnw, dnb, None, None, None, None, None, *dws)
 
 
 # =============================================================================================== the module

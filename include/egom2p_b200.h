@@ -94,13 +94,14 @@ int egom2p_embed_gather_bwd(const egom2p_embed_desc* desc, const float* dx0, con
  * ------------------------------------------------------------------------------------------------ */
 int egom2p_layernorm_fwd(const float* x, const float* weight, int64_t rows, int32_t dim, float eps, uint16_t* y_bf16,
                          float* y_f32, float* mean, float* rstd, void* stream);
-/* dx_out = dx_in (may be NULL) + LN'(dy); dy given as bf16 or fp32 (exactly one non-NULL); d_weight += sum_r dy*xhat.
- * dx_bf16 (optional) receives a bf16 copy of dx_out. */
+/* dx_out = dx_in (may be NULL) + LN'(dy); dy given as bf16 or fp32 (exactly one non-NULL); d_weight += sum_r dy*xhat
+ * (NULL: not reduced, for a frozen weight). dx_bf16 (optional) receives a bf16 copy of dx_out. */
 int egom2p_layernorm_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
                          const float* mean, const float* rstd, const float* dx_in, int64_t rows, int32_t dim,
                          float* dx_out, uint16_t* dx_bf16, float* d_weight, void* stream);
 /* nn.LayerNorm(dim, eps) with a learnable bias (the GELU / bias family, egom2p_model.py:882-978): the forward adds bias[c]
- * after the weight; the backward is the one above plus d_bias += sum_r dy (non-NULL), in the same pass. */
+ * after the weight; the backward is the one above plus d_bias += sum_r dy in the same pass. d_weight and d_bias may each be
+ * NULL (a frozen parameter's gradient is not reduced). */
 int egom2p_layernorm_bias_fwd(const float* x, const float* weight, const float* bias, int64_t rows, int32_t dim, float eps,
                               uint16_t* y_bf16, float* y_f32, float* mean, float* rstd, void* stream);
 int egom2p_layernorm_bias_bwd(const uint16_t* dy_bf16, const float* dy_f32, const float* x, const float* weight,
