@@ -83,6 +83,25 @@ def _req(t: torch.Tensor, dtype, name: str):
     return t
 
 
+def _req_dense(t: torch.Tensor, dtype, name: str, numel: Optional[int] = None):
+    """_req plus the layout a kernel reads through a raw pointer: contiguous and, when given, `numel` elements."""
+    _req(t, dtype, name)
+    if not t.is_contiguous():
+        raise ValueError(f"egom2p_b200: {name} must be contiguous (got strides {t.stride()} for shape {tuple(t.shape)})")
+    if numel is not None and t.numel() != numel:
+        raise ValueError(f"egom2p_b200: {name} must have {numel} elements, got shape {tuple(t.shape)}")
+    return t
+
+
+def _req_rows(t: torch.Tensor, dtype, name: str, cols: int):
+    """A 2-D matrix of `cols` columns whose rows follow each other without a gap (row pitch == cols)."""
+    _req(t, dtype, name)
+    if t.dim() != 2 or t.shape[1] != cols or t.stride(1) != 1 or (t.shape[0] > 1 and t.stride(0) != cols):
+        raise ValueError(f"egom2p_b200: {name} must be (rows, {cols}) with row pitch {cols}, got shape {tuple(t.shape)} "
+                         f"and strides {t.stride()}")
+    return t
+
+
 # ----------------------------------------------------------------------------------------------- index plan
 class Plan:
     """Outputs of egom2p_index_plan for one side (encoder or decoder)."""
@@ -150,14 +169,17 @@ def plan_rows(mod_mask: torch.Tensor, mod_ids: Sequence[int]):
 
 
 # ----------------------------------------------------------------------------------------------- embedding
-def _embed_desc(dim, lens, vocabs, ids, tables, pos, mod):
+def _embed_desc(B, dim, lens, vocabs, ids, tables, pos, mod):
     d = _lib.EmbedDesc()
     d.n_mods, d.dim = len(lens), dim
     for i in range(len(lens)):
         d.len[i], d.vocab[i] = lens[i], vocabs[i]
-        d.ids[i] = _p(ids[i]) if ids is not None else None
-        d.token_emb[i] = _p(tables[i]) if tables is not None else None
-        d.pos_emb[i], d.mod_emb[i] = _p(pos[i]), _p(mod[i])
+        if ids is not None:
+            d.ids[i] = _req_dense(ids[i], torch.int64, "ids", B * lens[i]).data_ptr()
+        if tables is not None:
+            d.token_emb[i] = _req_dense(tables[i], f32, "token table", vocabs[i] * dim).data_ptr()
+        d.pos_emb[i] = _req_dense(pos[i], f32, "pos_emb", lens[i] * dim).data_ptr()
+        d.mod_emb[i] = _req_dense(mod[i], f32, "mod_emb", dim).data_ptr()
     return d
 
 
@@ -166,9 +188,11 @@ def embed_gather_fwd(plan: Plan, dim: int, lens, vocabs, ids, tables, pos, mod, 
     packed = plan.rows is not None
     rows = plan.rows if packed else plan.B * plan.budget
     dev = plan.keep_mod.device
+    d = _embed_desc(plan.B, dim, lens, vocabs, ids, tables, pos, mod)
+    if mask_token is not None:
+        _req_dense(mask_token, f32, "mask_token", dim)
     x0 = torch.empty((rows, dim) if packed else (plan.B, plan.budget, dim), dtype=f32, device=dev)
     emb = torch.empty_like(x0) if want_emb else None
-    d = _embed_desc(dim, lens, vocabs, ids, tables, pos, mod)
     with _timed("embed_gather", rows * dim * 4.0 * (2 + (1 if mask_token is None else 0) + (1 if want_emb else 0)), "byte"):
         _lib.check(lib.egom2p_embed_gather_fwd(C.byref(d), _p(mask_token), _p(plan.keep_mod), _p(plan.keep_pos), _p(plan.pad),
                                                _p(plan.row_batch), rows, plan.budget, _p(x0), _p(emb), _s()), "embed_gather_fwd")
@@ -178,8 +202,19 @@ def embed_gather_fwd(plan: Plan, dim: int, lens, vocabs, ids, tables, pos, mod, 
 def embed_gather_bwd(plan: Plan, dim: int, lens, vocabs, ids, pos, mod, dx0, demb, d_tables, d_mod, d_mask_token):
     lib = _lib.load()
     rows = plan.rows if plan.rows is not None else plan.B * plan.budget
-    d = _embed_desc(dim, lens, vocabs, ids, None, pos, mod)
+    d = _embed_desc(plan.B, dim, lens, vocabs, ids, None, pos, mod)
     n = len(lens)
+    _req_dense(dx0, f32, "dx0", rows * dim)
+    if demb is not None:
+        _req_dense(demb, f32, "demb", rows * dim)
+    for i, t in enumerate(d_tables or []):
+        if t is not None:
+            _req_dense(t, f32, "d_tables", vocabs[i] * dim)
+    for t in d_mod or []:
+        if t is not None:
+            _req_dense(t, f32, "d_mod", dim)
+    if d_mask_token is not None:
+        _req_dense(d_mask_token, f32, "d_mask_token", dim)
     arr_t = (C.c_void_p * _lib.MAX_MODS)(*[(_p(t) if t is not None else None) for t in (d_tables or [None] * n)])
     arr_m = (C.c_void_p * _lib.MAX_MODS)(*[(_p(t) if t is not None else None) for t in (d_mod or [None] * n)])
     _lib.check(lib.egom2p_embed_gather_bwd(C.byref(d), _p(dx0), _p(demb), _p(plan.keep_mod), _p(plan.keep_pos),
@@ -502,7 +537,10 @@ def colsum_bf16(x: torch.Tensor, out: Optional[torch.Tensor] = None):
 
 
 def gather_rows_bf16(src: torch.Tensor, idx: torch.Tensor):
+    """dst[i] = src[idx[i]]: src (rows, cols) bf16 with row pitch cols, idx int64 contiguous (every entry < rows)."""
     lib = _lib.load()
+    _req_rows(src, bf16, "src", src.shape[-1])
+    _req_dense(idx, torch.int64, "idx")
     n, cols = idx.numel(), src.shape[1]
     dst = torch.empty(n, cols, dtype=bf16, device=src.device)
     if n:
@@ -511,7 +549,12 @@ def gather_rows_bf16(src: torch.Tensor, idx: torch.Tensor):
 
 
 def scatter_rows_f32(src: torch.Tensor, idx: torch.Tensor, dst: torch.Tensor):
+    """dst[idx[i]] = src[i]: src (n, cols) and dst (rows, cols) fp32 with row pitch cols, idx int64 contiguous (every entry
+    < rows); rows of dst that idx does not name are left as they are."""
     lib = _lib.load()
+    _req_rows(src, f32, "src", src.shape[-1])
+    _req_rows(dst, f32, "dst", src.shape[1])
+    _req_dense(idx, torch.int64, "idx", src.shape[0])
     n, cols = idx.numel(), src.shape[1]
     if n:
         _lib.check(lib.egom2p_scatter_rows_f32(_p(src), _p(idx), n, cols, _p(dst), _s()), "scatter_rows_f32")

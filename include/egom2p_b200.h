@@ -77,6 +77,7 @@ typedef struct {
 
 /* x0[r] = tok[r] + (pos_emb[p] + mod_emb)  and  emb[r] = pos_emb[p] + mod_emb  for kept slot r; pads -> 0.
  * tok[r] = token_emb[ids] (encoder) or mask_token (decoder, mask_token != NULL). emb may be NULL.
+ * A token id outside [0, vocab) is clamped to 0 or vocab - 1 here and in the backward (the reference raises on it).
  * row_batch: sample index of every row (int32, rows), or NULL when the rows are the (B, budget) slots in order (sample =
  * r / budget). A non-NULL row_batch is what lets the rows of a ragged batch be PACKED (valid slots only, sample after
  * sample), so that every per-row kernel downstream works on the valid tokens only. */
