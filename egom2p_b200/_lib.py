@@ -46,8 +46,11 @@ SIGNATURES = {
     "egom2p_gemm_gelu_fwd": [vp, vp, vp, i32, i32, i32, i64, i64, vp, i64, vp, i64, vp],
     "egom2p_gemm_gelu_bwd": [vp, vp, vp, i32, i32, i32, i64, i64, i64, vp, i64, vp],
     "egom2p_ce_partials": [vp, vp, vp, i32, i32, i32, i64, i64, vp, vp, vp, vp],
-    "egom2p_ce_finalize": [vp, vp, vp, i32, i32, vp, vp, vp],
-    "egom2p_ce_dlogits": [vp, vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, vp, i64, vp],
+    "egom2p_ce_probs": [vp, vp, vp, vp, i32, i32, i32, i64, i64, vp, i64, vp, vp, vp, vp],
+    "egom2p_ce_row_ref": [vp, vp, i32, i32, i32, i64, i64, vp, vp, vp],
+    "egom2p_ce_finalize": [vp, vp, vp, i32, i32, vp, vp, vp, vp, i32, vp, i64, vp, vp, vp],
+    "egom2p_ce_dlogits": [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i64, i64, vp, i64, vp],
+    "egom2p_ce_row_scale": [vp, i32, i32, i64, vp, vp, vp, vp, vp],
     "egom2p_attn_lse_stride": [i32],
     "egom2p_attn_ranges_bytes": [i32, i32],
     "egom2p_attn_ranges": [vp, vp, i32, i32, i32, f32, i32, vp, vp],
@@ -66,7 +69,7 @@ SIGNATURES = {
     "egom2p_colsum_f32": [vp, i64, i32, vp, vp],
     "egom2p_colsum_bf16": [vp, i64, i32, i64, vp, vp],
     "egom2p_gather_rows_bf16": [vp, vp, i64, i32, vp, vp],
-    "egom2p_scatter_rows_f32": [vp, vp, i64, i32, vp, vp],
+    "egom2p_scatter_rows_f32": [vp, vp, i64, i32, vp, vp, vp],
 }
 _RESTYPES = {"egom2p_last_error": C.c_char_p, "egom2p_launch_count": i64, "egom2p_attn_bwd_scratch_bytes": i64, "egom2p_attn_ranges_bytes": i64}
 

@@ -297,13 +297,21 @@ __global__ void __launch_bounds__(kEwThreads) gather_rows_bf16_kernel(const uint
     reinterpret_cast<uint4*>(dst)[i] = reinterpret_cast<const uint4*>(src)[idx[r] * cols8 + c];
   }
 }
+// row_scale (optional): dst[idx[i], :] = row_scale[i] * src[i, :] -- the head backward's per-row softmax normaliser, applied
+// where dY is read anyway.
 __global__ void __launch_bounds__(kEwThreads) scatter_rows_f32_kernel(const float* __restrict__ src, const int64_t* __restrict__ idx,
-                                                                      int64_t n, int cols4, float* __restrict__ dst) {
+                                                                      int64_t n, int cols4, const float* __restrict__ row_scale,
+                                                                      float* __restrict__ dst) {
   const int64_t total = n * cols4;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t r = i / cols4;
     const int c = (int)(i - r * cols4);
-    reinterpret_cast<float4*>(dst)[idx[r] * cols4 + c] = reinterpret_cast<const float4*>(src)[i];
+    float4 v = reinterpret_cast<const float4*>(src)[i];
+    if (row_scale) {
+      const float s = row_scale[r];
+      v.x *= s; v.y *= s; v.z *= s; v.w *= s;
+    }
+    reinterpret_cast<float4*>(dst)[idx[r] * cols4 + c] = v;
   }
 }
 
@@ -336,10 +344,11 @@ extern "C" int egom2p_gather_rows_bf16(const uint16_t* src, const int64_t* idx, 
   gather_rows_bf16_kernel<<<ew_grid(n * (cols / 8)), kEwThreads, 0, (cudaStream_t)stream>>>(src, idx, n, cols / 8, dst);
   return check_launch("gather_rows_bf16");
 }
-extern "C" int egom2p_scatter_rows_f32(const float* src, const int64_t* idx, int64_t n, int32_t cols, float* dst, void* stream) {
+extern "C" int egom2p_scatter_rows_f32(const float* src, const int64_t* idx, int64_t n, int32_t cols, const float* row_scale,
+                                       float* dst, void* stream) {
   using namespace egom2p;
   EGO_REQUIRE(src && idx && dst && n > 0 && cols > 0 && cols % 4 == 0, "scatter_rows_f32: bad argument (cols %% 4 == 0)");
-  scatter_rows_f32_kernel<<<ew_grid(n * (cols / 4)), kEwThreads, 0, (cudaStream_t)stream>>>(src, idx, n, cols / 4, dst);
+  scatter_rows_f32_kernel<<<ew_grid(n * (cols / 4)), kEwThreads, 0, (cudaStream_t)stream>>>(src, idx, n, cols / 4, row_scale, dst);
   return check_launch("scatter_rows_f32");
 }
 

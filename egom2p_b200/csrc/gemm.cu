@@ -24,8 +24,12 @@ constexpr int kGemmThreads = 64 + 32 * kEpiWarps;
 
 // EPI_STORE_BIAS_BF16: EPI_STORE with bf16 output and a bias -- its own instantiation, so that the bias code does not cost
 // the plain stores registers.
+// EPI_CE_PROBS: the loss pass of a head that needs a backward -- EPI_CE_PARTIAL's statistics plus the softmax numerators
+// P = 2^(logit * log2 e - ref[r]) stored as bf16.
 enum { EPI_STORE = 0, EPI_CE_PARTIAL = 1, EPI_CE_DLOGITS = 2, EPI_SWIGLU_FWD = 3, EPI_SWIGLU_BWD = 4, EPI_GELU_FWD = 5,
-       EPI_GELU_BWD = 6, EPI_STORE_BIAS_BF16 = 7 };
+       EPI_GELU_BWD = 6, EPI_STORE_BIAS_BF16 = 7, EPI_CE_PROBS = 8 };
+
+constexpr float kLog2e = 1.4426950408889634f;
 
 struct GemmParams {
   int M, N, K;
@@ -37,8 +41,9 @@ struct GemmParams {
   int out_bf16, out_f32;
   // CE epilogues
   const int64_t* target;
-  const float* lse;
-  const float* gscale;
+  const float* lse;        // per-row offset of the exponent: the lse (EPI_CE_DLOGITS) or the numerators' reference
+                           // in log2 units (EPI_CE_PROBS)
+  const float* gscale;     // EPI_CE_DLOGITS: null = 1
   // SwiGLU epilogues: ab = [a | b] interleaved in groups of 32 columns (bf16), row pitch ld_ab.
   // GELU backward: ab = the saved pre-activation u (bf16), row pitch ld_ab; GELU forward: ld_ab = row pitch of GELU(u).
   const uint16_t* ab;
@@ -47,6 +52,10 @@ struct GemmParams {
   float* part_max;
   float* part_sum;
   float* tgt_logit;
+  // (one more field here costs the SwiGLU backward instantiation, at the 168-register cap, 130 B of extra spills)
+  // EPI_CE_DLOGITS: non-null = only the 128-row tiles whose flag is set are computed (the loss pass's fall-back); the
+  // items are then walked statically by a grid of one round of pairs instead of by cluster launch control
+  const uint8_t* tile_flag;
 };
 
 // The kernel runs as CTA pairs (cluster 2x1x1) issuing tcgen05.mma.cta_group::2 -- a 256 x BN tile per pair, each CTA
@@ -79,6 +88,11 @@ __device__ __forceinline__ float sigmoid_fast(float x) {
 __device__ __forceinline__ float gelu_erf(float u) { return 0.5f * u * (1.f + erff(u * 0.70710678118654752f)); }
 __device__ __forceinline__ float gelu_erf_grad(float u) {
   return 0.5f * (1.f + erff(u * 0.70710678118654752f)) + u * 0.39894228040143268f * __expf(-0.5f * u * u);
+}
+__device__ __forceinline__ float ce_ex2(float x) {  // one MUFU.EX2; 0 for x below -126 (flushed), as the softmax wants
+  float y;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
+  return y;
 }
 __device__ __forceinline__ uint32_t box_off(int row, int chunk) {  // 16-byte chunk inside a [32][128 B] SW128 box
   return (uint32_t)row * 128u + (uint32_t)((chunk ^ (row & 7)) << 4);
@@ -121,9 +135,41 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
   constexpr int cl = 2;
   const uint32_t crank = cluster_ctarank();
   const bool leader = crank == 0;
+  // Gated fall-back (EPI_CE_DLOGITS with tile flags): the items of the 256-row tile pairs that hold a flagged 128-row tile,
+  // in order, every (gridDim.x / 2)-th one starting at this pair's index. Every role walks the same sequence. A pair with
+  // nothing to do (every pair when no flag is set) reads the flags once and exits before its barrier / TMEM set-up.
+  constexpr bool kGate = EPI == EPI_CE_DLOGITS;
+  const bool gated = kGate && p.tile_flag != nullptr;
+  const int n_pairs_m = (m_tiles + 1) / 2;
+  int g_mp = 0, g_n = 0;
+  auto flagged = [&](int mp) {
+    return p.tile_flag[2 * mp] != 0 || (2 * mp + 1 < m_tiles && p.tile_flag[2 * mp + 1] != 0);
+  };
+  auto gate_step = [&](int step) {
+    g_n += step;
+    while (g_mp < n_pairs_m && g_n >= n_tiles) {
+      g_n -= n_tiles;
+      do ++g_mp; while (g_mp < n_pairs_m && !flagged(g_mp));
+    }
+  };
+  bool have_item = true;
+  int first_item = blockIdx.x / cl;
+  if (kGate && gated) {
+    g_mp = 0;
+    while (g_mp < n_pairs_m && !flagged(g_mp)) ++g_mp;
+    gate_step(blockIdx.x / cl);
+    have_item = g_mp < n_pairs_m;
+    first_item = g_mp * n_tiles + g_n;
+    if (!have_item) return;   // both CTAs of the pair see the same flags: they leave together, before any set-up
+  }
   // One request per processed item, issued by the leader's producer warp when it starts the item; every role of both CTAs
   // reads the response after its own work on the item. Returns false when nothing was left to take over.
   auto next_item = [&](int it, int& item, bool is_scheduler) -> bool {
+    if (kGate && gated) {
+      gate_step(gridDim.x / cl);
+      item = g_mp * n_tiles + g_n;
+      return g_mp < n_pairs_m;
+    }
     const int slot = it % kSched;
     mbar_wait(&clc_full[slot], (it / kSched) & 1);
     int x;
@@ -169,9 +215,9 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     // The whole warp walks the loop (addresses / coordinates stay in uniform registers); one elected lane issues.
     int stage = 0;
     uint32_t phase = 0;
-    int item = blockIdx.x / cl;
-    for (int it = 0;; ++it) {
-      if (leader) {  // ask for the item after this one now: the answer is there long before this item's k loop ends
+    int item = first_item;
+    for (int it = 0; have_item; ++it) {
+      if (leader && !gated) {  // ask for the item after this one now: the answer is there long before this item's k loop ends
         const int slot = it % kSched;
         if (elect_one()) {
           mbar_wait(&clc_empty[slot], ((it / kSched) & 1) ^ 1);
@@ -219,8 +265,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     constexpr uint64_t kStepA = A_MN ? (2048 >> 4) : (32 >> 4), kStepB = B_MN ? (2048 >> 4) : (32 >> 4);
     int stage = 0;
     uint32_t phase = 0;
-    int item = blockIdx.x / cl;
-    for (int it = 0; leader; ++it) {  // pair: only the leader CTA issues
+    int item = first_item;
+    for (int it = 0; leader && have_item; ++it) {  // pair: only the leader CTA issues
       const int split = item % splits;
       const int kb0 = split * kb_per, kb1 = min(k_blocks, kb0 + kb_per);
       const int acc = it & 1;
@@ -253,8 +299,8 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
     const int half = (warp - 2) >> 2;    // which half of the tile's columns
     uint8_t* box = staging + (warp - 2) * 4096;
     constexpr int kHalfCols = BN / 2;
-    int item = blockIdx.x / cl;
-    for (int it = 0;; ++it) {
+    int item = first_item;
+    for (int it = 0; have_item; ++it) {
       const int tile = item / splits;
       const int acc = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1;
@@ -266,17 +312,20 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
       mbar_wait(&tfull_bar[acc], acc_phase);
       tc_fence_after();
       const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN + half * kHalfCols;
-      float row_lse = 0.f, gs = 0.f;
+      float row_lse = 0.f, gs = 0.f, row_ref = 0.f;
       int row_tgt = -1;
       float run_max = -INFINITY, run_sum = 0.f, tl = 0.f;
       bool has_tl = false;
-      if ((EPI == EPI_CE_PARTIAL || EPI == EPI_CE_DLOGITS) && row_ok) {
+      if ((EPI == EPI_CE_PARTIAL || EPI == EPI_CE_DLOGITS || EPI == EPI_CE_PROBS) && row_ok) {
         row_tgt = (int)p.target[my_row] - p.v0;
         if (EPI == EPI_CE_DLOGITS) {
           row_lse = p.lse[my_row];
-          gs = *p.gscale;
+          gs = p.gscale ? *p.gscale : 1.f;
         }
+        if (EPI == EPI_CE_PROBS) row_ref = p.lse[my_row];
       }
+      // gated fall-back: a CTA whose own 128-row tile is not flagged computes along with its peer but stores nothing
+      const bool store_tile = !kGate || !gated || (m0 < p.M && p.tile_flag[m0 / BM] != 0);
       if (EPI == EPI_CE_PARTIAL) {
 #pragma unroll 1
         for (int c = 0; c < kHalfCols / 32; ++c) {
@@ -543,8 +592,30 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
             tma_store_commit();
           }
         }
-      } else if (EPI == EPI_CE_DLOGITS || EPI == EPI_STORE_BIAS_BF16 || p.out_bf16) {
+      } else if (EPI == EPI_CE_DLOGITS || EPI == EPI_CE_PROBS || EPI == EPI_STORE_BIAS_BF16 || p.out_bf16) {
         // ---- bf16 output: 64 columns (one 128-byte box row) per step
+        // EPI_CE_PROBS: a first sweep over the half's columns takes their maximum m; the stored numerator of a logit l is
+        // then 2^(l log2e - m log2e) * 2^(m log2e - ref): one exponential per element, the factor in [0, 1] relative to m
+        // summed into the same per-(tile, row) statistics as EPI_CE_PARTIAL, so the lse is exact whatever ref is.
+        float neg_ml = 0.f, pscale = 0.f;
+        if constexpr (EPI == EPI_CE_PROBS) {
+#pragma unroll 1
+          for (int c = 0; c < kHalfCols / 32; ++c) {
+            uint32_t v[32];
+            tmem_ld32(t_addr + c * 32, v);
+            tmem_ld_wait();
+            const int cbase = n0 + c * 32;
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              const float f = (cbase + j < p.N) ? __uint_as_float(v[j]) : -INFINITY;
+              run_max = fmaxf(run_max, f);
+              if (cbase + j == row_tgt) { tl = f; has_tl = true; }
+            }
+          }
+          const float ml = run_max > -INFINITY ? run_max * kLog2e : 0.f;
+          neg_ml = -ml;
+          pscale = ce_ex2(ml - row_ref);
+        }
 #pragma unroll 1
         for (int c = 0; c < kHalfCols / 64; ++c) {
           uint32_t v0[32], v1[32];
@@ -560,6 +631,16 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
               if (cbase + 32 + j == row_tgt) p1 -= 1.f;
               v0[j] = __float_as_uint(p0 * gs);
               v1[j] = __float_as_uint(p1 * gs);
+            }
+          }
+          if constexpr (EPI == EPI_CE_PROBS) {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              const float e0 = (cbase + j < p.N) ? ce_ex2(fmaf(__uint_as_float(v0[j]), kLog2e, neg_ml)) : 0.f;
+              const float e1 = (cbase + 32 + j < p.N) ? ce_ex2(fmaf(__uint_as_float(v1[j]), kLog2e, neg_ml)) : 0.f;
+              run_sum += e0 + e1;
+              v0[j] = __float_as_uint(e0 * pscale);
+              v1[j] = __float_as_uint(e1 * pscale);
             }
           }
           if constexpr (EPI == EPI_STORE_BIAS_BF16) {   // N % 8 == 0: a float4 of the bias is either wholly inside or wholly outside
@@ -596,9 +677,15 @@ gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
           fence_async_smem();
           __syncwarp();
           if (lane == 0) {
-            if (row0 < p.M && cbase < p.N) tma_store_2d(&tmCb, bx, cbase, row0);
+            if (row0 < p.M && cbase < p.N && store_tile) tma_store_2d(&tmCb, bx, cbase, row0);
             tma_store_commit();
           }
+        }
+        if (EPI == EPI_CE_PROBS && row_ok) {
+          const int64_t o = (int64_t)(n_blk * 2 + half) * p.M + my_row;
+          p.part_max[o] = run_max;
+          p.part_sum[o] = run_sum;
+          if (has_tl) p.tgt_logit[my_row] = tl;
         }
       } else {
         // ---- fp32 output (+bias, +residual / accumulate): 32 columns (one 128-byte box row) per step. The residual row
@@ -752,6 +839,7 @@ static int launch_gemm(const uint16_t* A, const uint16_t* B, int64_t lda, int64_
   attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.blockDim = dim3(kGemmThreads); cfg.dynamicSmemBytes = S::kTotal; cfg.stream = stream; cfg.attrs = attr; cfg.numAttrs = 1;
   cfg.gridDim = dim3(2 * pair_items);   // one pair per work item; the pairs that get to run cancel and absorb the rest
+  if (EPI == EPI_CE_DLOGITS && p.tile_flag) cfg.gridDim = dim3(2 * (pair_items < workers ? pair_items : workers));   // static walk
   cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmCb, tmCf, p);
   if (e != cudaSuccess) { set_error("gemm: cluster launch: %s", cudaGetErrorString(e)); return EGOM2P_ERR_CUDA; }
   return check_launch("gemm_bf16");
@@ -816,14 +904,27 @@ extern "C" int egom2p_ce_partials(const uint16_t* Y, const uint16_t* W, const in
   return dispatch_gemm<EPI_CE_PARTIAL>(Y, W, ldy, ldw, 0, 0, nullptr, nullptr, 0, p, (cudaStream_t)stream);
 }
 
-extern "C" int egom2p_ce_dlogits(const uint16_t* Y, const uint16_t* W, const int64_t* target, const float* lse,
-                                 const float* gscale, int32_t R, int32_t v0, int32_t Vc, int32_t K, int64_t ldy, int64_t ldw,
-                                 uint16_t* dlogits, int64_t ldd, void* stream) {
+extern "C" int egom2p_ce_probs(const uint16_t* Y, const uint16_t* W, const int64_t* target, const float* ref, int32_t R,
+                               int32_t V, int32_t K, int64_t ldy, int64_t ldw, uint16_t* probs, int64_t ldp, float* part_max,
+                               float* part_sum, float* tgt_logit, void* stream) {
   using namespace egom2p;
-  EGO_REQUIRE(Y && W && target && lse && gscale && dlogits && R > 0 && Vc > 0 && K > 0 && v0 >= 0, "ce_dlogits: bad argument");
+  EGO_REQUIRE(Y && W && target && ref && probs && part_max && part_sum && tgt_logit && R > 0 && V > 0 && K > 0,
+              "ce_probs: bad argument");
+  EGO_REQUIRE(V % 8 == 0 && ldp % 8 == 0 && ldp >= V, "ce_probs: V and ldp must be multiples of 8, ldp >= V");
+  GemmParams p{};
+  p.M = R; p.N = V; p.K = K; p.target = target; p.lse = ref; p.v0 = 0;
+  p.part_max = part_max; p.part_sum = part_sum; p.tgt_logit = tgt_logit;
+  return dispatch_gemm<EPI_CE_PROBS>(Y, W, ldy, ldw, 0, 0, probs, nullptr, ldp, p, (cudaStream_t)stream);
+}
+
+extern "C" int egom2p_ce_dlogits(const uint16_t* Y, const uint16_t* W, const int64_t* target, const float* lse,
+                                 const float* gscale, const uint8_t* tile_flag, int32_t R, int32_t v0, int32_t Vc, int32_t K,
+                                 int64_t ldy, int64_t ldw, uint16_t* dlogits, int64_t ldd, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(Y && W && target && lse && dlogits && R > 0 && Vc > 0 && K > 0 && v0 >= 0, "ce_dlogits: bad argument");
   EGO_REQUIRE(Vc % 8 == 0 && ldd % 8 == 0, "ce_dlogits: Vc and ldd must be multiples of 8");
   GemmParams p{};
-  p.M = R; p.N = Vc; p.K = K; p.target = target; p.lse = lse; p.gscale = gscale; p.v0 = v0;
+  p.M = R; p.N = Vc; p.K = K; p.target = target; p.lse = lse; p.gscale = gscale; p.v0 = v0; p.tile_flag = tile_flag;
   return dispatch_gemm<EPI_CE_DLOGITS>(Y, W + (int64_t)v0 * ldw, ldy, ldw, 0, 0, dlogits, nullptr, ldd, p, (cudaStream_t)stream);
 }
 
@@ -870,14 +971,20 @@ extern "C" int egom2p_gemm_gelu_bwd(const uint16_t* dY, const uint16_t* W2, cons
 }
 
 namespace egom2p {
-__global__ void ce_finalize_kernel(const float* __restrict__ pm, const float* __restrict__ ps, const float* __restrict__ tl,
-                                   int R, int n_parts, float* __restrict__ lse, float* __restrict__ loss_sum) {
-  const int r = blockIdx.x * blockDim.x + threadIdx.x;
-  float contrib = 0.f;
+constexpr int kFinRows = 128;   // one block per 128-row tile: the tile's fall-back flag is one block-wide vote
+// lse[r] = logsumexp over the (tile, row) partials; loss_sum += sum_r (lse[r] - tgt_logit[r]). With ref (the loss pass
+// that stored the numerators P[r, v] = 2^(l log2e - ref[r])): Z[r] = sum_v P[r, v]; a row is exact when
+// ref[r] - max_v l log2e <= 60 (its largest numerator >= 2^-60, so every entry within 2^-66 of it is a normal bf16). A
+// 128-row tile holding a row that is not is flagged for the backward's recompute (rscale = 1); on the others rscale =
+// 1 / Z and the target entry becomes P - Z, so that rscale * P[r, :] = softmax - onehot.
+__global__ void __launch_bounds__(kFinRows) ce_finalize_kernel(const float* __restrict__ pm, const float* __restrict__ ps,
+    const float* __restrict__ tl, int R, int n_parts, float* __restrict__ lse, float* __restrict__ loss_sum,
+    const float* __restrict__ ref, const int64_t* __restrict__ target, int V, uint16_t* __restrict__ probs, int64_t ldp,
+    float* __restrict__ rscale, uint8_t* __restrict__ tile_flag) {
+  const int r = blockIdx.x * kFinRows + threadIdx.x;
+  float contrib = 0.f, m = -INFINITY, s = 0.f;
   if (r < R) {
-    float m = -INFINITY;
     for (int t = 0; t < n_parts; ++t) m = fmaxf(m, pm[(int64_t)t * R + r]);
-    float s = 0.f;
     for (int t = 0; t < n_parts; ++t) {
       const float pmv = pm[(int64_t)t * R + r];
       if (pmv > -INFINITY) s += ps[(int64_t)t * R + r] * __expf(pmv - m);
@@ -886,22 +993,114 @@ __global__ void ce_finalize_kernel(const float* __restrict__ pm, const float* __
     lse[r] = l;
     contrib = l - tl[r];
   }
+  if (ref) {
+    const float c = r < R ? ref[r] : 0.f;
+    const bool bad = r < R && !(c - m * kLog2e <= 60.f);
+    const bool flag = __syncthreads_or(bad);
+    if (threadIdx.x == 0) tile_flag[blockIdx.x] = flag;
+    if (r < R) {
+      const float z = s * ce_ex2(m * kLog2e - c);
+      rscale[r] = flag ? 1.f : 1.f / z;
+      const int64_t t = target[r];
+      if (!flag && t >= 0 && t < V) {
+        const __nv_bfloat16 d = __float2bfloat16_rn(ce_ex2(tl[r] * kLog2e - c) - z);
+        probs[(int64_t)r * ldp + t] = *reinterpret_cast<const uint16_t*>(&d);
+      }
+    }
+  }
   contrib = warp_sum(contrib);
-  __shared__ float sh[8];
+  __shared__ float sh[kFinRows / 32];
   if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = contrib;
   __syncthreads();
   if (threadIdx.x < 32) {
-    float t = threadIdx.x < 8 ? sh[threadIdx.x] : 0.f;
+    float t = threadIdx.x < kFinRows / 32 ? sh[threadIdx.x] : 0.f;
     t = warp_sum(t);
     if (threadIdx.x == 0 && loss_sum) atomicAdd(loss_sum, t);
   }
 }
+
+// ref[r] = ||y_r|| * max_v ||w_v|| * log2 e >= every logit of row r in log2 units (Cauchy-Schwarz over the bf16 operands).
+// Warp per row, 16-byte loads; the table's largest squared norm is an atomicMax on the (non-negative) float bits.
+__device__ __forceinline__ float row_sumsq_bf16(const uint16_t* row, int K, int lane) {
+  float a = 0.f;
+  for (int k = lane * 8; k < K; k += 256) {
+    const uint4 u = __ldg(reinterpret_cast<const uint4*>(row + k));
+    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[i]));
+      a = fmaf(f.x, f.x, fmaf(f.y, f.y, a));
+    }
+  }
+  return warp_sum(a);
+}
+__global__ void ce_wmax_kernel(const uint16_t* __restrict__ W, int V, int K, int64_t ldw, unsigned* __restrict__ wmax2) {
+  const int lane = threadIdx.x & 31, warps = gridDim.x * (blockDim.x >> 5);
+  float mx = 0.f;
+  for (int v = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); v < V; v += warps)
+    mx = fmaxf(mx, row_sumsq_bf16(W + (int64_t)v * ldw, K, lane));
+  if (lane == 0) atomicMax(wmax2, __float_as_uint(mx));
+}
+__global__ void ce_ref_kernel(const uint16_t* __restrict__ Y, int R, int K, int64_t ldy, const unsigned* __restrict__ wmax2,
+                              float* __restrict__ ref) {
+  const int lane = threadIdx.x & 31, r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (r >= R) return;
+  const float y2 = row_sumsq_bf16(Y + (int64_t)r * ldy, K, lane);
+  if (lane == 0) ref[r] = sqrtf(y2) * sqrtf(__uint_as_float(*wmax2)) * kLog2e;
+}
+
+// The backward's row scales: s[r] = gscale * rscale[r], and ys = bf16(s[r] * y[r, :]) (the dW GEMM's operand).
+__global__ void ce_row_scale_kernel(const uint16_t* __restrict__ Y, int R, int K, int64_t ldy, const float* __restrict__ rscale,
+                                    const float* __restrict__ gscale, float* __restrict__ s, uint16_t* __restrict__ ys) {
+  const int chunks = K / 8;
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)R * chunks) return;
+  const int r = (int)(i / chunks), k = (int)(i - (int64_t)r * chunks) * 8;
+  const float sr = *gscale * rscale[r];
+  if (k == 0) s[r] = sr;
+  if (!ys) return;
+  const uint4 u = __ldg(reinterpret_cast<const uint4*>(Y + (int64_t)r * ldy + k));
+  uint32_t w[4] = {u.x, u.y, u.z, u.w};
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w[j]));
+    w[j] = pack_bf16(f.x * sr, f.y * sr);
+  }
+  *reinterpret_cast<uint4*>(ys + (int64_t)r * K + k) = make_uint4(w[0], w[1], w[2], w[3]);
+}
 }  // namespace egom2p
 
 extern "C" int egom2p_ce_finalize(const float* part_max, const float* part_sum, const float* tgt_logit, int32_t R,
-                                  int32_t n_tiles, float* lse, float* loss_sum, void* stream) {
+                                  int32_t n_tiles, float* lse, float* loss_sum, const float* ref, const int64_t* target,
+                                  int32_t V, uint16_t* probs, int64_t ldp, float* rscale, uint8_t* tile_flag, void* stream) {
   using namespace egom2p;
   EGO_REQUIRE(part_max && part_sum && tgt_logit && lse && R > 0 && n_tiles > 0, "ce_finalize: bad argument");
-  ce_finalize_kernel<<<(R + 255) / 256, 256, 0, (cudaStream_t)stream>>>(part_max, part_sum, tgt_logit, R, n_tiles, lse, loss_sum);
+  EGO_REQUIRE(!ref || (target && probs && rscale && tile_flag && V > 0 && ldp >= V), "ce_finalize: bad loss-pass argument");
+  ce_finalize_kernel<<<(R + kFinRows - 1) / kFinRows, kFinRows, 0, (cudaStream_t)stream>>>(
+      part_max, part_sum, tgt_logit, R, n_tiles, lse, loss_sum, ref, target, V, probs, ldp, rscale, tile_flag);
   return check_launch("ce_finalize");
+}
+
+extern "C" int egom2p_ce_row_ref(const uint16_t* Y, const uint16_t* W, int32_t R, int32_t V, int32_t K, int64_t ldy,
+                                 int64_t ldw, float* wmax2, float* ref, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(Y && W && wmax2 && ref && R > 0 && V > 0 && K > 0, "ce_row_ref: bad argument");
+  EGO_REQUIRE(K % 8 == 0 && ldy % 8 == 0 && ldw % 8 == 0, "ce_row_ref: K, ldy and ldw must be multiples of 8");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaError_t e = cudaMemsetAsync(wmax2, 0, sizeof(float), st);
+  if (e != cudaSuccess) { set_error("ce_row_ref: memset: %s", cudaGetErrorString(e)); return EGOM2P_ERR_CUDA; }
+  const int wblocks = (V + 7) / 8 < 8 * device_sm_count() ? (V + 7) / 8 : 8 * device_sm_count();
+  ce_wmax_kernel<<<wblocks, 256, 0, st>>>(W, V, K, ldw, reinterpret_cast<unsigned*>(wmax2));
+  if (int rc = check_launch("ce_wmax")) return rc;
+  ce_ref_kernel<<<(R + 7) / 8, 256, 0, st>>>(Y, R, K, ldy, reinterpret_cast<const unsigned*>(wmax2), ref);
+  return check_launch("ce_ref");
+}
+
+extern "C" int egom2p_ce_row_scale(const uint16_t* Y, int32_t R, int32_t K, int64_t ldy, const float* rscale, const float* gscale,
+                                   float* s, uint16_t* ys, void* stream) {
+  using namespace egom2p;
+  EGO_REQUIRE(Y && rscale && gscale && s && R > 0 && K > 0 && K % 8 == 0 && ldy % 8 == 0, "ce_row_scale: bad argument");
+  const int64_t n = (int64_t)R * (K / 8);
+  ce_row_scale_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(Y, R, K, ldy, rscale, gscale, s, ys);
+  return check_launch("ce_row_scale");
 }

@@ -514,26 +514,29 @@ class _EmbedFn(torch.autograd.Function):
 
 class _HeadLossFn(torch.autograd.Function):
     """decoder_norm -> per-modality vocabulary head -> cross-entropy (egom2p_model.py:523,614-680) with the head GEMM
-    fused into the softmax statistics: logits live in TMEM only. Returns the per-modality mean CE (0 for empty). The
-    backward skips the dW GEMM of a frozen head, and the dY GEMMs, the scatter and the decoder_norm backward when neither
-    y nor decoder_norm wants a gradient."""
-    CHUNK = 8192
+    fused into the softmax statistics: logits live in TMEM only. Returns the per-modality mean CE (0 for empty).
+
+    grad_on (torch.is_grad_enabled() at the call): a head whose backward will run keeps its softmax numerators P (bf16,
+    R x V) from the loss pass, so the backward is one dY GEMM and one dW GEMM over P -- no second logits GEMM; P is freed
+    there. The backward skips the dW GEMM of a frozen head, and the dY GEMM, the scatter and the decoder_norm backward
+    when neither y nor decoder_norm wants a gradient."""
 
     @staticmethod
-    def forward(ctx, y, norm_w, norm_b, rows, targets, wbs, eps, epoch_ref, *head_w):
+    def forward(ctx, y, norm_w, norm_b, rows, targets, wbs, eps, epoch_ref, grad_on, *head_w):
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
         yn, _, mean, rstd = ops.layernorm_fwd(y, norm_w, eps, bias=norm_b)
-        losses, lses, yms = [], [], []
-        for idx, tgt, wb in zip(rows, targets, wbs):
+        want_dyn = any(ctx.needs_input_grad[:3])
+        losses, lses, yms, probs = [], [], [], []
+        for idx, tgt, wb, need_w in zip(rows, targets, wbs, ctx.needs_input_grad[9:]):
             if idx.numel() == 0:
                 losses.append(torch.zeros((), dtype=f32, device=y.device))
-                lses.append(None); yms.append(None)
+                lses.append(None); yms.append(None); probs.append(None)
                 continue
             ym = ops.gather_rows_bf16(yn, idx)
-            loss_sum, lse = ops.ce_forward(ym, wb, tgt)
-            losses.append(loss_sum[0] / idx.numel())
-            lses.append(lse); yms.append(ym)
-        ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms = rows, targets, wbs, lses, yms
+            out = ops.ce_forward(ym, wb, tgt, keep_probs=grad_on and (want_dyn or need_w))
+            losses.append(out[0][0] / idx.numel())
+            lses.append(out[1]); yms.append(ym); probs.append(out[2] if len(out) > 2 else None)
+        ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms, ctx.probs = rows, targets, wbs, lses, yms, probs
         ctx.save_for_backward(y, norm_w, mean, rstd)
         return tuple(losses)
 
@@ -545,31 +548,37 @@ class _HeadLossFn(torch.autograd.Function):
         dev = y.device
         D = y.shape[1]
         need_y, need_nw, need_nb = ctx.needs_input_grad[:3]
-        need_heads = ctx.needs_input_grad[8:]
-        want_dyn = need_y or need_nw or need_nb   # the dY GEMMs, the scatter and the decoder_norm backward
+        need_heads = ctx.needs_input_grad[9:]
+        want_dyn = need_y or need_nw or need_nb   # the dY GEMM, the scatter and the decoder_norm backward
         dyn = torch.zeros_like(y) if want_dyn else None  # rows of pads / modalities without targets get zero gradient
         dws = []
-        for idx, tgt, wb, lse, ym, dl, need_w in zip(ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms, dlosses, need_heads):
+        for i, (idx, tgt, wb, lse, ym, dl, need_w) in enumerate(zip(ctx.rows, ctx.targets, ctx.wbs, ctx.lses, ctx.yms, dlosses,
+                                                                    need_heads)):
             V = wb.shape[0]
             if idx.numel() == 0 or dl is None or not (need_w or want_dyn):
                 dws.append(torch.zeros(V, D, dtype=f32, device=dev) if need_w else None)
                 continue
+            if ctx.probs[i] is None:
+                raise RuntimeError("egom2p_b200: the vocabulary head's backward ran twice (retain_graph) or its forward ran "
+                                   "without grad mode; its softmax numerators are freed by the first backward")
+            probs, rscale, tile_flag = ctx.probs[i]
+            ctx.probs[i] = None
             R = idx.numel()
             gscale = (dl.reshape(1).to(f32) / R).contiguous()
-            dw = torch.empty(V, D, dtype=f32, device=dev) if need_w else None
-            dym = torch.empty(R, D, dtype=f32, device=dev) if want_dyn else None
-            chunk = min(V, _HeadLossFn.CHUNK)
-            buf = torch.empty(R, chunk, dtype=bf16, device=dev)
-            for v0 in range(0, V, chunk):
-                vc = min(chunk, V - v0)
-                dlog = buf[:, :vc]
-                ops.ce_dlogits(ym, wb, tgt, lse, gscale, v0, vc, dlog)
-                if want_dyn:
-                    ops.gemm(dlog, wb[v0:v0 + vc], R, D, vc, b_mn=True, addend=dym if v0 else None, out_f32=dym)
-                if need_w:   # a frozen (tied) head gets no dW GEMM
-                    ops.gemm(dlog, ym, vc, D, R, a_mn=True, b_mn=True, out_f32=dw[v0:v0 + vc])
+            # rows of 128-row tiles whose numerators are not exact in bf16 get softmax - onehot recomputed (no launch work
+            # when no tile is flagged); then rscale * probs = softmax - onehot on every row, and with s = gscale * rscale:
+            # dY = diag(s) (probs W) (the scale applied by the scatter), dW = probs^T (diag(s) ym)
+            ops.ce_dlogits(ym, wb, tgt, lse, None, 0, V, probs, tile_flag=tile_flag)
+            s, ys = ops.ce_row_scale(ym, rscale, gscale, want_ys=need_w)
             if want_dyn:
-                ops.scatter_rows_f32(dym, idx, dyn)
+                dym = torch.empty(R, D, dtype=f32, device=dev)
+                ops.gemm(probs, wb, R, D, V, b_mn=True, out_f32=dym)
+                ops.scatter_rows_f32(dym, idx, dyn, row_scale=s)
+            dw = None
+            if need_w:   # a frozen (tied) head gets no dW GEMM
+                dw = torch.empty(V, D, dtype=f32, device=dev)
+                ops.gemm(probs, ys, V, D, R, a_mn=True, b_mn=True, out_f32=dw)
+            del probs
             dws.append(dw)
         dy = dnw = dnb = None
         if want_dyn:
@@ -577,7 +586,7 @@ class _HeadLossFn(torch.autograd.Function):
             dnb = _zeros(D, dev) if need_nb else None
             dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=need_y, d_bias=dnb)
             dy = _with_bf16(dy, dyb) if need_y else None
-        return (dy, dnw, dnb, None, None, None, None, None, *dws)
+        return (dy, dnw, dnb, None, None, None, None, None, None, *dws)
 
 
 # =============================================================================================== the module
@@ -1120,7 +1129,7 @@ class EgoM2P(nn.Module):
             heads.append(w)
             wbs.append(self._bf16(("head", m), w))
         per_mod = _HeadLossFn.apply(y, self.decoder_norm.weight, _bias(self.decoder_norm), rows, targets, wbs,
-                                    self.eps, self._epoch, *heads)
+                                    self.eps, self._epoch, torch.is_grad_enabled(), *heads)
         mod_loss = {}
         for m, l in zip(dec_mods, per_mod):
             if loss_type == "weighted_mod" and rows[dec_mods.index(m)].numel():

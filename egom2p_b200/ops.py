@@ -366,11 +366,19 @@ def linear_wgrad(dy: torch.Tensor, x: torch.Tensor, out: Optional[torch.Tensor] 
 
 
 # ----------------------------------------------------------------------------------------------- head + CE
-def ce_forward(y: torch.Tensor, w: torch.Tensor, target: torch.Tensor):
-    """Returns (loss_sum (1,) fp32, lse (R,) fp32) for logits = y @ w^T without materialising them."""
+def ce_forward(y: torch.Tensor, w: torch.Tensor, target: torch.Tensor, keep_probs: bool = False):
+    """Returns (loss_sum (1,) fp32, lse (R,) fp32) for logits = y @ w^T without materialising them.
+
+    keep_probs (a head that needs a backward): the same pass also stores the softmax numerators, and the result gets a third
+    item (probs (R, V) bf16, rscale (R,) fp32, tile_flag (ceil(R / 128),) uint8) with rscale[r] * probs[r, :] = softmax - onehot
+    on the rows of unflagged 128-row tiles; a flagged tile's numerators are not exact in bf16, and `ce_dlogits(...,
+    tile_flag=tile_flag)` recomputes them."""
     lib = _lib.load()
+    _req(y, bf16, "y"); _req(w, bf16, "w")
     R, K = y.shape
     V = w.shape[0]
+    _req_dense(target, torch.int64, "target", R)
+    assert y.stride(1) == 1 and w.stride(1) == 1 and w.shape[1] == K
     nt = 2 * ((V + 255) // 256)  # two column halves per 256-wide vocabulary tile
     dev = y.device
     pm = torch.empty(nt, R, dtype=f32, device=dev)
@@ -378,20 +386,51 @@ def ce_forward(y: torch.Tensor, w: torch.Tensor, target: torch.Tensor):
     tl = torch.zeros(R, dtype=f32, device=dev)
     lse = torch.empty(R, dtype=f32, device=dev)
     loss = torch.zeros(1, dtype=f32, device=dev)
+    if not keep_probs:
+        with _timed("head_ce", 2.0 * R * V * K, "flop"):
+            _lib.check(lib.egom2p_ce_partials(_p(y), _p(w), _p(target), R, V, K, y.stride(0), w.stride(0), _p(pm), _p(ps),
+                                              _p(tl), _s()), "ce_partials")
+        _lib.check(lib.egom2p_ce_finalize(_p(pm), _p(ps), _p(tl), R, nt, _p(lse), _p(loss), None, None, 0, None, 0, None, None,
+                                          _s()), "ce_finalize")
+        return loss, lse
+    ref = torch.empty(R, dtype=f32, device=dev)
+    wmax2 = torch.empty(1, dtype=f32, device=dev)
+    probs = torch.empty(R, V, dtype=bf16, device=dev)
+    rscale = torch.empty(R, dtype=f32, device=dev)
+    tile_flag = torch.empty((R + 127) // 128, dtype=torch.uint8, device=dev)
     with _timed("head_ce", 2.0 * R * V * K, "flop"):
-        _lib.check(lib.egom2p_ce_partials(_p(y), _p(w), _p(target), R, V, K, y.stride(0), w.stride(0), _p(pm), _p(ps), _p(tl),
-                                          _s()), "ce_partials")
-    _lib.check(lib.egom2p_ce_finalize(_p(pm), _p(ps), _p(tl), R, nt, _p(lse), _p(loss), _s()), "ce_finalize")
-    return loss, lse
+        _lib.check(lib.egom2p_ce_row_ref(_p(y), _p(w), R, V, K, y.stride(0), w.stride(0), _p(wmax2), _p(ref), _s()), "ce_row_ref")
+        _lib.check(lib.egom2p_ce_probs(_p(y), _p(w), _p(target), _p(ref), R, V, K, y.stride(0), w.stride(0), _p(probs),
+                                       probs.stride(0), _p(pm), _p(ps), _p(tl), _s()), "ce_probs")
+    _lib.check(lib.egom2p_ce_finalize(_p(pm), _p(ps), _p(tl), R, nt, _p(lse), _p(loss), _p(ref), _p(target), V, _p(probs),
+                                      probs.stride(0), _p(rscale), _p(tile_flag), _s()), "ce_finalize")
+    return loss, lse, (probs, rscale, tile_flag)
 
 
-def ce_dlogits(y, w, target, lse, gscale: torch.Tensor, v0: int, vc: int, out: torch.Tensor):
+def ce_dlogits(y, w, target, lse, gscale: Optional[torch.Tensor], v0: int, vc: int, out: torch.Tensor,
+               tile_flag: Optional[torch.Tensor] = None):
+    """out = (softmax - onehot) * gscale over the vocabulary columns [v0, v0 + vc) (gscale None: 1). With tile_flag (from
+    ce_forward(keep_probs=True)) only the rows of flagged 128-row tiles are computed and written."""
     lib = _lib.load()
     R, K = y.shape
+    if tile_flag is not None:
+        _req_dense(tile_flag, torch.uint8, "tile_flag", (R + 127) // 128)
     with _timed("head_ce", 2.0 * R * vc * K, "flop"):
-        _lib.check(lib.egom2p_ce_dlogits(_p(y), _p(w), _p(target), _p(lse), _p(gscale), R, v0, vc, K, y.stride(0), w.stride(0),
-                                         _p(out), out.stride(0), _s()), "ce_dlogits")
+        _lib.check(lib.egom2p_ce_dlogits(_p(y), _p(w), _p(target), _p(lse), _p(gscale), _p(tile_flag), R, v0, vc, K, y.stride(0),
+                                         w.stride(0), _p(out), out.stride(0), _s()), "ce_dlogits")
     return out
+
+
+def ce_row_scale(y: torch.Tensor, rscale: torch.Tensor, gscale: torch.Tensor, want_ys: bool = True):
+    """s = gscale * rscale (R,) fp32, and ys = bf16(s[:, None] * y) (R, K) when want_ys (else None)."""
+    lib = _lib.load()
+    _req(y, bf16, "y")
+    R, K = y.shape
+    _req_dense(rscale, f32, "rscale", R); _req_dense(gscale, f32, "gscale", 1)
+    s = torch.empty(R, dtype=f32, device=y.device)
+    ys = torch.empty(R, K, dtype=bf16, device=y.device) if want_ys else None
+    _lib.check(lib.egom2p_ce_row_scale(_p(y), R, K, y.stride(0), _p(rscale), _p(gscale), _p(s), _p(ys), _s()), "ce_row_scale")
+    return s, ys
 
 
 # ----------------------------------------------------------------------------------------------- attention
@@ -548,16 +587,18 @@ def gather_rows_bf16(src: torch.Tensor, idx: torch.Tensor):
     return dst
 
 
-def scatter_rows_f32(src: torch.Tensor, idx: torch.Tensor, dst: torch.Tensor):
-    """dst[idx[i]] = src[i]: src (n, cols) and dst (rows, cols) fp32 with row pitch cols, idx int64 contiguous (every entry
-    < rows); rows of dst that idx does not name are left as they are."""
+def scatter_rows_f32(src: torch.Tensor, idx: torch.Tensor, dst: torch.Tensor, row_scale: Optional[torch.Tensor] = None):
+    """dst[idx[i]] = src[i] (times row_scale[i] when given, fp32 (n,)): src (n, cols) and dst (rows, cols) fp32 with row
+    pitch cols, idx int64 contiguous (every entry < rows); rows of dst that idx does not name are left as they are."""
     lib = _lib.load()
     _req_rows(src, f32, "src", src.shape[-1])
     _req_rows(dst, f32, "dst", src.shape[1])
     _req_dense(idx, torch.int64, "idx", src.shape[0])
+    if row_scale is not None:
+        _req_dense(row_scale, f32, "row_scale", src.shape[0])
     n, cols = idx.numel(), src.shape[1]
     if n:
-        _lib.check(lib.egom2p_scatter_rows_f32(_p(src), _p(idx), n, cols, _p(dst), _s()), "scatter_rows_f32")
+        _lib.check(lib.egom2p_scatter_rows_f32(_p(src), _p(idx), n, cols, _p(row_scale), _p(dst), _s()), "scatter_rows_f32")
     return dst
 
 

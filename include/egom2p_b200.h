@@ -151,14 +151,31 @@ int egom2p_gemm_gelu_bwd(const uint16_t* dY, const uint16_t* W2, const uint16_t*
  * n_tiles = 2 * ceil(V / 256) (two column halves per 256-wide vocabulary tile); tgt_logit (R) fp32. */
 int egom2p_ce_partials(const uint16_t* Y, const uint16_t* W, const int64_t* target, int32_t R, int32_t V, int32_t K,
                        int64_t ldy, int64_t ldw, float* part_max, float* part_sum, float* tgt_logit, void* stream);
-/* Pass 2: lse[r] = logsumexp over tiles; loss_sum += sum_r (lse[r] - tgt_logit[r]) (one fp32, atomically). */
+/* Pass 1 of a head that needs a backward: the same partials, and the softmax numerators
+ * probs[r, v] = 2^(logit * log2 e - ref[r]) as bf16 (R, V), row pitch ldp. ref (R) fp32 from egom2p_ce_row_ref. */
+int egom2p_ce_probs(const uint16_t* Y, const uint16_t* W, const int64_t* target, const float* ref, int32_t R, int32_t V,
+                    int32_t K, int64_t ldy, int64_t ldw, uint16_t* probs, int64_t ldp, float* part_max, float* part_sum,
+                    float* tgt_logit, void* stream);
+/* ref[r] = ||Y_r|| * max_v ||W_v|| * log2 e (an upper bound of every logit of row r, in log2 units); wmax2: one fp32 of
+ * scratch. K, ldy, ldw multiples of 8. */
+int egom2p_ce_row_ref(const uint16_t* Y, const uint16_t* W, int32_t R, int32_t V, int32_t K, int64_t ldy, int64_t ldw,
+                      float* wmax2, float* ref, void* stream);
+/* Pass 2: lse[r] = logsumexp over tiles; loss_sum += sum_r (lse[r] - tgt_logit[r]) (one fp32, atomically).
+ * After egom2p_ce_probs (ref non-null, else the last six arguments are ignored): per 128-row tile, tile_flag = 1 when a
+ * row has ref[r] - max logit * log2 e > 60 (its numerators are not exact in bf16); otherwise rscale[r] = 1 / sum_v probs[r, v]
+ * and probs[r, target[r]] -= that sum, so that rscale[r] * probs[r, :] = softmax - onehot. Flagged tiles get rscale = 1. */
 int egom2p_ce_finalize(const float* part_max, const float* part_sum, const float* tgt_logit, int32_t R,
-                       int32_t n_tiles, float* lse, float* loss_sum, void* stream);
+                       int32_t n_tiles, float* lse, float* loss_sum, const float* ref, const int64_t* target, int32_t V,
+                       uint16_t* probs, int64_t ldp, float* rscale, uint8_t* tile_flag, void* stream);
 /* Backward recompute: dlogits[r, v0:v0+Vc] = (exp(logit - lse[r]) - [v == target[r]]) * gscale[0] as bf16 (R, Vc),
- * for the vocab chunk [v0, v0+Vc). gscale is a device scalar (upstream grad / R). */
+ * for the vocab chunk [v0, v0+Vc). gscale is a device scalar (upstream grad / R), or null for 1. With tile_flag
+ * (the loss pass's flags) only the flagged 128-row tiles are computed and written; the launch is one round of CTA pairs. */
 int egom2p_ce_dlogits(const uint16_t* Y, const uint16_t* W, const int64_t* target, const float* lse,
-                      const float* gscale, int32_t R, int32_t v0, int32_t Vc, int32_t K, int64_t ldy, int64_t ldw,
-                      uint16_t* dlogits, int64_t ldd, void* stream);
+                      const float* gscale, const uint8_t* tile_flag, int32_t R, int32_t v0, int32_t Vc, int32_t K,
+                      int64_t ldy, int64_t ldw, uint16_t* dlogits, int64_t ldd, void* stream);
+/* Row scales of the head backward: s[r] = gscale[0] * rscale[r]; ys (R, K) bf16 = s[r] * Y[r, :] when ys is non-null. */
+int egom2p_ce_row_scale(const uint16_t* Y, int32_t R, int32_t K, int64_t ldy, const float* rscale, const float* gscale,
+                        float* s, uint16_t* ys, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * (2) Attention, head_dim 64, tcgen05/TMEM tiles fed by TMA, online softmax in fp32
@@ -242,10 +259,12 @@ int egom2p_colsum_f32(const float* x, int64_t rows, int32_t cols, float* out, vo
 /* out[c] += sum_r x[r, c] for a bf16 (rows, cols) matrix of row pitch ld (cols, ld multiples of 8): the bias gradients of
  * the GELU / bias family's Linears from the bf16 output gradients, one atomic per column and row slab. */
 int egom2p_colsum_bf16(const uint16_t* x, int64_t rows, int32_t cols, int64_t ld, float* out, void* stream);
-/* dst[i, :] = src[idx[i], :] (bf16) and dst[idx[i], :] = src[i, :] (fp32): compaction of the rows of one modality for
- * its vocabulary head, replacing the boolean row-select y[decoder_mod_mask == id] (egom2p_model.py:633). */
+/* dst[i, :] = src[idx[i], :] (bf16) and dst[idx[i], :] = src[i, :] (fp32; times row_scale[i] when row_scale is given):
+ * compaction of the rows of one modality for its vocabulary head, replacing the boolean row-select
+ * y[decoder_mod_mask == id] (egom2p_model.py:633). */
 int egom2p_gather_rows_bf16(const uint16_t* src, const int64_t* idx, int64_t n, int32_t cols, uint16_t* dst, void* stream);
-int egom2p_scatter_rows_f32(const float* src, const int64_t* idx, int64_t n, int32_t cols, float* dst, void* stream);
+int egom2p_scatter_rows_f32(const float* src, const int64_t* idx, int64_t n, int32_t cols, const float* row_scale, float* dst,
+                            void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Device-side masking of the token modalities: UnifiedMasking.image_mask (egom2p/data/masking.py:236-266) for a whole batch
