@@ -18,6 +18,7 @@ from __future__ import annotations
 import math
 import random
 from functools import partial
+from itertools import chain, islice
 from typing import Any, Dict, List, Optional, Union
 
 import torch
@@ -56,7 +57,7 @@ def _bias(m: nn.Module) -> Optional[torch.Tensor]:
 
 
 def _weights_and_biases(*mods: nn.Module) -> List[Optional[torch.Tensor]]:
-    """weight, bias (or None) of each module in turn: the flat parameter list the block functions take."""
+    """weight, bias (or None) of each module in turn: a sub-layer's flat parameter list (see _SelfAttention)."""
     return [t for m in mods for t in (m.weight, _bias(m))]
 
 
@@ -75,10 +76,11 @@ class _Linear(nn.Linear):
         return y.reshape(*shape[:-1], -1)
 
 
-# The MLP is the only part of a block that differs between the two families. Each MLP container owns, for the shared block
-# code: params() -- its parameters, in the order the block functions take them; operands() -- their cached bf16 GEMM
-# operands; fwd() -- x1 + MLP(h2) from the normed h2, and what bwd() needs; bwd() -- dh2 and the gradients of params(), None
-# for each parameter whose flag in `need` is False (a frozen parameter gets neither its wgrad GEMM nor its bias column sum).
+# The MLP is the only part of a block that differs between the two families. Each MLP container owns, for the MLP sub-layer
+# (_MlpLayer, which adds norm2): params() -- its parameters, in the order the block function takes them; operands() -- their
+# cached bf16 GEMM operands; fwd() -- x1 + MLP(h2) from the normed h2, and what bwd() needs; bwd() -- dh2 and the gradients
+# of params(), None for each parameter whose flag in `need` is False (a frozen parameter gets neither its wgrad GEMM nor its
+# bias column sum).
 class GatedMlp(nn.Module):
     """fc2(SiLU(fc1 x) * fc3 x) without biases (the swiglu / no-bias family). fc1 and fc3 run as one GEMM over an operand
     with their rows interleaved (EgoM2P._bf16), the gate in its epilogue."""
@@ -169,6 +171,7 @@ class Block(nn.Module):
         self.attn = Attention(dim, num_heads, bias=gelu)
         self.norm2 = norm_layer(dim)
         self.mlp = Mlp(dim, int(dim * mlp_ratio)) if gelu else GatedMlp(dim, int(dim * mlp_ratio))
+        self.layers = (_SelfAttention(self.norm1, self.attn, decoder=False), _MlpLayer(self.norm2, self.mlp))
 
 
 class DecoderBlock(nn.Module):
@@ -181,6 +184,8 @@ class DecoderBlock(nn.Module):
         self.context_norm = norm_layer(dim)
         self.norm2 = norm_layer(dim)
         self.mlp = Mlp(dim, int(dim * mlp_ratio)) if gelu else GatedMlp(dim, int(dim * mlp_ratio))
+        self.layers = (_SelfAttention(self.norm1, self.self_attn, decoder=True),
+                       _CrossAttention(self.query_norm, self.context_norm, self.cross_attn), _MlpLayer(self.norm2, self.mlp))
 
 
 # =============================================================================================== kernels glue
@@ -246,200 +251,226 @@ def _bf16_of(dx):
     return ops.cast_bf16(dx)
 
 
-def _mlp_fwd(mlp, x1, n2w, n2b, w, params, eps):
-    """x1 + mlp(norm2 x1). w: the MLP's bf16 operands (mlp.operands), params: its parameters (mlp.params)."""
-    h2, _, mean2, rstd2 = ops.layernorm_fwd(x1, n2w, eps, bias=n2b)
-    x2, sm = mlp.fwd(h2, x1, w, params)
-    return x2, (mean2, rstd2, h2, *sm)
+def _split(seq, sizes):
+    """seq cut into consecutive tuples of the given sizes."""
+    it = iter(seq)
+    return [tuple(islice(it, n)) for n in sizes]
 
 
-def _mlp_bwd(mlp, dx2, x1, n2w, w, saved, need):
-    """need: whether norm2's weight and bias, then each of mlp.params(), want a gradient (False for an absent bias).
-    Returns dx1 (incl. the residual path), its bf16 copy, dn2w, dn2b and the gradients of mlp.params(), None where not
-    wanted."""
-    mean2, rstd2, h2, *sm = saved
-    dh2, dparams = mlp.bwd(_bf16_of(dx2), h2, w, sm, need[2:])
-    dn2w = _zeros(n2w.numel(), dx2.device) if need[0] else None
-    dn2b = _zeros(n2w.numel(), dx2.device) if need[1] else None
-    dx1, dx1b = ops.layernorm_bwd(dh2, x1, n2w, mean2, rstd2, dx_in=dx2, d_weight=dn2w, want_bf16=True, d_bias=dn2b)
-    return dx1, dx1b, dn2w, dn2b, dparams
+def _layernorm_bwd(dh, x, w, mean, rstd, need_w, need_b, dx_in=None, want_bf16=False):
+    """LayerNorm backward that reduces the weight and the bias gradient only where wanted: dx, its bf16 copy, dw, db."""
+    dw = _zeros(w.numel(), x.device) if need_w else None
+    db = _zeros(w.numel(), x.device) if need_b else None
+    dx, dxb = ops.layernorm_bwd(dh, x, w, mean, rstd, dx_in=dx_in, d_weight=dw, want_bf16=want_bf16, d_bias=db)
+    return dx, dxb, dw, db
 
 
-def _self_attn_fwd(x, n1w, wqkv, wproj, B, L, H, meta, eps, pairs, bias):
-    """bias: the (norm1, qkv, proj) biases, fp32 or None each."""
-    D = x.shape[-1]
-    n1b, bqkv, bproj = bias
-    h1, _, mean1, rstd1 = ops.layernorm_fwd(x, n1w, eps, bias=n1b)
-    qkv = ops.linear_fwd(h1, wqkv, bias=bqkv)
-    o, lse = ops.attn_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], B, H, L, L, meta=meta, pairs=pairs)
-    x1 = ops.linear_fwd(o, wproj, bias=bproj, addend=x, out_dtype=f32)
-    return x1, (mean1, rstd1, h1, qkv, o, lse)
+# A block is an ordered list of residual sub-layers (Block.layers, DecoderBlock.layers). Each is a view over modules of its
+# block -- it registers no module or parameter, so the state-dict names stay the reference's -- and owns:
+#   params()                 its flat parameter list, None for an absent bias: the only place their order is written;
+#   operands(cache, key)     its cached bf16 GEMM operands (EgoM2P._bf16 under the keys (*key, name));
+#   fwd(x, c, g, w, p, save) x + the sub-layer of x (c: the context rows, read by the cross-attention only) and the tensors
+#                            bwd() needs; save=False when no backward follows: LayerNorm statistics and lse are not written;
+#   bwd(dy, dyb, need_c, g, w, saved, need)
+#                            from the residual gradient and its bf16 copy: dx, its bf16 copy, the context's gradient (None
+#                            unless this sub-layer reads the context and need_c) and the gradients of params(), None for each
+#                            parameter whose flag in `need` is False (a frozen parameter gets no work launched for it).
+class _SelfAttention:
+    """x + proj(attention(qkv(norm x))) over the block's own rows: norm1 and attn (encoder) / self_attn (decoder)."""
+
+    def __init__(self, norm, attn, decoder):
+        self.norm, self.attn, self.decoder = norm, attn, decoder
+        self.n_params = len(self.params())
+
+    def params(self):
+        return _weights_and_biases(self.norm, self.attn.qkv, self.attn.proj)
+
+    def operands(self, cache, key):
+        return (cache((*key, "qkv"), self.attn.qkv.weight),
+                cache((*key, "sproj" if self.decoder else "proj"), self.attn.proj.weight))
+
+    def _rows(self, g):
+        """Rows per sample, range metadata and (query, key) pair count of this attention."""
+        return (g.M, g.m_dec, g.p_dec) if self.decoder else (g.N, g.m_enc, g.p_enc)
+
+    def fwd(self, x, c, g, w, p, save=True):
+        (wqkv, wproj), (nw, nb, _, bqkv, _, bproj) = w, p
+        D = x.shape[-1]
+        L, meta, pairs = self._rows(g)
+        h, _, mean, rstd = ops.layernorm_fwd(x, nw, g.eps, save_stats=save, bias=nb)
+        qkv = ops.linear_fwd(h, wqkv, bias=bqkv)
+        o, lse = ops.attn_fwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], g.B, g.H, L, L, want_lse=save, meta=meta, pairs=pairs)
+        return ops.linear_fwd(o, wproj, bias=bproj, addend=x, out_dtype=f32), (x, nw, mean, rstd, h, qkv, o, lse)
+
+    def bwd(self, dy, dyb, need_c, g, w, saved, need):
+        (wqkv, wproj), (x, nw, mean, rstd, h, qkv, o, lse) = w, saved
+        need_nw, need_nb, need_wqkv, need_bqkv, need_wproj, need_bproj = need
+        D = x.shape[-1]
+        L, meta, pairs = self._rows(g)
+        dwproj = ops.linear_wgrad(dyb, o) if need_wproj else None
+        do = ops.linear_dgrad(dyb, wproj)
+        dqkv = torch.empty_like(qkv)
+        ops.attn_bwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], o, do, lse, g.B, g.H, L, L, dqkv[:, :D], dqkv[:, D:2 * D],
+                     dqkv[:, 2 * D:], meta=meta, pairs=pairs)
+        dwqkv = ops.linear_wgrad(dqkv, h) if need_wqkv else None
+        dh = ops.linear_dgrad(dqkv, wqkv)
+        dbqkv = ops.colsum_bf16(dqkv) if need_bqkv else None
+        dbproj = ops.colsum_bf16(dyb) if need_bproj else None
+        dx, dxb, dnw, dnb = _layernorm_bwd(dh, x, nw, mean, rstd, need_nw, need_nb, dx_in=dy, want_bf16=True)
+        return dx, dxb, None, (dnw, dnb, dwqkv, dbqkv, dwproj, dbproj)
 
 
-def _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, saved, B, L, H, meta, pairs, need):
-    """need: whether the weight and bias of norm1, qkv and proj want a gradient (False for an absent bias). Returns dx,
-    dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj, None for each gradient not wanted."""
-    mean1, rstd1, h1, qkv, o, lse = saved
-    D = x.shape[-1]
-    need_n1w, need_n1b, need_wqkv, need_bqkv, need_wproj, need_bproj = need
-    dwproj = ops.linear_wgrad(dx1b, o) if need_wproj else None
-    do = ops.linear_dgrad(dx1b, wproj)
-    dqkv = torch.empty_like(qkv)
-    ops.attn_bwd(qkv[:, :D], qkv[:, D:2 * D], qkv[:, 2 * D:], o, do, lse, B, H, L, L, dqkv[:, :D], dqkv[:, D:2 * D],
-                 dqkv[:, 2 * D:], meta=meta, pairs=pairs)
-    dwqkv = ops.linear_wgrad(dqkv, h1) if need_wqkv else None
-    dh1 = ops.linear_dgrad(dqkv, wqkv)
-    dn1w = _zeros(n1w.numel(), x.device) if need_n1w else None
-    dn1b = _zeros(n1w.numel(), x.device) if need_n1b else None
-    dbqkv = ops.colsum_bf16(dqkv) if need_bqkv else None
-    dbproj = ops.colsum_bf16(dx1b) if need_bproj else None
-    dx, dxb = ops.layernorm_bwd(dh1, x, n1w, mean1, rstd1, dx_in=dx1, d_weight=dn1w, want_bf16=True, d_bias=dn1b)
-    return _with_bf16(dx, dxb), dn1w, dn1b, dwqkv, dbqkv, dwproj, dbproj
+class _CrossAttention:
+    """x + proj(attention(q(query_norm x), kv(context_norm c))): a decoder block's query_norm, context_norm and cross_attn."""
 
+    def __init__(self, query_norm, context_norm, attn):
+        self.query_norm, self.context_norm, self.attn = query_norm, context_norm, attn
+        self.n_params = len(self.params())
 
-def _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, bias):
-    """y2 = y1 + cross_attn(query_norm y1, context_norm context). bias: the (query_norm, context_norm, q, kv, proj) biases,
-    fp32 or None each."""
-    D = y1.shape[-1]
-    qnb, cnb, bq, bkv, bxproj = bias
-    hq, _, meanq, rstdq = ops.layernorm_fwd(y1, qnw, g.eps, bias=qnb)
-    q = ops.linear_fwd(hq, wq, bias=bq)
-    hc, _, meanc, rstdc = ops.layernorm_fwd(context, cnw, g.eps, bias=cnb)
-    kv = ops.linear_fwd(hc, wkv, bias=bkv)
-    o2, lse2 = ops.attn_fwd(q, kv[:, :D], kv[:, D:], g.B, g.H, g.M, g.N, meta=g.m_x, pairs=g.p_x)
-    y2 = ops.linear_fwd(o2, wxproj, bias=bxproj, addend=y1, out_dtype=f32)
-    return y2, (meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2)
+    def params(self):
+        return _weights_and_biases(self.query_norm, self.context_norm, self.attn.q, self.attn.kv, self.attn.proj)
 
+    def operands(self, cache, key):
+        a = self.attn
+        return cache((*key, "q"), a.q.weight), cache((*key, "kv"), a.kv.weight), cache((*key, "xproj"), a.proj.weight)
 
-def _cross_bwd(g, ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, saved, need, need_ctx):
-    """Backward of _cross_fwd. need: whether the weight and bias of query_norm, context_norm, q, kv and proj want a gradient
-    (False for an absent bias); need_ctx: whether `context` does. Returns dy1, dy1b, dctx (None unless this block returns
-    the summed context gradient), then dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj, None for each
-    gradient not wanted."""
-    meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o2, lse2 = saved
-    D = y1.shape[-1]
-    dev = y1.device
-    need_qnw, need_qnb, need_cnw, need_cnb, need_wq, need_bq, need_wkv, need_bkv, need_wxproj, need_bxproj = need
-    # the context side (kv dgrad, context_norm backward) runs for the context's gradient or for context_norm's own
-    ctx_side = need_ctx or need_cnw or need_cnb
-    dwxproj = ops.linear_wgrad(dy2b, o2) if need_wxproj else None
-    do2 = ops.linear_dgrad(dy2b, wxproj)
-    dq = torch.empty_like(q)
-    dkv = torch.empty_like(kv)
-    ops.attn_bwd(q, kv[:, :D], kv[:, D:], o2, do2, lse2, g.B, g.H, g.M, g.N, dq, dkv[:, :D], dkv[:, D:], meta=g.m_x, pairs=g.p_x)
-    dwq = ops.linear_wgrad(dq, hq) if need_wq else None
-    dhq = ops.linear_dgrad(dq, wq)
-    dwkv = ops.linear_wgrad(dkv, hc) if need_wkv else None
-    dhc = ops.linear_dgrad(dkv, wkv) if ctx_side else None
-    dqnw = _zeros(D, dev) if need_qnw else None
-    dcnw = _zeros(D, dev) if need_cnw else None
-    dqnb = _zeros(D, dev) if need_qnb else None
-    dcnb = _zeros(D, dev) if need_cnb else None
-    dbq = ops.colsum_bf16(dq) if need_bq else None
-    dbkv = ops.colsum_bf16(dkv) if need_bkv else None
-    dbxproj = ops.colsum_bf16(dy2b) if need_bxproj else None
-    dy1, dy1b = ops.layernorm_bwd(dhq, y1, qnw, meanq, rstdq, dx_in=dy2, d_weight=dqnw, want_bf16=True, d_bias=dqnb)
-    if not need_ctx:
-        if ctx_side:   # only context_norm's parameter reductions are wanted; its dx is discarded
-            ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, d_weight=dcnw, d_bias=dcnb)
-        return dy1, dy1b, None, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj
-    # All decoder blocks read the same `context`: instead of letting autograd add twelve (B*N, D) fp32 gradients pairwise,
-    # each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block that runs last
-    # returns it. g.ctx_users counts the blocks whose forward saw a context that wants a gradient (_DecoderBlockFn.forward).
-    # Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
-    acc = g.dctx_acc
-    chained = g.ctx_users > 0 and (acc is None or (acc[0] == ctx_key and acc[1].shape == context.shape))
-    last = chained and g.ctx_users == 1
-    dctx, dctxb = ops.layernorm_bwd(dhc, context, cnw, meanc, rstdc, dx_in=acc[1] if (chained and acc is not None) else None,
-                                    d_weight=dcnw, want_bf16=last, d_bias=dcnb)
-    if chained:
-        g.ctx_users -= 1
-        if last:
-            g.dctx_acc = None
-            dctx = _with_bf16(dctx, dctxb)
-        else:
-            g.dctx_acc = (ctx_key, dctx)
-            dctx = None
-    return dy1, dy1b, dctx, dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwxproj, dbxproj
-
-
-class _EncoderBlockFn(torch.autograd.Function):
-    """x + attn(norm1 x) then + mlp(norm2 .) -- egom2p_utils.py:356-359. Parameters: weight and bias of norm1, qkv, proj and
-    norm2, then mlp.params(); an absent bias is None. The backward computes the gradient of a parameter only when it
-    requires one (ctx.needs_input_grad): a frozen parameter gets None and no work is launched for it. dx is always computed."""
-
-    @staticmethod
-    def forward(ctx, x, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, proj_w, proj_b, n2w, n2b, *mlp_params):
-        wqkv, wproj, *wm = wb
-        g = geom
-        x1, sa = _self_attn_fwd(x, n1w, wqkv, wproj, g.B, g.N, g.H, g.m_enc, g.eps, g.p_enc, (n1b, qkv_b, proj_b))
-        x2, sm = _mlp_fwd(mlp, x1, n2w, n2b, wm, mlp_params, g.eps)
-        ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
-        ctx.op_epoch = geom.epoch_ref[0]
-        ctx.save_for_backward(x, n1w, n2w, x1, *sa, *sm)
-        return x2
-
-    @staticmethod
-    def backward(ctx, dx2):
-        _GRAD_GEN[0] += 1
-        _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
-        x, n1w, n2w, x1, *rest = ctx.saved_tensors
-        sa, sm = rest[:6], rest[6:]
-        wqkv, wproj, *wm = ctx.wb
-        g = ctx.geom
-        need = ctx.needs_input_grad
-        dx1, dx1b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dx2.contiguous(), x1, n2w, wm, sm, need[10:])
-        dx, *dsa = _self_attn_bwd(dx1, dx1b, x, n1w, wqkv, wproj, sa, g.B, g.N, g.H, g.m_enc, g.p_enc, need[4:10])
-        return (dx, None, None, None, *dsa, dn2w, dn2b, *dmlp)
-
-
-class _DecoderBlockFn(torch.autograd.Function):
-    """self-attn -> cross-attn(query_norm y, context_norm ctx) -> mlp -- egom2p_utils.py:387-391. Parameters: weight and bias
-    of norm1, qkv, self-attention proj, query_norm, context_norm, q, kv, cross-attention proj and norm2, then
-    mlp.params(); an absent bias is None. As in _EncoderBlockFn, only the parameters that require a gradient get one. dy is
-    always computed; the context's gradient (kv dgrad + context_norm backward) only when `context` requires one."""
-
-    @staticmethod
-    def forward(ctx, y, context, mlp, wb, geom, n1w, n1b, qkv_w, qkv_b, sproj_w, sproj_b, qnw, qnb, cnw, cnb, q_w, q_b, kv_w,
-                kv_b, xproj_w, xproj_b, n2w, n2b, *mlp_params):
-        wqkv, wsproj, wq, wkv, wxproj, *wm = wb
-        g = geom
-        y1, sa = _self_attn_fwd(y, n1w, wqkv, wsproj, g.B, g.M, g.H, g.m_dec, g.eps, g.p_dec, (n1b, qkv_b, sproj_b))
-        y2, sx = _cross_fwd(y1, context, qnw, cnw, wq, wkv, wxproj, g, (qnb, cnb, q_b, kv_b, xproj_b))
-        y3, sm = _mlp_fwd(mlp, y2, n2w, n2b, wm, mlp_params, g.eps)
-        ctx.geom, ctx.wb, ctx.mlp = geom, wb, mlp
-        ctx.op_epoch = geom.epoch_ref[0]
-        ctx.ctx_key = context.data_ptr()
-        if ctx.needs_input_grad[1]:   # this block's backward adds to the summed context gradient (_cross_bwd)
+    def fwd(self, x, c, g, w, p, save=True):
+        (wq, wkv, wproj), (qnw, qnb, cnw, cnb, _, bq, _, bkv, _, bproj) = w, p
+        D = x.shape[-1]
+        hq, _, meanq, rstdq = ops.layernorm_fwd(x, qnw, g.eps, save_stats=save, bias=qnb)
+        q = ops.linear_fwd(hq, wq, bias=bq)
+        hc, _, meanc, rstdc = ops.layernorm_fwd(c, cnw, g.eps, save_stats=save, bias=cnb)
+        kv = ops.linear_fwd(hc, wkv, bias=bkv)
+        o, lse = ops.attn_fwd(q, kv[:, :D], kv[:, D:], g.B, g.H, g.M, g.N, want_lse=save, meta=g.m_x, pairs=g.p_x)
+        if save and c.requires_grad:   # this block's backward adds to the summed context gradient (bwd)
             g.ctx_users += 1
-        ctx.save_for_backward(y, context, n1w, qnw, cnw, n2w, y1, y2, *sx, *sa, *sm)
-        return y3
+        return (ops.linear_fwd(o, wproj, bias=bproj, addend=x, out_dtype=f32),
+                (x, c, qnw, cnw, meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o, lse))
+
+    def bwd(self, dy, dyb, need_c, g, w, saved, need):
+        (wq, wkv, wproj), (x, c, qnw, cnw, meanq, rstdq, hq, q, meanc, rstdc, hc, kv, o, lse) = w, saved
+        need_qnw, need_qnb, need_cnw, need_cnb, need_wq, need_bq, need_wkv, need_bkv, need_wproj, need_bproj = need
+        D = x.shape[-1]
+        # the context side (kv dgrad, context_norm backward) runs for the context's gradient or for context_norm's own
+        ctx_side = need_c or need_cnw or need_cnb
+        dwproj = ops.linear_wgrad(dyb, o) if need_wproj else None
+        do = ops.linear_dgrad(dyb, wproj)
+        dq = torch.empty_like(q)
+        dkv = torch.empty_like(kv)
+        ops.attn_bwd(q, kv[:, :D], kv[:, D:], o, do, lse, g.B, g.H, g.M, g.N, dq, dkv[:, :D], dkv[:, D:], meta=g.m_x, pairs=g.p_x)
+        dwq = ops.linear_wgrad(dq, hq) if need_wq else None
+        dhq = ops.linear_dgrad(dq, wq)
+        dwkv = ops.linear_wgrad(dkv, hc) if need_wkv else None
+        dhc = ops.linear_dgrad(dkv, wkv) if ctx_side else None
+        dbq = ops.colsum_bf16(dq) if need_bq else None
+        dbkv = ops.colsum_bf16(dkv) if need_bkv else None
+        dbproj = ops.colsum_bf16(dyb) if need_bproj else None
+        dx, dxb, dqnw, dqnb = _layernorm_bwd(dhq, x, qnw, meanq, rstdq, need_qnw, need_qnb, dx_in=dy, want_bf16=True)
+        dc = dcnw = dcnb = None
+        if not need_c:
+            if ctx_side:   # only context_norm's parameter reductions are wanted; its dx is discarded
+                _, _, dcnw, dcnb = _layernorm_bwd(dhc, c, cnw, meanc, rstdc, need_cnw, need_cnb)
+        else:
+            # All decoder blocks read the same context: instead of letting autograd add twelve (B*N, D) fp32 gradients
+            # pairwise, each block's context_norm backward adds the running sum in its own pass (dx_in) and only the block
+            # that runs last returns it. g.ctx_users counts the blocks whose forward saw a context that wants a gradient
+            # (fwd). Falls back to one gradient per block whenever the bookkeeping does not match a plain single backward.
+            acc, key = g.dctx_acc, c.data_ptr()
+            chained = g.ctx_users > 0 and (acc is None or (acc[0] == key and acc[1].shape == c.shape))
+            last = chained and g.ctx_users == 1
+            dc, dcb, dcnw, dcnb = _layernorm_bwd(dhc, c, cnw, meanc, rstdc, need_cnw, need_cnb,
+                                                 dx_in=acc[1] if (chained and acc is not None) else None, want_bf16=last)
+            if chained:
+                g.ctx_users -= 1
+                if last:
+                    g.dctx_acc = None
+                    dc = _with_bf16(dc, dcb)
+                else:
+                    g.dctx_acc = (key, dc)
+                    dc = None
+        return dx, dxb, dc, (dqnw, dqnb, dcnw, dcnb, dwq, dbq, dwkv, dbkv, dwproj, dbproj)
+
+
+class _MlpLayer:
+    """x + mlp(norm2 x): a block's norm2 and its MLP container (GatedMlp or Mlp), which holds the family's GEMMs."""
+
+    def __init__(self, norm, mlp):
+        self.norm, self.mlp = norm, mlp
+        self.n_params = len(self.params())
+
+    def params(self):
+        return (*_weights_and_biases(self.norm), *self.mlp.params())
+
+    def operands(self, cache, key):
+        return self.mlp.operands(cache, key)
+
+    def fwd(self, x, c, g, w, p, save=True):
+        nw, nb, *mp = p
+        h, _, mean, rstd = ops.layernorm_fwd(x, nw, g.eps, save_stats=save, bias=nb)
+        y, sm = self.mlp.fwd(h, x, w, mp)
+        return y, (x, nw, mean, rstd, h, *sm)
+
+    def bwd(self, dy, dyb, need_c, g, w, saved, need):
+        x, nw, mean, rstd, h, *sm = saved
+        need_nw, need_nb, *need_mlp = need
+        dh, dmlp = self.mlp.bwd(dyb, h, w, sm, need_mlp)
+        dx, dxb, dnw, dnb = _layernorm_bwd(dh, x, nw, mean, rstd, need_nw, need_nb, dx_in=dy, want_bf16=True)
+        return dx, dxb, None, (dnw, dnb, *dmlp)
+
+
+class _BlockFn(torch.autograd.Function):
+    """One encoder or decoder block (egom2p_utils.py:356-359, 387-391): h through block.layers in order. operands: each
+    sub-layer's operands(); params: each sub-layer's params() in turn. The backward walks the sub-layers in reverse and
+    computes the gradient of a parameter only when it requires one (ctx.needs_input_grad): a frozen parameter gets None and
+    no work is launched for it. dh is always computed; the context's gradient only when `context` requires one. One
+    autograd node per block, so that DDP's bucketed all-reduce overlaps the backward as for the reference."""
 
     @staticmethod
-    def backward(ctx, dy3):
+    def forward(ctx, h, context, block, operands, geom, *params):
+        saved = []
+        for layer, w, p in zip(block.layers, operands, _split(params, [layer.n_params for layer in block.layers])):
+            h, s = layer.fwd(h, context, geom, w, p)
+            saved.append(s)
+        ctx.block, ctx.operands, ctx.geom = block, operands, geom
+        ctx.op_epoch = geom.epoch_ref[0]
+        ctx.n_saved = [len(s) for s in saved]
+        ctx.save_for_backward(*chain.from_iterable(saved))
+        return h
+
+    @staticmethod
+    def backward(ctx, dh):
         _GRAD_GEN[0] += 1
         _check_epoch(ctx.geom.epoch_ref, ctx.op_epoch)
-        (y, context, n1w, qnw, cnw, n2w, y1, y2, *rest) = ctx.saved_tensors
-        sx, sa, sm = rest[:10], rest[10:16], rest[16:]
-        wqkv, wsproj, wq, wkv, wxproj, *wm = ctx.wb
-        g = ctx.geom
-        need = ctx.needs_input_grad
-        dy2, dy2b, dn2w, dn2b, dmlp = _mlp_bwd(ctx.mlp, dy3.contiguous(), y2, n2w, wm, sm, need[21:])
-        dy1, dy1b, dctx, *dxa = _cross_bwd(g, ctx.ctx_key, dy2, dy2b, y1, context, qnw, cnw, wq, wkv, wxproj, sx, need[11:21],
-                                           need[1])
-        dy, *dsa = _self_attn_bwd(dy1, dy1b, y, n1w, wqkv, wsproj, sa, g.B, g.M, g.H, g.m_dec, g.p_dec, need[5:11])
-        return (dy, dctx, None, None, None, *dsa, *dxa, dn2w, dn2b, *dmlp)
+        layers = ctx.block.layers
+        _, need_c, _, _, _, *need = ctx.needs_input_grad
+        steps = list(zip(layers, ctx.operands, _split(ctx.saved_tensors, ctx.n_saved),
+                         _split(need, [layer.n_params for layer in layers])))
+        dh = dh.contiguous()
+        dhb = _bf16_of(dh)
+        dctx, grads = None, []
+        for layer, w, saved, need_p in reversed(steps):
+            dh, dhb, dc, dp = layer.bwd(dh, dhb, need_c, ctx.geom, w, saved, need_p)
+            dctx = dctx if dc is None else dc
+            grads[:0] = dp
+        return (_with_bf16(dh, dhb), dctx, None, None, None, *grads)
+
+
+def _context_fwd(x, enc_emb, norm_w, norm_b, proj_b, operand, eps, save=True):
+    """context = decoder_proj_context(encoder_norm(x)) + encoder_emb -- egom2p_model.py:499,722, and the encoder_norm
+    statistics and output the backward needs (save=False: no statistics are written). norm_b: encoder_norm's bias (GELU /
+    bias family) or None. operand(): the projection's bf16 operand, asked for after encoder_norm is launched (where
+    encode_tokens casts it on first use)."""
+    h, _, mean, rstd = ops.layernorm_fwd(x, norm_w, eps, save_stats=save, bias=norm_b)
+    return ops.linear_fwd(h, operand(), bias=proj_b, addend=enc_emb, out_dtype=f32), (mean, rstd, h)
 
 
 class _ContextFn(torch.autograd.Function):
-    """context = decoder_proj_context(encoder_norm(x)) + encoder_emb -- egom2p_model.py:499,722. norm_b: encoder_norm's
-    bias (GELU / bias family) or None. The backward skips the projection's dw / db when frozen, and the dgrad and
+    """_context_fwd as an autograd node. The backward skips the projection's dw / db when frozen, and the dgrad and
     encoder_norm backward when neither x nor encoder_norm wants a gradient."""
 
     @staticmethod
     def forward(ctx, x, enc_emb, norm_w, norm_b, proj_w, proj_b, wb, eps, epoch_ref):
-        h, _, mean, rstd = ops.layernorm_fwd(x, norm_w, eps, bias=norm_b)
-        context = ops.linear_fwd(h, wb, bias=proj_b, addend=enc_emb, out_dtype=f32)
+        context, (mean, rstd, h) = _context_fwd(x, enc_emb, norm_w, norm_b, proj_b, lambda: wb, eps)
         ctx.wb = wb
         ctx.epoch_ref, ctx.op_epoch = epoch_ref, epoch_ref[0]
         ctx.save_for_backward(x, norm_w, mean, rstd, h)
@@ -459,9 +490,7 @@ class _ContextFn(torch.autograd.Function):
         dx = dnw = dnb = None
         if upstream:
             dh = ops.linear_dgrad(dcb, ctx.wb)
-            dnw = _zeros(norm_w.numel(), x.device) if need_nw else None
-            dnb = _zeros(norm_w.numel(), x.device) if need_nb else None
-            dx, dxb = ops.layernorm_bwd(dh, x, norm_w, mean, rstd, d_weight=dnw, want_bf16=need_x, d_bias=dnb)
+            dx, dxb, dnw, dnb = _layernorm_bwd(dh, x, norm_w, mean, rstd, need_nw, need_nb, want_bf16=need_x)
             dx = _with_bf16(dx, dxb) if need_x else None
         return dx, dctx if need_emb else None, dnw, dnb, dw, db, None, None, None
 
@@ -582,9 +611,7 @@ class _HeadLossFn(torch.autograd.Function):
             dws.append(dw)
         dy = dnw = dnb = None
         if want_dyn:
-            dnw = _zeros(D, dev) if need_nw else None
-            dnb = _zeros(D, dev) if need_nb else None
-            dy, dyb = ops.layernorm_bwd(dyn, y, norm_w, mean, rstd, d_weight=dnw, want_bf16=need_y, d_bias=dnb)
+            dy, dyb, dnw, dnb = _layernorm_bwd(dyn, y, norm_w, mean, rstd, need_nw, need_nb, want_bf16=need_y)
             dy = _with_bf16(dy, dyb) if need_y else None
         return (dy, dnw, dnb, None, None, None, None, None, None, *dws)
 
@@ -782,58 +809,30 @@ class EgoM2P(nn.Module):
         neither bumps Tensor._version nor follows a backward of this module (see _GRAD_GEN)."""
         _GRAD_GEN[0] += 1
 
-    def _enc_weights(self, i: int):
-        b = self.encoder[i]
-        return (self._bf16(("e", i, "qkv"), b.attn.qkv.weight), self._bf16(("e", i, "proj"), b.attn.proj.weight),
-                *b.mlp.operands(self._bf16, ("e", i)))
-
-    def _dec_weights(self, i: int):
-        b = self.decoder[i]
-        return (self._bf16(("d", i, "qkv"), b.self_attn.qkv.weight), self._bf16(("d", i, "sproj"), b.self_attn.proj.weight),
-                self._bf16(("d", i, "q"), b.cross_attn.q.weight), self._bf16(("d", i, "kv"), b.cross_attn.kv.weight),
-                self._bf16(("d", i, "xproj"), b.cross_attn.proj.weight), *b.mlp.operands(self._bf16, ("d", i)))
+    def _operands(self, blk, key):
+        """The bf16 GEMM operands of each sub-layer of a block; key: ("e", i) or ("d", i)."""
+        return [layer.operands(self._bf16, key) for layer in blk.layers]
 
     # ------------------------------------------------------------------ block application (training)
-    def _enc_block(self, i, blk, h, g):
-        return _EncoderBlockFn.apply(h, blk.mlp, self._enc_weights(i), g,
-                                     *_weights_and_biases(blk.norm1, blk.attn.qkv, blk.attn.proj, blk.norm2), *blk.mlp.params())
-
-    def _dec_block(self, i, blk, h, c, g):
-        sa, xa = blk.self_attn, blk.cross_attn
-        return _DecoderBlockFn.apply(h, c, blk.mlp, self._dec_weights(i), g,
-                                     *_weights_and_biases(blk.norm1, sa.qkv, sa.proj, blk.query_norm, blk.context_norm, xa.q,
-                                                          xa.kv, xa.proj, blk.norm2), *blk.mlp.params())
+    def _block(self, blk, key, h, c, g):
+        return _BlockFn.apply(h, c, blk, self._operands(blk, key), g, *[p for layer in blk.layers for p in layer.params()])
 
     # ------------------------------------------------------------------ blocks without autograd (generation / sampler paths)
-    def _self_attn_infer(self, attn, norm, h, wqkv, wproj, B, L, meta):
-        return _self_attn_fwd(h, norm.weight, wqkv, wproj, B, L, self.num_heads, meta, self.eps, None,
-                              (_bias(norm), _bias(attn.qkv), _bias(attn.proj)))[0]
-
-    def _mlp_infer(self, blk, h, wm):
-        return _mlp_fwd(blk.mlp, h, blk.norm2.weight, _bias(blk.norm2), wm, blk.mlp.params(), self.eps)[0]
-
     def _decoder_infer(self, h, c, g):
         """The decoder blocks over h (g.B * g.M rows, fp32). c: the context rows that g.m_x ranges over, or None when no
         sample has context: a softmax over zero keys times an empty V is exactly 0 (SURVEY.md A5), so each cross-attention
         then adds only its projection's bias, if it has one."""
-        B, M, D = g.B, g.M, g.D
         zero = None
         for i, blk in enumerate(self.decoder):
-            wqkv, wsproj, wq, wkv, wxproj, *wm = self._dec_weights(i)
-            h = self._self_attn_infer(blk.self_attn, blk.norm1, h, wqkv, wsproj, B, M, g.m_dec)
-            xa = blk.cross_attn
+            (sa, xa, mlp), (w_sa, w_xa, w_mlp) = blk.layers, self._operands(blk, ("d", i))
+            h = sa.fwd(h, None, g, w_sa, sa.params())[0]
             if c is not None:
-                hq, _, _, _ = ops.layernorm_fwd(h, blk.query_norm.weight, g.eps, save_stats=False, bias=_bias(blk.query_norm))
-                q = ops.linear_fwd(hq, wq, bias=_bias(xa.q))
-                hc, _, _, _ = ops.layernorm_fwd(c, blk.context_norm.weight, g.eps, save_stats=False, bias=_bias(blk.context_norm))
-                kv = ops.linear_fwd(hc, wkv, bias=_bias(xa.kv))
-                o2, _ = ops.attn_fwd(q, kv[:, :D], kv[:, D:], B, g.H, M, g.N, meta=g.m_x, want_lse=False)
-                h = ops.linear_fwd(o2, wxproj, bias=_bias(xa.proj), addend=h, out_dtype=f32)
-            elif _bias(xa.proj) is not None:
+                h = xa.fwd(h, c, g, w_xa, xa.params(), save=False)[0]
+            elif _bias(xa.attn.proj) is not None:
                 if zero is None:
-                    zero = torch.zeros(B * M, D, dtype=bf16, device=h.device)
-                h = ops.linear_fwd(zero, wxproj, bias=_bias(xa.proj), addend=h, out_dtype=f32)
-            h = self._mlp_infer(blk, h, wm)
+                    zero = torch.zeros(g.B * g.M, g.D, dtype=bf16, device=h.device)
+                h = ops.linear_fwd(zero, w_xa[2], bias=_bias(xa.attn.proj), addend=h, out_dtype=f32)
+            h = mlp.fwd(h, None, g, w_mlp, mlp.params())[0]
         return h
 
     # ------------------------------------------------------------------ sampler-facing pieces (reference :251-283,483-551)
@@ -882,7 +881,7 @@ class EgoM2P(nn.Module):
         g.build_meta(x.device)
         h = x.reshape(B * N, D).float().contiguous()
         for i, blk in enumerate(self.encoder):
-            h = self._enc_block(i, blk, h, g)
+            h = self._block(blk, ("e", i), h, None, g)
         return self.encoder_norm(h).reshape(B, N, D)
 
     def forward_decoder(self, y, context, encoder_mask, decoder_attention_mask):
@@ -901,7 +900,7 @@ class EgoM2P(nn.Module):
         else:
             c = context.reshape(B * N, D).float().contiguous()
             for i, blk in enumerate(self.decoder):
-                h = self._dec_block(i, blk, h, c, g)
+                h = self._block(blk, ("d", i), h, c, g)
         return self.decoder_norm(h).reshape(B, M, D)
 
     def forward_logits(self, y, decoder_mod_dict, decoder_mod_mask, return_all_logits: bool = False):
@@ -934,13 +933,11 @@ class EgoM2P(nn.Module):
         g.enc_hi = ep.n_valid[:, None].expand(B, N).contiguous()
         g.build_meta(dev)
         for i, blk in enumerate(self.encoder):
-            wqkv, wproj, *wm = self._enc_weights(i)
-            x = self._self_attn_infer(blk.attn, blk.norm1, x, wqkv, wproj, B, N, g.m_enc)
-            x = self._mlp_infer(blk, x, wm)
-        h, _, _, _ = ops.layernorm_fwd(x, self.encoder_norm.weight.detach(), self.eps, save_stats=False,
-                                       bias=_det(_bias(self.encoder_norm)))
-        context = ops.linear_fwd(h, self._bf16("ctx", self.decoder_proj_context.weight), bias=self.decoder_proj_context.bias.detach(),
-                                 addend=emb, out_dtype=f32)
+            for layer, w in zip(blk.layers, self._operands(blk, ("e", i))):
+                x = layer.fwd(x, None, g, w, layer.params())[0]
+        context, _ = _context_fwd(x, emb, self.encoder_norm.weight.detach(), _det(_bias(self.encoder_norm)),
+                                  self.decoder_proj_context.bias.detach(),
+                                  partial(self._bf16, "ctx", self.decoder_proj_context.weight), self.eps, save=False)
         return context.reshape(B, N, D), ep.n_valid
 
     @torch.no_grad()
@@ -1002,6 +999,7 @@ class EgoM2P(nn.Module):
         g.B, g.N, g.M, g.H, g.D, g.eps = B, N, M, self.num_heads, self.dim, self.eps
         g.enc_lo = g.enc_hi = g.dec_lo = g.dec_hi = g.x_lo = g.x_hi = None
         g.m_enc = g.m_dec = g.m_x = None
+        g.p_enc = g.p_dec = g.p_x = None
         g.ctx_users, g.dctx_acc = 0, None   # decoder blocks of this forward that read `context` / their running gradient
         g.epoch_ref = self._epoch
         return g
@@ -1101,13 +1099,13 @@ class EgoM2P(nn.Module):
 
         # ---- encoder
         for i, blk in enumerate(self.encoder):
-            x = self._enc_block(i, blk, x, g)
+            x = self._block(blk, ("e", i), x, None, g)
         context = _ContextFn.apply(x, enc_emb, self.encoder_norm.weight, _bias(self.encoder_norm), self.decoder_proj_context.weight,
                                    self.decoder_proj_context.bias, self._bf16("ctx", self.decoder_proj_context.weight), self.eps,
                                    self._epoch)
         # ---- decoder
         for i, blk in enumerate(self.decoder):
-            y = self._dec_block(i, blk, y, context, g)
+            y = self._block(blk, ("d", i), y, context, g)
 
         if return_logits:
             yn = self.decoder_norm(y)
